@@ -2,6 +2,7 @@
 """bench.py -- the driver's measurement contract for the attention hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload flux|...] [--extras all|none|a,b]
+                    [--dump-outputs DIR]
 
 Headline (unchanged since round 1): a "step" is one forward pass of the fused attention kernel over the FLUX.1-schnell
 joint-attention shape (BASELINE.json configs[1]: bf16, B=1, H=24, N=4608, D=128, non-causal) per GPU.  With N>1 every rank
@@ -29,6 +30,11 @@ Printed JSON (rank 0, one line):
                ring128k_fwdbwd          the same with the native ring backward behind every forward
 
 --impl reference times that CPU oracle alone (the reference's Metal path cannot run on Linux; DESIGN.md).
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step of the selected workload computed (rank 0) as
+DIR/<name>.npy in float32: o (forward), lse dq dk dv dterm (forward + backward).  Inputs come from fixed seeds, so two
+builds run with the same arguments can be compared output for output.  Outputs larger than DUMP_BYTES in all are stored
+as a fixed, seeded sample of rows (sample_outputs).
 """
 import argparse
 import ctypes
@@ -73,6 +79,7 @@ WORKLOADS = {
 }
 ALL_EXTRAS = ["fwdbwd_flux", "c4_fwdbwd_heads_sharded", "int8_block", "int4_block", "fp32_flux", "d256_fwd", "mask_bf16_dense", "ring128k",
               "ring128k_fwdbwd"]
+DUMP_BYTES = 60_000_000          # float32 payload of --dump-outputs; with the .npy headers the files stay under 64 MB
 
 
 def visible_pairs(Sq, Skv, causal, window):
@@ -89,6 +96,31 @@ def visible_pairs(Sq, Skv, causal, window):
 
 def fwd_flops(w):
     return 4.0 * w["B"] * w["H"] * visible_pairs(w["Sq"], w["Skv"], w["causal"], w["window"]) * w["D"]
+
+
+def sample_outputs(named):
+    """Float32 device copies of the named output tensors ([B, H, S, D] or [B, H, S]), DUMP_BYTES at most together.  Arrays
+    that fit are copied whole; otherwise each keeps the same share of its rows (rows of D for [B, H, S, D], single values for
+    [B, H, S]), picked by a fixed seed and kept in order, as a 2-D [rows, D or 1] array."""
+    import torch
+    total = sum(t.numel() * 4 for t in named.values())
+    out = {}
+    for name, t in named.items():
+        if total <= DUMP_BYTES:
+            out[name] = t.to(torch.float32, copy=True)
+            continue
+        rows = t.reshape(-1, t.shape[-1]) if t.dim() == 4 else t.reshape(-1, 1)
+        keep = max(1, rows.shape[0] * DUMP_BYTES // total)
+        idx = torch.randperm(rows.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        out[name] = rows.index_select(0, idx.to(t.device)).to(torch.float32)
+    return out
+
+
+def write_outputs(out_dir, named):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in named.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy())
 
 
 def kernel_source_sha():
@@ -256,9 +288,10 @@ class Harness:
     def buf(self, t):
         return self.umfa.MFABuffer(self.ctx, device_ptr=t.data_ptr(), size=t.numel() * t.element_size())
 
-    def timed(self, enqueue, steps, warmup, load_seconds=0.6):
+    def timed(self, enqueue, steps, warmup, load_seconds=0.6, after_steps=None):
         """W warm-up steps, then exactly K steps between barrier + synchronize, CUDA events on the launching stream around
-        every step; returns (total ms = max over ranks, per-step ms list of this rank, clocks, launches)."""
+        every step; returns (total ms = max over ranks, per-step ms list of this rank, clocks, launches).  after_steps()
+        runs once the K steps are done, before anything else is enqueued."""
         torch = self.torch
         for i in range(warmup):
             enqueue(i)
@@ -277,6 +310,8 @@ class Harness:
         total_ms = evs[0].elapsed_time(evs[-1])
         per = [evs[i].elapsed_time(evs[i + 1]) for i in range(steps)]
         launches = self.ctx.launch_count - launches0
+        if after_steps is not None:
+            after_steps()
         # keep the GPU loaded a little longer so the clock sampler sees the steady state
         if self.rank == 0 and load_seconds > 0:
             t_end = time.time() + load_seconds
@@ -363,9 +398,10 @@ def attention_enqueue(hz, w, H, mode, sets, o_prec=2, mask=None):
     return enqueue
 
 
-def section_attention(hz, w, mode, steps, warmup, heads_sharded=False, o_dtype="fp32", dense_mask=False):
+def section_attention(hz, w, mode, steps, warmup, heads_sharded=False, o_dtype="fp32", dense_mask=False, dump_dir=None):
     """Dense attention section: weak replicas (every rank the whole workload) or -- heads_sharded -- the workload's heads
-    split over the ranks (strong scaling, no collective: heads are independent, MultiHeadAttention.swift:373-377)."""
+    split over the ranks (strong scaling, no collective: heads are independent, MultiHeadAttention.swift:373-377).
+    dump_dir: write the outputs of the last timed step there (write_outputs)."""
     import numpy as np
     H = w["H"]
     if heads_sharded:
@@ -379,7 +415,16 @@ def section_attention(hz, w, mode, steps, warmup, heads_sharded=False, o_dtype="
         g = hz.torch.Generator(device=hz.dev).manual_seed(99 + hz.rank)
         mask = hz.torch.randn(1, H, w["Sq"], w["Skv"], device=hz.dev, dtype=hz.torch.float32, generator=g).to(hz.torch.bfloat16)
     enqueue = attention_enqueue(hz, w, H, mode, sets, o_prec, mask)
-    total_ms, per, clocks, launches = hz.timed(enqueue, steps, warmup)
+    snap = {}
+
+    def keep_last_step():
+        ts = sets[(warmup + steps - 1) % len(sets)][0]
+        named = {"o": ts[3]} if mode == "fwd" else dict(zip(("o", "lse", "dq", "dk", "dv", "dterm"), ts[3:5] + ts[6:10]))
+        snap.update(sample_outputs(named))
+    total_ms, per, clocks, launches = hz.timed(enqueue, steps, warmup,
+                                               after_steps=keep_last_step if dump_dir and hz.rank == 0 else None)
+    if snap:
+        write_outputs(dump_dir, snap)
     kernel = hz.ctx.last_kernel
     per_rank_flops = fwd_flops(dict(w, H=H)) * (3.5 if mode == "fwdbwd" else 1.0)   # fwd 4, bwd 10 FLOP per pair per d
     job_flops = per_rank_flops * hz.world
@@ -508,8 +553,9 @@ def section_quant(hz, steps, warmup, target, label):
     return rec
 
 
-def section_ring(hz, w, steps, warmup, mode="fwd"):
-    """Config 5: causal ring attention over `world` GPUs, total sequence fixed (strong scaling)."""
+def section_ring(hz, w, steps, warmup, mode="fwd", dump_dir=None):
+    """Config 5: causal ring attention over `world` GPUs, total sequence fixed (strong scaling).
+    dump_dir: write this rank's outputs of the last timed step there (write_outputs), low and high chunk joined."""
     import numpy as np
     torch = hz.torch
     from umfa import ring
@@ -527,9 +573,10 @@ def section_ring(hz, w, steps, warmup, mode="fwd"):
     dop = (mk(), mk()) if fwdbwd else None
 
     def one_step():
-        runner.forward_packed(pk, scale)
+        res = {"o_l": runner.forward_packed(pk, scale)}
         if fwdbwd:
-            runner.backward_packed(pk, dop, scale)     # (synchronises the stream at its end: the gradients are returned)
+            res["grads"] = runner.backward_packed(pk, dop, scale)     # (synchronises the stream at its end: the gradients are returned)
+        return res
     for _ in range(warmup):
         one_step()
     hz.barrier()
@@ -541,9 +588,16 @@ def section_ring(hz, w, steps, warmup, mode="fwd"):
     hz.barrier()
     e0.record(hz.stream)
     for _ in range(steps):
-        one_step()
+        last = one_step()
     e1.record(hz.stream)
     hz.barrier()
+    if dump_dir and rank == 0:
+        join = lambda pair: torch.cat([torch.as_tensor(x, device=dev) for x in pair], dim=2)
+        (o_lo, l_lo), (o_hi, l_hi) = last["o_l"]
+        named = {"o": join((o_lo, o_hi)), "lse": join((l_lo, l_hi))}
+        if fwdbwd:
+            named.update(zip(("dq", "dk", "dv"), (join(g) for g in last["grads"])))
+        write_outputs(dump_dir, sample_outputs(named))
     ms = hz.max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     flops = (14.0 if fwdbwd else 4.0) * B * H * ring.visible_pairs_causal(N) * D      # fwd 4, bwd 10 FLOP per pair per d (FA convention)
@@ -619,6 +673,8 @@ def main():
                     help="all | none | comma list of " + ",".join(ALL_EXTRAS) + " (default: all for the headline workload, none otherwise)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the workload to DIR/<name>.npy (float32)")
     args = ap.parse_args()
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -626,6 +682,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", "1"))
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the CUDA path computed: use it with --impl ours")
         run_reference(args, w, rank)
         return
 
@@ -653,7 +711,7 @@ def main():
         extras = [x for x in args.extras.split(",") if x]
 
     if w.get("ring"):
-        rec = section_ring(hz, w, args.steps, args.warmup)
+        rec = section_ring(hz, w, args.steps, args.warmup, dump_dir=args.dump_outputs)
         if rank == 0:
             rec.update({"vs_baseline": None, "data": "synthetic", "e2e": None})
             print(json.dumps(rec), flush=True)
@@ -662,7 +720,8 @@ def main():
             dist.destroy_process_group()
         return
 
-    line, in_bytes, out_bytes, flops = section_attention(hz, w, args.mode, args.steps, args.warmup, o_dtype=args.o_dtype)
+    line, in_bytes, out_bytes, flops = section_attention(hz, w, args.mode, args.steps, args.warmup, o_dtype=args.o_dtype,
+                                                         dump_dir=args.dump_outputs)
     line.update({"vs_baseline": None, "data": "synthetic"})
     if args.mode == "fwd":
         tr, tnote = load_traffic(args.workload, line["config"]["kernel"], out_bytes + w["B"] * w["H"] * w["Sq"] * 4)

@@ -1,6 +1,7 @@
 """CPU tests of the boundary: the library loads, exports every symbol the headers declare, prototypes match the
 reference header, and the no-device error behaviour follows the reference bridge."""
 import ctypes
+import json
 import os
 import re
 import subprocess
@@ -10,7 +11,27 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 INCLUDE = os.path.join(ROOT, "include")
-REF_HEADER = "/root/reference/Sources/MFAFFI/include/mfa_ffi.h"
+# prototypes and probe output of the reference's Sources/MFAFFI/include/mfa_ffi.h (tests/golden/make_reference_abi.py)
+REF_ABI = os.path.join(ROOT, "tests", "golden", "reference_abi.json")
+PROBE = r'''
+#include <stdio.h>
+#include <stddef.h>
+#include HDR
+int main(void){
+  printf("%d %d %d %d %d %d\n", MFA_SUCCESS, MFA_ERROR_INVALID_ARGS, MFA_ERROR_MEMORY_ALLOCATION,
+         MFA_ERROR_DEVICE_NOT_SUPPORTED, MFA_ERROR_KERNEL_COMPILATION, MFA_ERROR_EXECUTION_FAILED);
+  printf("%d %d %d %d %d\n", MFA_PRECISION_FP16, MFA_PRECISION_BF16, MFA_PRECISION_FP32, MFA_PRECISION_INT8, MFA_PRECISION_INT4);
+  printf("%d %d %d | %d %d %d %d\n", MFA_MASK_TYPE_NONE, MFA_MASK_TYPE_BOOL, MFA_MASK_TYPE_ADDITIVE,
+         MFA_MASK_SCALAR_BYTE, MFA_MASK_SCALAR_FP16, MFA_MASK_SCALAR_BF16, MFA_MASK_SCALAR_FP32);
+  printf("%d %d %d\n", MFA_QUANT_KERNEL_FORWARD, MFA_QUANT_KERNEL_BACKWARD_QUERY, MFA_QUANT_KERNEL_BACKWARD_KEY_VALUE);
+  printf("%zu %zu %zu %zu %zu\n", sizeof(mfa_quantized_layout_t), offsetof(mfa_quantized_layout_t, qScale),
+         offsetof(mfa_quantized_layout_t, maskBuffer), offsetof(mfa_quantized_layout_t, scratch1),
+         offsetof(mfa_quantized_layout_t, qBlockScales));
+  printf("%zu %zu %zu\n", sizeof(mfa_quantized_capabilities_t), offsetof(mfa_quantized_capabilities_t, max_heads),
+         offsetof(mfa_quantized_capabilities_t, max_block_size));
+  printf("%zu %zu %zu %zu\n", sizeof(mfa_error_t), sizeof(mfa_precision_t), sizeof(mfa_context_t), sizeof(mfa_mla_context_t));
+  return 0; }
+'''
 
 
 def _lib():
@@ -59,45 +80,32 @@ def test_exports_only_mfa_symbols():
     assert names and all(n.startswith("mfa_") for n in names)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_HEADER), reason="reference checkout not present")
+def probe_output(header, tmp_dir):
+    """What PROBE prints when compiled against `header`: enum values, struct sizes and offsets."""
+    src = os.path.join(tmp_dir, "probe.c")
+    exe = os.path.join(tmp_dir, "probe")
+    with open(src, "w") as f:
+        f.write(PROBE)
+    subprocess.run(["/usr/bin/gcc", "-std=c11", f'-DHDR="{os.path.abspath(header)}"', src, "-o", exe], check=True)
+    return subprocess.run([exe], capture_output=True, text=True, check=True).stdout
+
+
+def _reference_abi():
+    with open(REF_ABI) as f:
+        return json.load(f)
+
+
 def test_header_matches_reference_prototypes():
     ours = _prototypes(open(os.path.join(INCLUDE, "mfa_ffi.h")).read())
-    ref = _prototypes(open(REF_HEADER).read())
+    ref = {name: (ret, tuple(args)) for name, (ret, args) in _reference_abi()["prototypes"].items()}
     assert set(ref) == set(ours)
     for name, proto in ref.items():
         assert ours[name] == proto, name
 
 
-@pytest.mark.skipif(not os.path.exists(REF_HEADER), reason="reference checkout not present")
 def test_header_enums_and_structs_match_reference(tmp_path):
-    """Compile the same probe against both headers and compare what it prints (enum values, struct sizes/offsets)."""
-    probe = r'''
-#include <stdio.h>
-#include <stddef.h>
-#include HDR
-int main(void){
-  printf("%d %d %d %d %d %d\n", MFA_SUCCESS, MFA_ERROR_INVALID_ARGS, MFA_ERROR_MEMORY_ALLOCATION,
-         MFA_ERROR_DEVICE_NOT_SUPPORTED, MFA_ERROR_KERNEL_COMPILATION, MFA_ERROR_EXECUTION_FAILED);
-  printf("%d %d %d %d %d\n", MFA_PRECISION_FP16, MFA_PRECISION_BF16, MFA_PRECISION_FP32, MFA_PRECISION_INT8, MFA_PRECISION_INT4);
-  printf("%d %d %d | %d %d %d %d\n", MFA_MASK_TYPE_NONE, MFA_MASK_TYPE_BOOL, MFA_MASK_TYPE_ADDITIVE,
-         MFA_MASK_SCALAR_BYTE, MFA_MASK_SCALAR_FP16, MFA_MASK_SCALAR_BF16, MFA_MASK_SCALAR_FP32);
-  printf("%d %d %d\n", MFA_QUANT_KERNEL_FORWARD, MFA_QUANT_KERNEL_BACKWARD_QUERY, MFA_QUANT_KERNEL_BACKWARD_KEY_VALUE);
-  printf("%zu %zu %zu %zu %zu\n", sizeof(mfa_quantized_layout_t), offsetof(mfa_quantized_layout_t, qScale),
-         offsetof(mfa_quantized_layout_t, maskBuffer), offsetof(mfa_quantized_layout_t, scratch1),
-         offsetof(mfa_quantized_layout_t, qBlockScales));
-  printf("%zu %zu %zu\n", sizeof(mfa_quantized_capabilities_t), offsetof(mfa_quantized_capabilities_t, max_heads),
-         offsetof(mfa_quantized_capabilities_t, max_block_size));
-  printf("%zu %zu %zu %zu\n", sizeof(mfa_error_t), sizeof(mfa_precision_t), sizeof(mfa_context_t), sizeof(mfa_mla_context_t));
-  return 0; }
-'''
-    src = tmp_path / "probe.c"
-    src.write_text(probe)
-    outs = []
-    for hdr in (os.path.join(INCLUDE, "mfa_ffi.h"), REF_HEADER):
-        exe = tmp_path / ("p_" + str(len(outs)))
-        subprocess.run(["/usr/bin/gcc", "-std=c11", f'-DHDR="{hdr}"', str(src), "-o", str(exe)], check=True)
-        outs.append(subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout)
-    assert outs[0] == outs[1]
+    """Compile the probe against our header and compare what it prints with the reference header's output."""
+    assert probe_output(os.path.join(INCLUDE, "mfa_ffi.h"), str(tmp_path)) == _reference_abi()["probe"]
 
 
 def test_headers_compile_as_c_and_cxx(tmp_path):
