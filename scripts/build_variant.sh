@@ -2,7 +2,7 @@
 # Experiment builds of one kernel file (default: the forward, csrc/attn_fwd_tc.cu; VARIANT_SRC=attn_bwd_tc for another): compiles
 # it with extra -D flags and links it with the other objects of the current library into lib_variants/<name>/libMFAFFI.so
 # (select with MFA_LIBRARY=...).
-#   scripts/build_variant.sh nostage -DMFA_FWD_NOSTAGE
+#   VARIANT_SRC=attn_bwd_tc scripts/build_variant.sh bwd_ra2_rb2 -DMFA_BWD_RA=2 -DMFA_BWD_RB=2
 set -e
 NAME=$1; shift
 HERE=$(cd "$(dirname "$0")/.." && pwd)

@@ -233,7 +233,7 @@ int main(void) {
     assert r.returncode == 0 and "c consumer ok" in r.stdout, (r.returncode, r.stdout, r.stderr)
 
 
-def test_headline_forward_kernels_do_not_spill():
+def test_headline_forward_instantiations_do_not_spill():
     """The unmasked bf16 / fp16 / fp32-split / int8 forward instantiations must keep O and S in registers: a stack frame in them
     cost 6 % of the headline number once (an epilogue branch indexed the O registers dynamically; round 2)."""
     import re
@@ -244,16 +244,16 @@ def test_headline_forward_kernels_do_not_spill():
     if not os.path.exists(cuobjdump) or not os.path.exists(obj):
         pytest.skip("cuobjdump or the object file is not available")
     out = subprocess.run([cuobjdump, "-res-usage", obj], capture_output=True, text=True).stdout
-    seen = 0
-    for m in re.finditer(r"Function (\S*fwd_tc_kernelILi(\d+)ELi(\d+)ELi(\d+)ELb0ELi0E\S*):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
-        mode, stack = int(m.group(3)), int(m.group(6))
+    seen = set()
+    for m in re.finditer(r"Function (\S*fwd_tc_kernelILi(\d+)ELi(\d+)ELi0E\S*):\s*\n\s*REG:(\d+) STACK:(\d+)", out):
+        d, mode, stack = int(m.group(2)), int(m.group(3)), int(m.group(5))
         if mode in (0, 1, 3, 4, 8):          # f16, bf16, int8 + e4m3, fp32 split, wide bf16
-            seen += 1
+            seen.add((d, mode))
             assert stack == 0, (m.group(1), stack)
-    assert seen >= 8
+    assert seen == {(64, 0), (128, 0), (64, 1), (128, 1), (128, 3), (128, 4), (128, 8)}, seen
 
 
-def test_staged_mask_kernels_exist_and_do_not_spill():
+def test_staged_mask_instantiations_exist_and_do_not_spill():
     """The instantiations that stage external-mask tiles in shared memory (MASKED = 2: forward bf16 / fp16 at both head-dim
     widths, both backward kernels) are in the library and keep their working set in registers."""
     import re
@@ -265,8 +265,8 @@ def test_staged_mask_kernels_exist_and_do_not_spill():
         pytest.skip("cuobjdump or the object files are not available")
     fwd = subprocess.run([cuobjdump, "-res-usage", os.path.join(lib_dir, "attn_fwd_tc.o")], capture_output=True, text=True).stdout
     seen = set()
-    for m in re.finditer(r"Function \S*fwd_tc_kernelILi(\d+)ELi([01])ELi(\d+)ELb0ELi2E\S*:\s*\n\s*REG:(\d+) STACK:(\d+)", fwd):
-        assert int(m.group(5)) == 0, m.group(0)
+    for m in re.finditer(r"Function \S*fwd_tc_kernelILi(\d+)ELi([01])ELi2E\S*:\s*\n\s*REG:(\d+) STACK:(\d+)", fwd):
+        assert int(m.group(4)) == 0, m.group(0)
         seen.add((int(m.group(1)), int(m.group(2))))
     assert seen == {(64, 0), (64, 1), (128, 0), (128, 1)}
     bwd = subprocess.run([cuobjdump, "-res-usage", os.path.join(lib_dir, "attn_bwd_tc.o")], capture_output=True, text=True).stdout

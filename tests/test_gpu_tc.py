@@ -367,33 +367,6 @@ def test_tc_mask_tile_skipping_saves_time(ctx, monkeypatch):
     assert t_skip < 0.7 * t_all, f"skip {t_skip * 1e3:.3f} ms vs all tiles {t_all * 1e3:.3f} ms"
 
 
-def test_tc_persistent_grid_matches_oracle():
-    """MFA_FWD_PERSIST=1 (opt-in): one CTA per SM strides over the work items -- barrier phases, Q reload hand-shake and
-    the O hand-back carry across items.  Read once per process, hence a fresh interpreter."""
-    import os, subprocess, sys
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = r'''
-import sys, numpy as np
-sys.path.insert(0, "ROOT"); sys.path.insert(0, "ROOT/universal-metal-flash-attention_b200")
-import umfa
-from oracle import oracle as O
-rng = np.random.default_rng(5)
-ctx = umfa.MFAContext()
-for (B, H, Sq, Skv, D) in ((2, 40, 1100, 700, 128), (1, 96, 600, 300, 64)):      # > 148 items, ragged last query block
-    q, k, v = (rng.standard_normal(s).astype(np.float32) for s in ((B, H, Sq, D), (B, H, Skv, D), (B, H, Skv, D)))
-    (qv, qb), (kv, kb), (vv, vb) = (O.round_bf16(x) for x in (q, k, v))
-    out, lse = umfa.flash_attention_forward(ctx, qb, kb, vb, input_precision="bf16", output_precision="fp32", layout="bhsd", return_lse=True)
-    assert ctx.last_kernel.startswith("fwd_tc_"), ctx.last_kernel
-    ref, lref = O.attention_forward(qv, kv, vv)
-    err = float(np.abs(out - ref).max() / np.abs(ref).max())
-    assert err < 2e-2 and np.abs(lse - lref).max() < 2e-2, (err,)
-print("persistent ok")
-'''.replace("ROOT", root)
-    env = dict(os.environ, MFA_FWD_PERSIST="1")
-    r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "persistent ok" in r.stdout, r.stdout + r.stderr
-
-
 @pytest.mark.parametrize("shape", [(1, 2, 256, 256, 128), (2, 3, 300, 777, 128), (1, 2, 1000, 130, 64), (1, 1, 77, 515, 64)])
 @pytest.mark.parametrize("causal", [False, True])
 def test_tc_fp16_output_tma_store(ctx, shape, causal):

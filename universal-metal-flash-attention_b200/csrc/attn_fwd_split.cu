@@ -31,16 +31,7 @@ namespace mfa {
 namespace {
 
 constexpr float kLog2e = 1.4426950408889634f;
-// keys per accumulator lifetime (see launch_fwd_split); MFA_FP32_SLICE_KEYS overrides it (a multiple of 128; 0 = no flush)
-int slice_keys() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("MFA_FP32_SLICE_KEYS");
-    v = e ? atoi(e) : 768;
-    if (v < 0 || (v & 127)) v = 768;
-  }
-  return v;
-}
+constexpr int kSliceKeys = 768;       // keys per accumulator lifetime (a multiple of 128, see launch_fwd_split)
 
 struct SplitView {
   const float* src;
@@ -168,9 +159,9 @@ bool fwd_split_eligible(const AttnParams& p) {
 // scratch: (hi, lo) fp16 copies of Q, K, V + three abs-max words + three inverse scales
 size_t fwd_split_scratch_bytes(const AttnParams& p) {
   const size_t nq = (size_t)p.B * p.H * p.Sq * p.D, nkv = (size_t)p.B * p.Hkv * p.Skv * p.D;
-  // + the running L of launch-wise slices, + the flush tiles of the in-kernel slices (128 KB per 256-row work item)
+  // + the flush tiles of the key slices (128 KB per 256-row work item)
   const size_t items = (size_t)((p.Sq + 255) / 256) * p.H * p.B;
-  return pad256(nq * 4) + 2 * pad256(nkv * 4) + 512 + pad256((size_t)p.B * p.H * p.Sq * 4) + items * 2 * 128 * 128 * 4 + 256;
+  return pad256(nq * 4) + 2 * pad256(nkv * 4) + 512 + items * 2 * 128 * 128 * 4 + 256;
 }
 
 cudaError_t launch_fwd_split(const AttnParams& p, void* scratch, cudaStream_t st) {
@@ -181,8 +172,6 @@ cudaError_t launch_fwd_split(const AttnParams& p, void* scratch, cudaStream_t st
   __half* vh = reinterpret_cast<__half*>(sc + pad256(nq * 4) + pad256(nkv * 4));
   unsigned int* amax = reinterpret_cast<unsigned int*>(sc + pad256(nq * 4) + 2 * pad256(nkv * 4));
   float* inv = reinterpret_cast<float*>(amax + 8);
-  // running L of the key slices: the caller's L buffer, else scratch behind the scales
-  float* slice_lse = p.lse ? p.lse : reinterpret_cast<float*>(sc + pad256(nq * 4) + 2 * pad256(nkv * 4) + 512);
   cudaError_t e = cudaMemsetAsync(amax, 0, 32, st);
   if (e != cudaSuccess) return e;
   const TensorView* src[3] = {&p.q, &p.k, &p.v};
@@ -227,43 +216,23 @@ cudaError_t launch_fwd_split(const AttnParams& p, void* scratch, cudaStream_t st
   prm.dv = p.D;
   prm.c = p.scale * kLog2e;
   prm.causal = p.causal; prm.window = p.window;
-  prm.pingpong = fwd_tc_pingpong();
   prm.qs = inv; prm.ks = inv + 1; prm.vs = inv + 2;          // inverse power-of-two scales, read by the softmax warps
   fwd_tc_set_out_map(prm, p);
   fwd_tc_set_mask(prm, p);
-  // Long key ranges run as slices of kSliceKeys keys, one launch each, merged in fp32 by the accumulate epilogue (the one ring
-  // attention uses).  Why: tcgen05 adds every MMA into the TMEM accumulator with truncation, a bias of ~2^-24 of the accumulator
-  // per MMA; O collects 24 MMAs per KV step, so one launch over N keys carries a relative error of N * 4e-9 (zero-mean V) to
-  // N * 9e-9 (same-sign V, the accumulator grows monotonically): 1.7e-5 .. 4.2e-5 at 4608 keys -- beyond the 1e-5 this path
-  // promises.  Slices of 768 keys keep the worst case at ~7e-6 (2048: 1.7e-5, 1024: ~9e-6; tests/test_gpu_fp32_tc.py).
-  // Two ways to bound the accumulator's lifetime: the kernel hands O over to its fp32 output row every kSliceKeys / 128 steps
-  // (default: one launch, no re-read of Q, no extra prologues), or -- MFA_FP32_SLICE_LAUNCHES=1, the first implementation, kept
-  // for A/B -- one launch per slice merged by the accumulate epilogue.
-  const int kSliceKeys = slice_keys();
-  const bool by_launch = getenv("MFA_FP32_SLICE_LAUNCHES") != nullptr;
-  if (!by_launch && kSliceKeys > 0 && !p.accumulate && p.Skv > kSliceKeys) {
+  // Long key ranges run as slices of kSliceKeys keys.  Why: tcgen05 adds every MMA into the TMEM accumulator with truncation, a
+  // bias of ~2^-24 of the accumulator per MMA; O collects 24 MMAs per KV step, so one accumulator over N keys carries a relative
+  // error of N * 4e-9 (zero-mean V) to N * 9e-9 (same-sign V, the accumulator grows monotonically): 1.7e-5 .. 4.2e-5 at 4608
+  // keys -- beyond the 1e-5 this path promises.  Slices of 768 keys keep the worst case at ~7e-6 (2048: 1.7e-5, 1024: ~9e-6;
+  // tests/test_gpu_fp32_tc.py).  The kernel hands O over to an fp32 scratch tile every kSliceKeys / 128 steps (one launch, no
+  // re-read of Q, no extra prologues).
+  if (!p.accumulate && p.Skv > kSliceKeys) {
     prm.flush_steps = kSliceKeys / 128;
-    prm.flush_buf = reinterpret_cast<float*>(sc + pad256(nq * 4) + 2 * pad256(nkv * 4) + 512 + pad256((size_t)p.B * p.H * p.Sq * 4));
+    prm.flush_buf = reinterpret_cast<float*>(sc + pad256(nq * 4) + 2 * pad256(nkv * 4) + 512);
   }
-  const int n_slices = (by_launch && kSliceKeys > 0 && p.o_dtype == kF32 && !p.accumulate && slice_lse) ? (p.Skv + kSliceKeys - 1) / kSliceKeys : 1;
-  if (n_slices <= 1) {
-    if ((e = fwd_tc_build_mask_tiles(prm, p, st)) != cudaSuccess) return e;
-    e = launch_fwd_tc_kernel(prm, 128, kFwdSplit, st, p.B);
-    if (e != cudaSuccess) return e;
-    ++g_launch_count;
-  } else {
-    prm.mtiles = nullptr; prm.mcounts = nullptr; prm.m_nkt = 0;       // slices walk their own key range (masks are read in place)
-    prm.lse = slice_lse;
-    prm.lse_sh = p.lse ? prm.lse_sh : p.Sq;
-    for (int i = 0; i < n_slices; ++i) {
-      prm.kv_begin = i * kSliceKeys;
-      prm.kv_end = min(p.Skv, (i + 1) * kSliceKeys);
-      if (i == 1) { prm.accumulate = 1; prm.o_tma = 0; }
-      e = launch_fwd_tc_kernel(prm, 128, kFwdSplit, st, p.B);
-      if (e != cudaSuccess) return e;
-      ++g_launch_count;
-    }
-  }
+  if ((e = fwd_tc_build_mask_tiles(prm, p, st)) != cudaSuccess) return e;
+  e = launch_fwd_tc_kernel(prm, 128, kFwdSplit, st, p.B);
+  if (e != cudaSuccess) return e;
+  ++g_launch_count;
   g_last_kernel = prm.mask ? "fwd_tc_fp32split_d128_mask" : "fwd_tc_fp32split_d128";
   return cudaGetLastError();
 }

@@ -33,7 +33,6 @@
 #include <cuda_fp16.h>
 #include <math_constants.h>
 
-#include <cstdio>
 #include <mutex>
 #include <type_traits>
 
@@ -78,14 +77,12 @@ struct Cfg {
   static constexpr bool kMaskTma = MASKED == 2 && (MODE == kFwdF16 || MODE == kFwdBF16);
   static constexpr int kMaskTile = 128 * 128 * 2;                    // one query tile x 128 keys of 16-bit terms (bool bytes use half)
   static constexpr bool kShallow = MASKED != 0 && !kI4;
-#ifdef MFA_FORCE_NS3                                                 // experiment: the unmasked kernel on the shallow ring
-  static constexpr int kDeep = 3;
-#else
-  static constexpr int kDeep = 5;
-#endif
   static constexpr int kStages = (kSplit || kWide) ? 3               // split / wide: 2 x 64 KB of Q leave room for 3 x 32 KB
-                               : (D == 128 && !kF8) ? (kShallow ? 3 : kDeep) : (kShallow ? 6 : 10);
-  static constexpr int kBarBytes = 112 + 16 * kStages + 16 + 32 + 64 + 32; // + q_empty, o_empty, + raw-tile barriers (int4), + mask tile barriers
+                               : (D == 128 && !kF8) ? (kShallow ? 3 : 5) : (kShallow ? 6 : 10);
+  static constexpr int kBarBytes = 112 + 16 * kStages + 16 + 16 + 64 + 32; // + TMEM slot, o_empty, + raw-tile barriers (int4), + mask tile barriers
+  // element pairs of every 8 whose exp2 runs on the FMA pipe (exp2_poly2) instead of MUFU.EX2; the fp32 split mode keeps exact
+  // exp2 only (the polynomial's 8.6e-5 would show at fp32 tolerances)
+  static constexpr int kPoly = kSplit ? 0 : 3;
   // int4: raw (packed) tiles as TMA delivers them -- a 3-deep ring of K tiles + one Q tile, 128 rows x 64 bytes each -- and
   // the per-row sums of the Q codes (2 x 128 ints)
   static constexpr int kRawTile = 128 * 64, kRawStages = 3;
@@ -123,14 +120,15 @@ __device__ __forceinline__ f32x2 exp2_poly2(f32x2 x) {
 // in a packed register.  NP of every 8 element pairs take the polynomial (compile-time pattern, so the loop body is branch-free).
 template <int PF, int NP>
 __device__ __forceinline__ void exp_part(const float* s, f32x2 a2, f32x2 nk2, uint32_t* pk, f32x2& acc_a, f32x2& acc_b) {
-  constexpr int kSel[5] = {0x00, 0x08, 0x22, 0x52, 0xAA};
+  static_assert(NP == 0 || NP == 3, "exp2 mixes: all MUFU, or pairs 1, 4, 6 of every 8 on the polynomial");
+  constexpr int kSel = NP == 3 ? 0x52 : 0x00;
   uint32_t half16[PF == 2 ? 16 : 1];
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
     const f32x2 x = fma2(pack2(s[2 * i], s[2 * i + 1]), a2, nk2);
     f32x2 pp;
     float p0, p1;
-    if ((kSel[NP] >> (i & 7)) & 1) {
+    if ((kSel >> (i & 7)) & 1) {
       pp = exp2_poly2(x);
     } else {
       float x0, x1;
@@ -158,9 +156,9 @@ __device__ __forceinline__ void exp_part(const float* s, f32x2 a2, f32x2 nk2, ui
 // of arithmetic later (so tcgen05.wait::st never stalls on the store just issued).  One straight-line block: ptxas
 // interleaves the MUFU and polynomial work of neighbouring parts.  Sums of the two 64-key halves are kept apart
 // (int8 mode folds the V block scale of each half into its exponent).
-template <int PF, int NP, bool TR>
+template <int PF, int NP>
 __device__ __forceinline__ void exp_phase(const float* s, float a0, float a1, float nk0, float nk1, uint32_t tS,
-                                          uint32_t bar0, int lane, float& sum_lo, float& sum_hi, unsigned long long* tr) {
+                                          uint32_t bar0, int lane, float& sum_lo, float& sum_hi) {
   constexpr int kW = PF == 2 ? 8 : 16;             // TMEM columns of one part
   f32x2 acc[2][2] = {{pack2(0.f, 0.f), pack2(0.f, 0.f)}, {pack2(0.f, 0.f), pack2(0.f, 0.f)}};
   uint32_t pk[kParts][PF == 3 ? 32 : kW];
@@ -174,7 +172,6 @@ __device__ __forceinline__ void exp_phase(const float* s, float a0, float a1, fl
       tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(bar0 + 8 * (part - 1));
-      if (TR && tr) tr[3 + part - 1] = clock64();
     }
     if constexpr (PF == 2) tmem_st_x8(tS + kW * part, pk[part]);
     else tmem_st_x16(tS + kW * part, pk[part]);
@@ -184,7 +181,6 @@ __device__ __forceinline__ void exp_phase(const float* s, float a0, float a1, fl
   tc_fence_before();
   __syncwarp();
   if (lane == 0) mbar_arrive(bar0 + 8 * (kParts - 1));
-  if (TR && tr) tr[3 + kParts - 1] = clock64();
   float x0, x1;
   unpack2(add2(acc[0][0], acc[0][1]), x0, x1); sum_lo = x0 + x1;
   unpack2(add2(acc[1][0], acc[1][1]), x0, x1); sum_hi = x0 + x1;
@@ -207,12 +203,12 @@ __device__ __forceinline__ void add_mask_pair(float& s0, float& s1, uint32_t w, 
   unpack2(fma2(pack2(s0, s1), cn2, pack2(lo, hi)), s0, s1);
 }
 
-// POLY = n in 0..4: n of every 8 element pairs go through exp2_poly2 instead of MUFU.EX2 (on masked tiles too: the polynomial
+// Cfg::kPoly of every 8 element pairs go through exp2_poly2 instead of MUFU.EX2 (on masked tiles too: the polynomial
 // returns an exact zero for hidden elements, see its clamp).
 // MASKED: an external mask (bool or additive, SURVEY A4 with the PyTorch placement softmax(scale * QK^T + mask)) is read by
 // the softmax warps straight from global memory -- each thread owns one row, so it reads the 128 mask values of its row
 // and tile with 32-byte (one sector) loads; no dense fp32 expansion pass like the reference's mfa_prepare_mask (MFABridge.swift:153-243).
-template <int D, int MODE, int POLY, bool TR = false, int MASKED = 0>      // MASKED: 0 none, 1 read in place, 2 staged by TMA
+template <int D, int MODE, int MASKED>      // MASKED: 0 none, 1 read in place, 2 staged by TMA
 __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_constant__ FwdTcParams p) {
   using C = Cfg<D, MODE, MASKED>;
   constexpr bool I8 = C::kI8, F8 = C::kF8, SPLIT = C::kSplit, I4 = C::kI4, WIDE = C::kWide, MT = C::kMaskTma;
@@ -235,31 +231,23 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
   auto kv_full = [&](int s) { return sBar + 112 + 8 * s; };
   auto kv_empty = [&](int s) { return sBar + 112 + 8 * NS + 8 * s; };
   const uint32_t tmem_slot = sBar + 112 + 16 * NS;
-  auto q_empty = [&](int t) { return sBar + 112 + 16 * NS + 16 + 8 * t; };   // MMA warp: Q_t smem may be reloaded
-  auto o_empty = [&](int t) { return sBar + 112 + 16 * NS + 32 + 8 * t; };   // softmax warps: O_t left TMEM (epilogue read it)
+  auto o_empty = [&](int t) { return sBar + 112 + 16 * NS + 16 + 8 * t; };   // softmax warps: O_t left TMEM (fp32 split flush)
   // int4 operands: raw_full / raw_empty of the packed K ring, qraw_full / qraw_empty of the packed Q tile
   constexpr int NR = C::kRawStages, RAW = C::kRawTile;
-  auto raw_full = [&](int s) { return sBar + 112 + 16 * NS + 48 + 8 * s; };
-  auto raw_empty = [&](int s) { return sBar + 112 + 16 * NS + 72 + 8 * s; };
-  const uint32_t qraw_full = sBar + 112 + 16 * NS + 96, qraw_empty = sBar + 112 + 16 * NS + 104;
+  auto raw_full = [&](int s) { return sBar + 112 + 16 * NS + 32 + 8 * s; };
+  auto raw_empty = [&](int s) { return sBar + 112 + 16 * NS + 56 + 8 * s; };
+  const uint32_t qraw_full = sBar + 112 + 16 * NS + 80, qraw_empty = sBar + 112 + 16 * NS + 88;
   const uint32_t sRawK = (sBar + C::kBarBytes + 127u) & ~127u, sRawQ = sRawK + NR * RAW, sQsum = sRawQ + RAW;
   // staged external mask (MT): one 128 x 128 tile per query tile, 128-byte swizzled like the operand tiles
-  auto mk_full = [&](int t) { return sBar + 112 + 16 * NS + 112 + 8 * t; };
-  auto mk_empty = [&](int t) { return sBar + 112 + 16 * NS + 128 + 8 * t; };
+  auto mk_full = [&](int t) { return sBar + 112 + 16 * NS + 96 + 8 * t; };
+  auto mk_empty = [&](int t) { return sBar + 112 + 16 * NS + 112 + 8 * t; };
   const uint32_t sMask = (sBar + C::kBarBytes + 1023u) & ~1023u;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for ptxas
-  // MFA_FWD_CTATRACE (debug build of the launch only): per-CTA wall-clock stamps written by thread 0
-  unsigned long long* ct = nullptr;
-  if constexpr (TR) { if (p.cta_trace && threadIdx.x == 0) { ct = p.cta_trace + (size_t)blockIdx.x * 16; ct[0] = globaltimer_ns(); ct[7] = clock64(); ct[6] = smid(); } }
-  // Work items = (batch, head, 256-row query block), x fastest so the CTAs of one head run together (K/V stay in L2).
-  // The grid is either one CTA per item or -- persistent mode, uniform-cost problems -- one CTA per SM striding over the
-  // items: the producer then prefetches the next item's Q/K/V and the MMA warps start its first S while the softmax warps
-  // are still in the epilogue of the previous one, so the per-item prologue / epilogue latency is hidden.
-  const int nqb = (p.Sq + 255) / 256;
-  const int n_items = nqb * p.H * p.nbatch * (WIDE ? 2 : 1);
+  // One CTA per work item = (batch, head, 256-row query block), x fastest so the CTAs of one head run together (K/V stay in L2).
   struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half; };
   auto decode = [&](int w) {
+    const int nqb = (p.Sq + 255) / 256;
     Item it;
     it.half = 0;
     if constexpr (WIDE) { it.half = w & 1; w >>= 1; }           // the two O halves of a query block run next to each other
@@ -271,7 +259,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     it.nt = (it.r0 + 128 < p.Sq) ? 2 : 1;
     int klo, khi;
     visible_key_range(p.causal, p.window, p.Skv, it.r0, min(it.r0 + 256, p.Sq), klo, khi);
-    if (p.kv_end > 0) { klo = max(klo, p.kv_begin); khi = max(klo, min(khi, p.kv_end)); }      // this launch covers a slice of the keys
     it.j_lo = klo >> 7;
     it.n = khi > klo ? ((khi + 127) >> 7) - it.j_lo : 0;
     it.lid = 0;
@@ -295,7 +282,7 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
       for (int k = 0; k < kParts; ++k) mbar_init(p_part(t, k), 4);
     }
     for (int s = 0; s < NS; ++s) { mbar_init(kv_full(s), 1); mbar_init(kv_empty(s), 2); }   // a lone tile releases twice
-    for (int t = 0; t < 2; ++t) { mbar_init(q_empty(t), 1); mbar_init(o_empty(t), 4); }
+    for (int t = 0; t < 2; ++t) mbar_init(o_empty(t), 4);
     if constexpr (I4) {
       for (int r = 0; r < NR; ++r) { mbar_init(raw_full(r), 1); mbar_init(raw_empty(r), 1); }
       mbar_init(qraw_full, 1); mbar_init(qraw_empty, 1);
@@ -315,74 +302,65 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw)), 0);
-  if (TR && ct) ct[1] = globaltimer_ns();
 
   if (warp == 9) {
     // ------------------------------------------------------------------ TMA producer
     reg_dealloc<kWg2Regs>();
     if (lane == 0) {
-      int kvi = 0, qc[2] = {0, 0};                      // running ring index; items in which tile t took part
+      const Item im = decode(blockIdx.x);
+      const int r0 = im.r0, h = im.h, b = im.b, hk = im.hk, nt = im.nt, n = im.n;
+      int kvi = 0;                                      // running ring index
       int kr = 0, nqraw = 0;                            // int4: packed K / Q tiles requested so far
-      for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-        const Item im = decode(w);
-        const int r0 = im.r0, h = im.h, b = im.b, hk = im.hk, nt = im.nt, n = im.n;
-        if (n == 0) continue;
-        // one Q / K tile (or one hi / lo half of a split tile); the caller has armed the barrier with the bytes
-        auto load_half = [&](uint32_t dst, const CUtensorMap* m, uint32_t bar, int row, int head, int col0 = 0) {
+      // one Q / K tile (or one hi / lo half of a split tile); the caller has armed the barrier with the bytes
+      auto load_half = [&](uint32_t dst, const CUtensorMap* m, uint32_t bar, int row, int head, int col0 = 0) {
 #pragma unroll
-          for (int c = 0; c < C::kQChunks; ++c) tma_load_4d(dst + c * CHB, m, bar, col0 + c * (I8 ? 128 : 64), row, head, b);
-        };
-        auto load_q = [&](int t2) {
-          if constexpr (I4) {              // packed tile into the raw Q buffer; the converter warp unpacks it into sQ
-            if (nqraw > 0) mbar_wait(qraw_empty, (nqraw - 1) & 1);
-            mbar_arrive_expect_tx(qraw_full, RAW);
-            tma_load_4d(sRawQ, &p.tq, qraw_full, 0, r0 + t2 * 128, h, b);
-            ++nqraw;
-            return;
-          }
-          if (qc[t2] > 0) mbar_wait(q_empty(t2), (qc[t2] - 1) & 1);
-          mbar_arrive_expect_tx(q_full(t2), QT);
-          load_half(sQ + t2 * QT, &p.tq, q_full(t2), r0 + t2 * 128, h);
-          if constexpr (SPLIT) load_half(sQ + t2 * QT + HT, &p.tq2, q_full(t2), r0 + t2 * 128, h);
-          if constexpr (WIDE) load_half(sQ + t2 * QT + HT, &p.tq, q_full(t2), r0 + t2 * 128, h, 128);
-        };
-        auto load_k = [&](const CUtensorMap* m, int row, int col0 = 0) {
-          if constexpr (I4) {              // packed tile into the raw ring; its operand stage (ring index kvi) is the converter's
-            const int rs = kr % NR;
-            mbar_wait(raw_empty(rs), ((kr / NR) & 1) ^ 1);
-            mbar_arrive_expect_tx(raw_full(rs), RAW);
-            tma_load_4d(sRawK + rs * RAW, m, raw_full(rs), 0, row, hk, b);
-            ++kr; ++kvi;
-            return;
-          }
-          const int s = kvi % NS;
-          mbar_wait(kv_empty(s), ((kvi / NS) & 1) ^ 1);
-          mbar_arrive_expect_tx(kv_full(s), HT);
-          load_half(sKV + s * STG, m, kv_full(s), row, hk, col0);
-          ++kvi;
-        };
-        auto load_v = [&](const CUtensorMap* m, int row, int col0 = 0) {
-          const int s = kvi % NS;
-          mbar_wait(kv_empty(s), ((kvi / NS) & 1) ^ 1);
-          mbar_arrive_expect_tx(kv_full(s), VT);
-#pragma unroll
-          for (int c = 0; c < C::kVChunks; ++c) tma_load_4d(sKV + s * STG + c * CHB, m, kv_full(s), col0 + c * 64, row, hk, b);
-          ++kvi;
-        };
-        load_q(0);
-        ++qc[0];
-        for (int it = 0; it < n; ++it) {
-          const int row = (tile_of(im, it) & (kTileNoMask - 1)) * 128;
-          if constexpr (SPLIT) load_k(&p.tk2, row);         // K_lo first: its stage is released after the first MMA group
-          load_k(&p.tk, row);
-          if constexpr (WIDE) load_k(&p.tk, row, 128);      // K_b: head dims 128 .. 255
-          if (it == 0 && nt == 2) {
-            load_q(1);
-            ++qc[1];
-          }
-          load_v(&p.tv, row, WIDE ? 128 * im.half : 0);
-          if constexpr (SPLIT) load_v(&p.tv2, row);         // V_lo last: only the closing MMA group of the step reads it
+        for (int c = 0; c < C::kQChunks; ++c) tma_load_4d(dst + c * CHB, m, bar, col0 + c * (I8 ? 128 : 64), row, head, b);
+      };
+      auto load_q = [&](int t2) {
+        if constexpr (I4) {              // packed tile into the raw Q buffer; the converter warp unpacks it into sQ
+          if (nqraw > 0) mbar_wait(qraw_empty, (nqraw - 1) & 1);
+          mbar_arrive_expect_tx(qraw_full, RAW);
+          tma_load_4d(sRawQ, &p.tq, qraw_full, 0, r0 + t2 * 128, h, b);
+          ++nqraw;
+          return;
         }
+        mbar_arrive_expect_tx(q_full(t2), QT);
+        load_half(sQ + t2 * QT, &p.tq, q_full(t2), r0 + t2 * 128, h);
+        if constexpr (SPLIT) load_half(sQ + t2 * QT + HT, &p.tq2, q_full(t2), r0 + t2 * 128, h);
+        if constexpr (WIDE) load_half(sQ + t2 * QT + HT, &p.tq, q_full(t2), r0 + t2 * 128, h, 128);
+      };
+      auto load_k = [&](const CUtensorMap* m, int row, int col0 = 0) {
+        if constexpr (I4) {              // packed tile into the raw ring; its operand stage (ring index kvi) is the converter's
+          const int rs = kr % NR;
+          mbar_wait(raw_empty(rs), ((kr / NR) & 1) ^ 1);
+          mbar_arrive_expect_tx(raw_full(rs), RAW);
+          tma_load_4d(sRawK + rs * RAW, m, raw_full(rs), 0, row, hk, b);
+          ++kr; ++kvi;
+          return;
+        }
+        const int s = kvi % NS;
+        mbar_wait(kv_empty(s), ((kvi / NS) & 1) ^ 1);
+        mbar_arrive_expect_tx(kv_full(s), HT);
+        load_half(sKV + s * STG, m, kv_full(s), row, hk, col0);
+        ++kvi;
+      };
+      auto load_v = [&](const CUtensorMap* m, int row, int col0 = 0) {
+        const int s = kvi % NS;
+        mbar_wait(kv_empty(s), ((kvi / NS) & 1) ^ 1);
+        mbar_arrive_expect_tx(kv_full(s), VT);
+#pragma unroll
+        for (int c = 0; c < C::kVChunks; ++c) tma_load_4d(sKV + s * STG + c * CHB, m, kv_full(s), col0 + c * 64, row, hk, b);
+        ++kvi;
+      };
+      if (n > 0) load_q(0);
+      for (int it = 0; it < n; ++it) {
+        const int row = (tile_of(im, it) & (kTileNoMask - 1)) * 128;
+        if constexpr (SPLIT) load_k(&p.tk2, row);         // K_lo first: its stage is released after the first MMA group
+        load_k(&p.tk, row);
+        if constexpr (WIDE) load_k(&p.tk, row, 128);      // K_b: head dims 128 .. 255
+        if (it == 0 && nt == 2) load_q(1);
+        load_v(&p.tv, row, WIDE ? 128 * im.half : 0);
+        if constexpr (SPLIT) load_v(&p.tv2, row);         // V_lo last: only the closing MMA group of the step reads it
       }
     }
   } else if (warp == 8 || warp == 10) {
@@ -430,84 +408,69 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         }
       }
     };
-    int kvbase = 0, qc = 0, pc = 0;                // ring index at the start of the item; items / KV steps done by this tile
-    int oe = 0;                                    // o_empty phases consumed: one per O hand-over (flush or end of item)
+    int pc = 0;                                    // KV steps done by this tile
+    int oe = 0;                                    // o_empty phases consumed: one per O hand-over (flush)
     const int F = SPLIT ? p.flush_steps : 0;       // fp32 split mode: O leaves TMEM every F steps (see the softmax warps)
-    for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-      const Item im = decode(w);
-      const int nt = im.nt, n = im.n;
-      if (n > 0 && t < nt) {
-        // a lone tile (ragged last query block) releases every ring stage for the absent one as well
-        auto release = [&](int idx) { tc_commit_u(kv_empty(idx % NS)); if (nt == 1) tc_commit_u(kv_empty(idx % NS)); };
-        // all of S of the step whose stages start at ring index idx: wait for the K stages, issue, publish S, free the stages
-        auto do_s = [&](int idx) {
-          wait_full(idx);
+    const Item im = decode(blockIdx.x);
+    const int nt = im.nt, n = im.n;
+    if (n > 0 && t < nt) {
+      // a lone tile (ragged last query block) releases every ring stage for the absent one as well
+      auto release = [&](int idx) { tc_commit_u(kv_empty(idx % NS)); if (nt == 1) tc_commit_u(kv_empty(idx % NS)); };
+      // all of S of the step whose stages start at ring index idx: wait for the K stages, issue, publish S, free the stages
+      auto do_s = [&](int idx) {
+        wait_full(idx);
+        tc_fence_after();
+        if constexpr (SPLIT) {
+          issue_qk(q_lo, idx, false);                  // Q_hi K_lo^T
+          release(idx);
+          wait_full(idx + 1);
           tc_fence_after();
-          if constexpr (SPLIT) {
-            issue_qk(q_lo, idx, false);                  // Q_hi K_lo^T
-            release(idx);
-            wait_full(idx + 1);
-            tc_fence_after();
-            issue_qk(q_lo, idx + 1, true);               // Q_hi K_hi^T
-            issue_qk(q_lo + (HT >> 4), idx + 1, true);   // Q_lo K_hi^T
-            tc_commit_u(s_full(t));
-            release(idx + 1);
-          } else if constexpr (WIDE) {
-            issue_qk(q_lo, idx, false);                  // Q_a K_a^T
-            release(idx);
-            wait_full(idx + 1);
-            tc_fence_after();
-            issue_qk(q_lo + (HT >> 4), idx + 1, true);   // + Q_b K_b^T
-            tc_commit_u(s_full(t));
-            release(idx + 1);
-          } else {
-            issue_s(idx);
-            tc_commit_u(s_full(t));
-            release(idx);
-          }
-        };
-        unsigned long long* tr = nullptr;            // timeline of the first item of CTA 0: MFA_FWD_TRACE (debug builds of the launch only)
-        if (TR && p.trace && w == 0 && lane == 0) tr = p.trace + (size_t)t * 64 * 16;
-        mbar_wait(q_full(t), qc & 1);
-        do_s(kvbase);
-        if (n == 1) tc_commit_u(q_empty(t));
-        for (int it = 0; it < n; ++it) {
-          const int vi = kvbase + SPS * it + (SPS == 2 ? 1 : 2), ki = kvbase + SPS * (it + 1);
-          wait_full(vi);
-          if (TR && tr && it < 64) tr[it * 16 + 13] = clock64();
-#pragma unroll
-          for (int part = 0; part < kParts; ++part) {
-            mbar_wait(p_part(t, part), pc & 1);
-            // the first P V of an item (and, split mode, of a flush period) overwrites O: the softmax warps must have read the
-            // previous contents out of TMEM (epilogue of the previous item / flush) -- one o_empty phase per hand-over
-            const bool fresh = F > 0 ? (it % F == 0) : (it == 0);
-            if (part == 0 && fresh && (it > 0 || qc > 0)) { mbar_wait(o_empty(t), oe & 1); ++oe; }
-            tc_fence_after();
-            if (TR && tr && it < 64) tr[it * 16 + 8 + part] = clock64();
-            issue_o_part(vi, part, !fresh);
-          }
-          release(vi);
-          if constexpr (SPLIT) {                         // closing group of the step: P_hi V_lo over all 128 keys
-            wait_full(vi + 1);
-            tc_fence_after();
-            const uint32_t b0 = v_lo + ((vi + 1) % NS) * (STG >> 4);
-#pragma unroll
-            for (int kk = 0; kk < 8; ++kk) mma_f16_ts_u(tO, tS + kk * 8, b0 + kk * (2048 >> 4), kDescHiSw128, IDESC_O, 1u);
-            release(vi + 1);
-          }
-          if (it + 1 < n) {
-            if (TR && tr && it < 64) tr[it * 16 + 14] = clock64();
-            do_s(ki);
-            if (it + 2 == n) tc_commit_u(q_empty(t));          // last S of the item: Q_t may be reloaded for the next one
-            if (TR && tr && it < 64) tr[it * 16 + 12] = clock64();
-          } else {
-            tc_commit_u(o_full(t));
-          }
-          ++pc;
+          issue_qk(q_lo, idx + 1, true);               // Q_hi K_hi^T
+          issue_qk(q_lo + (HT >> 4), idx + 1, true);   // Q_lo K_hi^T
+          tc_commit_u(s_full(t));
+          release(idx + 1);
+        } else if constexpr (WIDE) {
+          issue_qk(q_lo, idx, false);                  // Q_a K_a^T
+          release(idx);
+          wait_full(idx + 1);
+          tc_fence_after();
+          issue_qk(q_lo + (HT >> 4), idx + 1, true);   // + Q_b K_b^T
+          tc_commit_u(s_full(t));
+          release(idx + 1);
+        } else {
+          issue_s(idx);
+          tc_commit_u(s_full(t));
+          release(idx);
         }
-        ++qc;
+      };
+      mbar_wait(q_full(t), 0);
+      do_s(0);
+      for (int it = 0; it < n; ++it) {
+        const int vi = SPS * it + (SPS == 2 ? 1 : 2), ki = SPS * (it + 1);
+        wait_full(vi);
+#pragma unroll
+        for (int part = 0; part < kParts; ++part) {
+          mbar_wait(p_part(t, part), pc & 1);
+          // the first P V of a flush period (split mode) overwrites O: the softmax warps must have read the previous contents
+          // out of TMEM (flush) -- one o_empty phase per hand-over
+          const bool fresh = F > 0 ? (it % F == 0) : (it == 0);
+          if (part == 0 && fresh && it > 0) { mbar_wait(o_empty(t), oe & 1); ++oe; }
+          tc_fence_after();
+          issue_o_part(vi, part, !fresh);
+        }
+        release(vi);
+        if constexpr (SPLIT) {                         // closing group of the step: P_hi V_lo over all 128 keys
+          wait_full(vi + 1);
+          tc_fence_after();
+          const uint32_t b0 = v_lo + ((vi + 1) % NS) * (STG >> 4);
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk) mma_f16_ts_u(tO, tS + kk * 8, b0 + kk * (2048 >> 4), kDescHiSw128, IDESC_O, 1u);
+          release(vi + 1);
+        }
+        if (it + 1 < n) do_s(ki);
+        else tc_commit_u(o_full(t));
+        ++pc;
       }
-      kvbase += SPS * n;
     }
   } else if (warp < 8) {
     // ------------------------------------------------------------------ softmax warpgroups
@@ -517,17 +480,15 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     const uint32_t lane_base = (uint32_t)((warp & 3) * 32) << 16;
     const uint32_t tS = tmem + lane_base + t * 128;
     const uint32_t tO = tmem + lane_base + 256 + t * D;
-    int pc = 0, qc = 0;                                    // KV steps / items done by this tile (barrier phases)
+    int pc = 0;                                            // KV steps done by this tile (barrier phases)
     int mkc = 0;                                           // staged mask tiles consumed by this tile
-    if (p.pingpong && t == 1) named_bar_arrive(2, 256);    // the first turn belongs to tile 0
-    for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-    const Item im = decode(w);
+    if (t == 1) named_bar_arrive(2, 256);                  // the first turn belongs to tile 0
+    const Item im = decode(blockIdx.x);
     const int r0 = im.r0, h = im.h, b = im.b, hk = im.hk, nt = im.nt, n = im.n;
     const int r = r0 + t * 128 + row;
     float m = -CUDART_INF_F, l = 0.f;                      // m in scaled log2 units (score * scale * log2 e)
-    const int kv_hi = p.kv_end > 0 ? p.kv_end : p.Skv, kv_lo = p.kv_end > 0 ? p.kv_begin : 0;
-    const int chi = p.causal ? min(kv_hi - 1, r) : kv_hi - 1;
-    const int clo = p.window >= 0 ? max(kv_lo, r - p.window) : kv_lo;
+    const int chi = p.causal ? min(p.Skv - 1, r) : p.Skv - 1;
+    const int clo = p.window >= 0 ? max(0, r - p.window) : 0;
     // int8 mode: per-row Q scale (folded with c), per-64-key K and V block scales
     float qsc = p.c;
     const float* ksp = nullptr;
@@ -545,7 +506,7 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     int nflush = 0;
     const int dv_row = p.dv > 0 ? p.dv : D;                // head dims this row holds in global memory
     const bool v_blocks = I8 && !F8 && vsp != nullptr;     // (e4m3 V carries one scale per (b, head): applied in the epilogue)
-    const bool pingpong = nt == 2 && p.pingpong;
+    const bool pingpong = nt == 2;
 
     if (t < nt) {
       // int8 mode: raw K / V block scales of the two 64-key halves of a tile.  They are fetched one KV step ahead (right
@@ -583,9 +544,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
             iv0 = 1.f / vsn0; iv1 = 1.f / vsn1;
           }
         }
-        unsigned long long* tr = nullptr;
-        if (TR && p.trace && w == 0 && (threadIdx.x & 127) == 0 && it < 64)
-          tr = p.trace + ((size_t)t * 64 + it) * 16;
         mbar_wait(s_full(t), pc & 1);
         ++pc;
         tc_fence_after();
@@ -600,7 +558,7 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
             // the flushed part lives in a scratch tile private to this (item, tile), laid out [column / 4][row][4]: the 32 rows
             // of a warp touch consecutive 16-byte units, so every access is a fully coalesced 512-byte request (row-major rows
             // of the output would cost 32 sectors in 32 lines per request)
-            float4* fbuf = reinterpret_cast<float4*>(p.flush_buf) + ((size_t)w * 2 + t) * (size_t)(D / 4) * 128 + row;
+            float4* fbuf = reinterpret_cast<float4*>(p.flush_buf) + ((size_t)blockIdx.x * 2 + t) * (size_t)(D / 4) * 128 + row;
 #pragma unroll
             for (int ch = 0; ch < D / 32; ++ch) {
               uint32_t ou[32];
@@ -631,8 +589,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
             cb1 = -sb_row * a1;
           }
         }
-        if (TR && tr) tr[0] = clock64();
-        if (TR && ct && it == 0 && w == (int)blockIdx.x) ct[2] = globaltimer_ns();
         uint32_t su[128];
         tmem_ld_x32(tS, su);
         tmem_ld_x32(tS + 32, su + 32);
@@ -640,7 +596,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         tmem_ld_x32(tS + 96, su + 96);
         tmem_wait_ld();
         float* s = reinterpret_cast<float*>(su);
-        if (TR && tr) tr[1] = clock64();
         if (it + 1 < n) { jt_next = tile_of(im, it + 1); fetch_scales(jt_next); }
         if constexpr (I8) {
           // Widening without a conversion instruction: (s << k) plus the bit pattern of B = 1.5 * 2^(23-k), read as a float, IS
@@ -655,7 +610,6 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
 #pragma unroll
           for (int i = 0; i < 128; ++i) su[i] = su[i] * smul + sadd;
         }
-        if (TR && tr) tr[15] = clock64();
         if (MT && !mask_noop) {
           if constexpr (MT) {
             // the mask tile of this (step, query tile) is in shared memory (TMA, 128-byte swizzle: 16-byte unit j of row r sits
@@ -852,19 +806,15 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         // exp2 turn-taking: the two tiles' exp2 phases are MUFU-bound and share the four SMSPs, so run them one after
         // the other (tile 0 first) -- this locks the tiles in anti-phase: one is in exp2 while the tensor pipe works
         // for the other.  Left alone they drift in phase (the in-order tensor pipe queues S_1 right behind S_0) and
-        // each exp2 phase takes twice as long (profiles/: timeline).  Strict alternation, also across the items of the opt-in
-        // persistent loop: tile 0 takes its k-th turn on the credit tile 1 posts after its (k-1)-th (the first credit is
-        // posted before the item loop), so neither named barrier ever sees two arrivals of one side in a row.  (Letting tile 0
-        // start an item without waiting dead-locks when tile 1 is held back at an item boundary: tile 0 then arrives twice on
-        // barrier 3 and the barrier completes without tile 1 -- profiles/r02/r02e_watchdog_pingpong.txt.)
-        if (TR && tr) tr[7] = clock64();
+        // each exp2 phase takes twice as long (profiles/: timeline).  Strict alternation: tile 0 takes its k-th turn on the
+        // credit tile 1 posts after its (k-1)-th (the first credit is posted before the KV loop), so neither named barrier ever
+        // sees two arrivals of one side in a row.  (A turn taken without the credit lets tile 0 arrive twice on barrier 3, and
+        // the barrier then completes without tile 1 -- profiles/r02/r02e_watchdog_pingpong.txt.)
         if (pingpong) {
           if (t == 0) named_bar_sync(2, 256);
           else named_bar_sync(3, 256);
         }
-        if (TR && tr) tr[2] = clock64();
-        if (POLY > 0) exp_phase<PF, POLY, TR>(s, a0, a1, nk0, nk1, tS, p_part(t, 0), lane, sum_lo, sum_hi, tr);
-        else exp_phase<PF, 0, TR>(s, a0, a1, nk0, nk1, tS, p_part(t, 0), lane, sum_lo, sum_hi, tr);
+        exp_phase<PF, C::kPoly>(s, a0, a1, nk0, nk1, tS, p_part(t, 0), lane, sum_lo, sum_hi);
         if (pingpong) {
           if (t == 0) named_bar_arrive(3, 256);
           else named_bar_arrive(2, 256);
@@ -872,17 +822,14 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         l += sum_lo * iv0 + sum_hi * iv1;
       }
       // ---------------------------------------------------------------- epilogue: O / l, L = m + log2(l)
-      if (TR && ct && w == (int)blockIdx.x) ct[3] = globaltimer_ns();
       if (n > 0) {
-        mbar_wait(o_full(t), qc & 1);
-        ++qc;
+        mbar_wait(o_full(t), 0);
         tc_fence_after();
       }
-      if (TR && ct && w == (int)blockIdx.x) ct[4] = globaltimer_ns();
       float inv = (l > 0.f ? 1.f / l : 0.f) * ((I8 && !v_blocks) ? p.vs1 : 1.f);
       if constexpr (F8) { if (p.vs) inv = (l > 0.f ? 1.f / l : 0.f) * __ldg(p.vs + (size_t)b * p.Hkv + hk); }     // per-(b, head) scale of the e4m3 V
       if constexpr (SPLIT) inv *= __ldg(p.vs);
-      const bool live = r < p.Sq && !p.debug_skip_store;
+      const bool live = r < p.Sq;
       // zero-padded head dims: the columns past the true head dim p.dv are not written
       const bool padded_d = p.dv > 0 && p.dv < (WIDE ? 256 : D);
       const int dv_tile = p.dv - (WIDE ? 128 * im.half : 0);
@@ -893,10 +840,10 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
       //   L = log2(2^L_old + 2^L_new),  O = O_old 2^(L_old - L) + O_new 2^(L_new - L)      (fp32 O only)
       float c_old = 0.f;
       const bool acc_mode = p.accumulate && p.o_dtype == kF32;
-      const bool tma_out = p.o_tma && !acc_mode && !p.debug_skip_store;
+      const bool tma_out = p.o_tma && !acc_mode;
       if (tma_out) {
         // the staging area reuses the operand memory: wait until the other tile has retired its last MMA too
-        if (n > 0 && nt == 2) { mbar_wait(o_full(t ^ 1), 0); tc_fence_after(); }      // (o_tma is off in persistent mode)
+        if (n > 0 && nt == 2) { mbar_wait(o_full(t ^ 1), 0); tc_fence_after(); }
       }
       if (acc_mode && live) {
         const float l_old = p.lse[lrow];
@@ -915,14 +862,10 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
 #pragma unroll
         for (int ch = 0; ch < D / 32; ++ch) tmem_ld_x32(tO + ch * 32, oall + ch * 32);
         tmem_wait_ld();
-        // O has left TMEM: the MMA warp may overwrite it with the first P V of this CTA's next item
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(o_empty(t));
         if constexpr (SPLIT) {
           if (nflush > 0) {        // + what the flushes left in the scratch tile, brought to the final running max
             const float fs = m_flush != -CUDART_INF_F ? ex2(m_flush - m) : 0.f;
-            const float4* src = reinterpret_cast<const float4*>(p.flush_buf) + ((size_t)w * 2 + t) * (size_t)(D / 4) * 128 + row;
+            const float4* src = reinterpret_cast<const float4*>(p.flush_buf) + ((size_t)blockIdx.x * 2 + t) * (size_t)(D / 4) * 128 + row;
 #pragma unroll
             for (int i = 0; i < D / 4; ++i) {
               const float4 g4 = src[(size_t)i * 128];
@@ -1041,10 +984,8 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         }
       }
       if (live && p.lse && (!WIDE || im.half == 0)) p.lse[lrow] = l_out;
-      if (TR && ct && w == (int)blockIdx.x) { ct[5] = globaltimer_ns(); ct[8] = clock64(); }
     }
-    }   // items
-    if (p.pingpong && t == 0) named_bar_sync(2, 256);      // take the credit nobody will use: the barriers end balanced
+    if (t == 0) named_bar_sync(2, 256);                    // take the credit nobody will use: the barriers end balanced
   }
   else {
     reg_dealloc<kWg2Regs>();      // warp 11 (setmaxnreg is warpgroup-wide): idle, the mask producer, or the int4 converter
@@ -1058,34 +999,27 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         prefetch_tmap(&p.tm);
         // the mask streams through once (up to GBs): evict-first keeps it from pushing the K / V tiles the other CTAs of a
         // head re-read out of L2
-#ifdef MFA_MASK_NO_HINT
-        const uint64_t pol = l2_policy_evict_normal();
-#else
         const uint64_t pol = l2_policy_evict_first();
-#endif
         const bool one_byte = p.mask_kind == kMaskBool;
         int mc[2] = {0, 0};
-        for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-          const Item im = decode(w);
-          if (im.n == 0) continue;
-          const int mb = p.mask_sb ? im.b : 0, mh = p.mask_sh ? im.h : 0;
-          for (int it = 0; it < im.n; ++it) {
-            const int jt = tile_of(im, it);
-            if (jt & kTileNoMask) continue;
-            const int c0 = (jt & (kTileNoMask - 1)) * 128;
-            for (int t = 0; t < im.nt; ++t) {
-              if (mc[t] > 0) mbar_wait(mk_empty(t), (mc[t] - 1) & 1);
-              const uint32_t dst = sMask + (uint32_t)t * C::kMaskTile;
-              if (one_byte) {
-                mbar_arrive_expect_tx(mk_full(t), 16384);
-                tma_load_4d_hint(dst, &p.tm, mk_full(t), c0, im.r0 + t * 128, mh, mb, pol);
-              } else {
-                mbar_arrive_expect_tx(mk_full(t), 32768);
-                tma_load_4d_hint(dst, &p.tm, mk_full(t), c0, im.r0 + t * 128, mh, mb, pol);
-                tma_load_4d_hint(dst + 16384, &p.tm, mk_full(t), c0 + 64, im.r0 + t * 128, mh, mb, pol);
-              }
-              ++mc[t];
+        const Item im = decode(blockIdx.x);
+        const int mb = p.mask_sb ? im.b : 0, mh = p.mask_sh ? im.h : 0;
+        for (int it = 0; it < im.n; ++it) {
+          const int jt = tile_of(im, it);
+          if (jt & kTileNoMask) continue;
+          const int c0 = (jt & (kTileNoMask - 1)) * 128;
+          for (int t = 0; t < im.nt; ++t) {
+            if (mc[t] > 0) mbar_wait(mk_empty(t), (mc[t] - 1) & 1);
+            const uint32_t dst = sMask + (uint32_t)t * C::kMaskTile;
+            if (one_byte) {
+              mbar_arrive_expect_tx(mk_full(t), 16384);
+              tma_load_4d_hint(dst, &p.tm, mk_full(t), c0, im.r0 + t * 128, mh, mb, pol);
+            } else {
+              mbar_arrive_expect_tx(mk_full(t), 32768);
+              tma_load_4d_hint(dst, &p.tm, mk_full(t), c0, im.r0 + t * 128, mh, mb, pol);
+              tma_load_4d_hint(dst + 16384, &p.tm, mk_full(t), c0 + 64, im.r0 + t * 128, mh, mb, pol);
             }
+            ++mc[t];
           }
         }
       }
@@ -1132,40 +1066,36 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
           }
         }
       };
-      int kvbase = 0, kr = 0, cq = 0, qc[2] = {0, 0};
-      for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-        const Item im = decode(w);
-        const int nt = im.nt, n = im.n;
-        if (n == 0) continue;
-        auto convert_q = [&](int t2) {
-          if (qc[t2] > 0) mbar_wait(q_empty(t2), (qc[t2] - 1) & 1);      // the MMA warp has issued the last S that reads Q_t2
-          mbar_wait(qraw_full, cq & 1);
-          unpack_tile(sRawQ, sQ + t2 * QT, std::true_type{}, sQsum + t2 * 512);
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (lane == 0) { mbar_arrive(q_full(t2)); mbar_arrive(qraw_empty); }
-          ++cq; ++qc[t2];
-        };
-        convert_q(0);
-        for (int it = 0; it < n; ++it) {
-          const int idx = kvbase + 2 * it, s = idx % NS, rs = kr % NR;
-          mbar_wait(raw_full(rs), (kr / NR) & 1);
-          mbar_wait(kv_empty(s), ((idx / NS) & 1) ^ 1);
-          unpack_tile(sRawK + rs * RAW, sKV + s * STG, std::false_type{}, 0u);
-          fence_proxy_async_smem();
-          __syncwarp();
-          if (lane == 0) { mbar_arrive(kv_full(s)); mbar_arrive(raw_empty(rs)); }
-          ++kr;
-          if (it == 0 && nt == 2) convert_q(1);
-        }
-        kvbase += 2 * n;
+      int kr = 0, cq = 0;
+      const Item im = decode(blockIdx.x);
+      const int nt = im.nt, n = im.n;
+      auto convert_q = [&](int t2) {
+        mbar_wait(qraw_full, cq & 1);
+        unpack_tile(sRawQ, sQ + t2 * QT, std::true_type{}, sQsum + t2 * 512);
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) { mbar_arrive(q_full(t2)); mbar_arrive(qraw_empty); }
+        ++cq;
+      };
+      if (n > 0) convert_q(0);
+      for (int it = 0; it < n; ++it) {
+        const int idx = 2 * it, s = idx % NS, rs = kr % NR;
+        mbar_wait(raw_full(rs), (kr / NR) & 1);
+        mbar_wait(kv_empty(s), ((idx / NS) & 1) ^ 1);
+        unpack_tile(sRawK + rs * RAW, sKV + s * STG, std::false_type{}, 0u);
+        fence_proxy_async_smem();
+        __syncwarp();
+        if (lane == 0) { mbar_arrive(kv_full(s)); mbar_arrive(raw_empty(rs)); }
+        ++kr;
+        if (it == 0 && nt == 2) convert_q(1);
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (TR && ct) ct[9] = globaltimer_ns();
-  if (warp == 9) tmem_dealloc(tmem, 512);
+  // the allocating warp frees the columns, reading their address back from the slot: keeping `tmem` live through every role
+  // costs a register that ptxas then finds by spilling (fp32 split kernel)
+  if (warp == 9) tmem_dealloc(*reinterpret_cast<volatile uint32_t*>(smem_raw + (tmem_slot - raw)), 512);
 }
 
 // ---- tile skipping under an external mask (north_star item 3): a two-kernel pre-pass reads the mask once and leaves, per
@@ -1319,7 +1249,7 @@ __global__ void __launch_bounds__(WARP_TILE ? 256 : 64, WARP_TILE ? 4 : 16) mask
 template <typename M>
 void launch_flags(const MaskTileParams& q, const M& m, uint8_t* flags, cudaStream_t st) {
   const long long tiles = (long long)m.nkt * m.nqb * m.MB * m.MH;
-  if (tiles >= 4096 && !getenv("MFA_MASK_FLAGS_CTA_TILE"))
+  if (tiles >= 4096)
     mask_flags_kernel<true><<<dim3((unsigned)((m.nkt + 7) / 8), (unsigned)m.nqb, (unsigned)(m.MB * m.MH)), 256, 0, st>>>(q, flags);
   else
     mask_flags_kernel<false><<<dim3((unsigned)m.nkt, (unsigned)m.nqb, (unsigned)(m.MB * m.MH)), 64, 0, st>>>(q, flags);
@@ -1343,98 +1273,10 @@ using tc::make_map;
 
 bool view_ok(const TensorView& t, int64_t, int64_t Hn, int64_t B) { return tc::view_ok(t, Hn, B); }
 
-}  // namespace
-
-int fwd_tc_pingpong() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("MFA_FWD_PINGPONG"); v = e ? atoi(e) : 1; }
-  return v;
-}
-
-namespace {
-
-int poly_setting() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("MFA_FWD_POLY"); v = e ? atoi(e) : 3; }
-  return v;
-}
-
-template <int D, int MODE, int POLY>
+template <int D, int MODE, int MASKED>
 cudaError_t launch_k(const FwdTcParams& prm, dim3 grid, cudaStream_t st) {
   static bool attr_set = false;
-  auto kern = fwd_tc_kernel<D, MODE, POLY>;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<D, MODE>::kSmem);
-    if (e != cudaSuccess) return e;
-    attr_set = true;
-  }
-  kern<<<grid, kThreads, Cfg<D, MODE>::kSmem, st>>>(prm);
-  return cudaGetLastError();
-}
-
-// MFA_FWD_TRACE=<file>: run the instrumented build of the D=128 kernel and dump the clock64 timeline of CTA (0,0,0)
-// (rows: tile, step; 16 stamps: 0 S ready, 1 S in registers, 2 max done, 3-6 P part published, 8-11 part seen by the
-// MMA warp, 12 next S issued, 13 V tile landed, 14 K tile landed).  Debug aid; synchronises the stream.
-// MFA_FWD_CTATRACE=<file>: same instrumented build, per-CTA stamps (globaltimer ns: 0 entry, 1 set-up done, 2 first S seen,
-// 3 main loop done, 4 last P V retired, 5 epilogue done, 9 CTA end; 6 = SM id; 7 / 8 = clock64 at entry / epilogue end).
-template <int MODE, int POLY>
-cudaError_t launch_cta_traced(FwdTcParams prm, dim3 grid, cudaStream_t st, const char* path) {
-  const size_t words = (size_t)grid.x * 16;
-  unsigned long long* dev = nullptr;
-  if (cudaMalloc(&dev, words * 8) != cudaSuccess) return cudaErrorMemoryAllocation;
-  cudaMemsetAsync(dev, 0, words * 8, st);
-  prm.cta_trace = dev;
-  auto kern = fwd_tc_kernel<128, MODE, POLY, true>;
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128, MODE>::kSmem);
-  kern<<<grid, kThreads, Cfg<128, MODE>::kSmem, st>>>(prm);
-  cudaError_t e = cudaStreamSynchronize(st);
-  unsigned long long* host = (unsigned long long*)malloc(words * 8);
-  cudaMemcpy(host, dev, words * 8, cudaMemcpyDeviceToHost);
-  cudaFree(dev);
-  if (FILE* f = fopen(path, "w")) {
-    for (unsigned c = 0; c < grid.x; ++c) {
-      fprintf(f, "%u", c);
-      for (int k = 0; k < 10; ++k) fprintf(f, " %llu", host[(size_t)c * 16 + k]);
-      fprintf(f, "\n");
-    }
-    fclose(f);
-  }
-  free(host);
-  return e;
-}
-
-template <int MODE, int POLY>
-cudaError_t launch_traced(FwdTcParams prm, dim3 grid, cudaStream_t st, const char* path) {
-  constexpr size_t kWords = 2 * 64 * 16;
-  unsigned long long* dev = nullptr;
-  if (cudaMalloc(&dev, kWords * 8) != cudaSuccess) return cudaErrorMemoryAllocation;
-  cudaMemsetAsync(dev, 0, kWords * 8, st);
-  prm.trace = dev;
-  auto kern = fwd_tc_kernel<128, MODE, POLY, true>;
-  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<128, MODE>::kSmem);
-  kern<<<grid, kThreads, Cfg<128, MODE>::kSmem, st>>>(prm);
-  cudaError_t e = cudaStreamSynchronize(st);
-  static unsigned long long host[kWords];
-  cudaMemcpy(host, dev, kWords * 8, cudaMemcpyDeviceToHost);
-  cudaFree(dev);
-  if (FILE* f = fopen(path, "w")) {
-    for (int t = 0; t < 2; ++t)
-      for (int it = 0; it < 64; ++it) {
-        const unsigned long long* r = host + ((size_t)t * 64 + it) * 16;
-        if (!r[0] && !r[8]) continue;
-        fprintf(f, "%d %d", t, it);
-        for (int k = 0; k < 16; ++k) fprintf(f, " %llu", r[k]);
-        fprintf(f, "\n");
-      }
-    fclose(f);
-  }
-  return e;
-}
-
-template <int D, int MODE, int POLY, int MASKED>
-cudaError_t launch_masked_v(const FwdTcParams& prm, dim3 grid, cudaStream_t st) {
-  static bool attr_set = false;
-  auto kern = fwd_tc_kernel<D, MODE, POLY, false, MASKED>;
+  auto kern = fwd_tc_kernel<D, MODE, MASKED>;
   constexpr int kSmem = Cfg<D, MODE, MASKED>::kSmem;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
@@ -1446,62 +1288,15 @@ cudaError_t launch_masked_v(const FwdTcParams& prm, dim3 grid, cudaStream_t st) 
 }
 
 // dense 1- / 2-byte masks take the instantiation that stages mask tiles in shared memory (where the mode has one)
-template <int D, int MODE, int POLY>
-cudaError_t launch_masked_k(const FwdTcParams& prm, dim3 grid, cudaStream_t st) {
-  if constexpr (Cfg<D, MODE, 2>::kMaskTma) {
-    if (prm.mask_tma) return launch_masked_v<D, MODE, POLY, 2>(prm, grid, st);
-  }
-  return launch_masked_v<D, MODE, POLY, 1>(prm, grid, st);
-}
-
-// masked kernels come in two exp2 flavours only: all MUFU, or the default polynomial share on tiles the mask leaves alone
-template <int D, int MODE>
-cudaError_t launch_masked(const FwdTcParams& prm, dim3 grid, cudaStream_t st) {
-  return poly_setting() > 0 ? launch_masked_k<D, MODE, 3>(prm, grid, st) : launch_masked_k<D, MODE, 0>(prm, grid, st);
-}
-
 template <int D, int MODE>
 cudaError_t launch(const FwdTcParams& prm, dim3 grid, cudaStream_t st) {
-#ifdef MFA_DEV_ONE        // compile-time experiment builds: the D = 128 bf16 kernel (plain + masked) only
-  if constexpr (D == 128 && MODE == kFwdBF16) return prm.mask ? launch_masked_k<D, MODE, 3>(prm, grid, st) : launch_k<D, MODE, 3>(prm, grid, st);
-  else return cudaErrorNotSupported;
-#else
-  if (prm.mask) return launch_masked<D, MODE>(prm, grid, st);
-  if constexpr (D == 128 && (MODE == kFwdBF16 || MODE == kFwdI8F8)) {
-    if (const char* path = getenv("MFA_FWD_TRACE"))
-      return poly_setting() == 2 ? launch_traced<MODE, 2>(prm, grid, st, path) : launch_traced<MODE, 0>(prm, grid, st, path);
-    if (const char* path = getenv("MFA_FWD_CTATRACE"))
-      return poly_setting() == 3 ? launch_cta_traced<MODE, 3>(prm, grid, st, path) : launch_cta_traced<MODE, 0>(prm, grid, st, path);
+  if (!prm.mask) return launch_k<D, MODE, 0>(prm, grid, st);
+  if constexpr (Cfg<D, MODE, 2>::kMaskTma) {
+    if (prm.mask_tma) return launch_k<D, MODE, 2>(prm, grid, st);
   }
-  switch (poly_setting()) {
-    case 1: return launch_k<D, MODE, 1>(prm, grid, st);
-    case 2: return launch_k<D, MODE, 2>(prm, grid, st);
-    case 3: return launch_k<D, MODE, 3>(prm, grid, st);
-    case 4: return launch_k<D, MODE, 4>(prm, grid, st);
-    default: return launch_k<D, MODE, 0>(prm, grid, st);
-  }
-#endif
+  return launch_k<D, MODE, 1>(prm, grid, st);
 }
 
-}  // namespace
-
-namespace {
-int sm_count() {
-  static int v = 0;
-  if (!v) {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || v <= 0) v = 148;
-  }
-  return v;
-}
-int persist_setting() {
-  static int v = -1;
-  // measured (profiles/r01f_persist_notes.txt): at the 1 kW power cap the persistent grid does not beat one CTA per item
-  // with the TMA-store epilogue (FLUX 0.2199 vs 0.2161 ms), so it is opt-in
-  if (v < 0) { const char* e = getenv("MFA_FWD_PERSIST"); v = e ? atoi(e) : 0; }
-  return v;
-}
 }  // namespace
 
 cudaError_t launch_fwd_tc_kernel(const FwdTcParams& prm_in, int D, int mode, cudaStream_t st, int B) {
@@ -1511,47 +1306,24 @@ cudaError_t launch_fwd_tc_kernel(const FwdTcParams& prm_in, int D, int mode, cud
   const bool wide = mode == kFwdWideF16 || mode == kFwdWideBF16;
   const long long items = (long long)((prm.Sq + 255) / 256) * prm.H * B * (wide ? 2 : 1);
   if (items <= 0 || items > 0x7fffffffLL) return cudaErrorInvalidValue;
-  // Persistent grid (one CTA per SM striding over the items) when every item costs the same -- no causal / window
-  // imbalance that the hardware's dynamic CTA dispatch handles better -- and there is more than one item per SM.
-  // ... and for the key slices of the fp32 split mode (8 KV steps per item: the per-item prologue is a quarter of the work; the
-  // persistent loop hides it: FLUX fp32 0.781 -> 0.750 ms, profiles/r02af_*)
-  const bool persist = (persist_setting() || (mode == kFwdSplit && prm.kv_end > 0 && !getenv("MFA_FWD_NO_PERSIST"))) &&
-                       !prm.causal && prm.window < 0 && items > sm_count() && !prm.trace;
-  if (persist) prm.o_tma = 0;                    // the staging tile of the TMA-store epilogue aliases the operand ring
-  dim3 grid((unsigned)(persist ? sm_count() : items), 1, 1);
-#ifdef MFA_DEV_ONE
-  return (D == 128 && mode == kFwdBF16) ? launch<128, kFwdBF16>(prm, grid, st) : cudaErrorNotSupported;
-#else
-  if (mode == kFwdI8) return D == 128 ? launch<128, kFwdI8>(prm, grid, st) : cudaErrorInvalidValue;
-  if (mode == kFwdI8F8) return D == 128 ? launch<128, kFwdI8F8>(prm, grid, st) : cudaErrorInvalidValue;
-  if (mode == kFwdI4 || mode == kFwdI4F8) {       // packed int4 Q / K: default exp2 mix, or all-MUFU when the polynomial is off
-    if (D != 128) return cudaErrorInvalidValue;
-    const bool poly = poly_setting() > 0;
-    if (mode == kFwdI4) {
-      if (prm.mask) return poly ? launch_masked_k<128, kFwdI4, 3>(prm, grid, st) : launch_masked_k<128, kFwdI4, 0>(prm, grid, st);
-      return poly ? launch_k<128, kFwdI4, 3>(prm, grid, st) : launch_k<128, kFwdI4, 0>(prm, grid, st);
-    }
-    if (prm.mask) return poly ? launch_masked_k<128, kFwdI4F8, 3>(prm, grid, st) : launch_masked_k<128, kFwdI4F8, 0>(prm, grid, st);
-    return poly ? launch_k<128, kFwdI4F8, 3>(prm, grid, st) : launch_k<128, kFwdI4F8, 0>(prm, grid, st);
-  }
-  if (mode == kFwdWideF16 || mode == kFwdWideBF16) {      // D is the head dim of the problem (256); the kernel's tiles are 128 wide
+  const dim3 grid((unsigned)items, 1, 1);        // one CTA per work item
+  if (wide) {                                    // D is the head dim of the problem (256); the kernel's tiles are 128 wide
     if (D != 256) return cudaErrorInvalidValue;
-    const bool poly = poly_setting() > 0;
-    if (mode == kFwdWideBF16) {
-      if (prm.mask) return poly ? launch_masked_k<128, kFwdWideBF16, 3>(prm, grid, st) : launch_masked_k<128, kFwdWideBF16, 0>(prm, grid, st);
-      return poly ? launch_k<128, kFwdWideBF16, 3>(prm, grid, st) : launch_k<128, kFwdWideBF16, 0>(prm, grid, st);
-    }
-    if (prm.mask) return poly ? launch_masked_k<128, kFwdWideF16, 3>(prm, grid, st) : launch_masked_k<128, kFwdWideF16, 0>(prm, grid, st);
-    return poly ? launch_k<128, kFwdWideF16, 3>(prm, grid, st) : launch_k<128, kFwdWideF16, 0>(prm, grid, st);
+    return mode == kFwdWideBF16 ? launch<128, kFwdWideBF16>(prm, grid, st) : launch<128, kFwdWideF16>(prm, grid, st);
   }
-  if (mode == kFwdSplit) {        // exact exp2 only (the polynomial's 8.6e-5 would show at fp32 tolerances)
-    if (D != 128) return cudaErrorInvalidValue;
-    return prm.mask ? launch_masked_k<128, kFwdSplit, 0>(prm, grid, st) : launch_k<128, kFwdSplit, 0>(prm, grid, st);
+  if (D == 64 && mode == kFwdBF16) return launch<64, kFwdBF16>(prm, grid, st);
+  if (D == 64 && mode == kFwdF16) return launch<64, kFwdF16>(prm, grid, st);
+  if (D != 128) return cudaErrorInvalidValue;
+  switch (mode) {
+    case kFwdF16: return launch<128, kFwdF16>(prm, grid, st);
+    case kFwdBF16: return launch<128, kFwdBF16>(prm, grid, st);
+    case kFwdI8: return launch<128, kFwdI8>(prm, grid, st);
+    case kFwdI8F8: return launch<128, kFwdI8F8>(prm, grid, st);
+    case kFwdSplit: return launch<128, kFwdSplit>(prm, grid, st);
+    case kFwdI4: return launch<128, kFwdI4>(prm, grid, st);
+    case kFwdI4F8: return launch<128, kFwdI4F8>(prm, grid, st);
+    default: return cudaErrorInvalidValue;
   }
-  if (D == 128) return mode == kFwdBF16 ? launch<128, kFwdBF16>(prm, grid, st) : launch<128, kFwdF16>(prm, grid, st);
-  if (D == 64) return mode == kFwdBF16 ? launch<64, kFwdBF16>(prm, grid, st) : launch<64, kFwdF16>(prm, grid, st);
-  return cudaErrorInvalidValue;
-#endif
 }
 
 // external masks the tensor-core forward reads itself: keys contiguous (the row of a tile is one 128-element run)
@@ -1674,8 +1446,6 @@ cudaError_t launch_fwd_tc(const AttnParams& p, cudaStream_t st) {
   prm.H = p.H; prm.Hkv = p.Hkv; prm.Sq = p.Sq; prm.Skv = p.Skv;
   prm.c = p.scale * kLog2e;
   prm.causal = p.causal; prm.window = p.window;
-  prm.pingpong = fwd_tc_pingpong();
-  prm.debug_skip_store = getenv("MFA_DEBUG_SKIP_STORE") ? 1 : 0;       // timing experiment only: O / L are not written
   fwd_tc_set_out_map(prm, p);
   fwd_tc_set_mask(prm, p);
   if (cudaError_t me = fwd_tc_build_mask_tiles(prm, p, st); me != cudaSuccess) return me;

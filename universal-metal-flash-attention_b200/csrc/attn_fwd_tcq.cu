@@ -219,7 +219,6 @@ cudaError_t launch_fwd_tcq(const AttnParams& p, void* scratch, cudaStream_t st) 
   prm.H = p.H; prm.Hkv = p.Hkv; prm.Sq = p.Sq; prm.Skv = p.Skv;
   prm.c = p.scale * kLog2e;
   prm.causal = p.causal; prm.window = p.window;
-  prm.pingpong = fwd_tc_pingpong();
   fwd_tc_set_mask(prm, p);
   if ((e = fwd_tc_build_mask_tiles(prm, p, st)) != cudaSuccess) return e;
   fwd_tc_set_out_map(prm, p);

@@ -31,8 +31,6 @@ struct FwdTcParams {
   int nbatch;              // set by launch_fwd_tc_kernel (work items = query blocks x H x nbatch)
   float c;                 // softmax_scale * log2(e)
   int causal, window;
-  int kv_begin, kv_end;    // kv_end > 0: this launch attends to keys [kv_begin, kv_end) only (kv_begin a multiple of 128); the fp32
-                           // split mode covers long key ranges in slices merged by the accumulate epilogue
   int flush_steps;         // kFwdSplit: O leaves TMEM for an fp32 scratch tile every flush_steps KV steps (0 = never)
   float* flush_buf;        // [work items][2 tiles][D / 4][128 rows][4] floats
   // kFwdI8 only: symmetric scales of the int8 codes (value = code * scale)
@@ -57,13 +55,8 @@ struct FwdTcParams {
   const int* mtiles;       // [lists][m_nkt]
   const int* mcounts;      // [lists]
   int m_nkt;
-  int debug_skip_store;                                 // MFA_DEBUG_SKIP_STORE: epilogue writes nothing (timing experiments)
-  int pingpong;                                         // exp2 turn-taking between the two tiles (MFA_FWD_PINGPONG, default 1)
-  unsigned long long* trace;                            // debug timeline buffer (MFA_FWD_TRACE), normally null
-  unsigned long long* cta_trace;                        // debug per-CTA wall-clock stamps (MFA_FWD_CTATRACE), normally null
 };
 
-int fwd_tc_pingpong();
 bool fwd_tc_mask_ok(const AttnParams& p);
 void fwd_tc_set_mask(FwdTcParams& prm, const AttnParams& p);
 cudaError_t fwd_tc_build_mask_tiles(FwdTcParams& prm, const AttnParams& p, cudaStream_t st);
