@@ -214,6 +214,31 @@ mfa_error_t mfa_attention_backward_ex(
     uint32_t mask_ndim, mfa_mask_type_t mask_type, mfa_mask_scalar_t mask_scalar_type,
     void* stream);
 
+/* Attention over num_seqs sequences packed along the sequence axis, without a dense mask.  cu_seqlens_q / cu_seqlens_k are
+ * int32 [num_seqs + 1] offsets: 0, non-decreasing, ending at total_q / total_k.  Query row i of segment s sees key j only when j
+ * lies in segment s; causal and window_size then apply to the offsets inside the segment (i' = i - cu_q[s], j' = j - cu_k[s]:
+ * causal hides j' > i', the window hides i' > j' + window_size), so one call gives what one mfa_attention_forward_ex /
+ * mfa_attention_backward_ex call per segment gives.  A row that sees no key gets O = 0, L = -inf and no gradient.
+ * q is [1, num_heads, total_q, D], k / v [1, num_kv_heads, total_k, D] (strided handles give the [total, heads, D] layout);
+ * num_kv_heads divides num_heads, 0 = num_heads.  lse fp32 [num_heads, total_q] (log2 units, may be NULL in the forward).
+ * Backward: out fp32 and dout in input_precision, contiguous [num_heads, total_q, D]; dq fp32 [num_heads, total_q, D], dk / dv
+ * fp32 [num_kv_heads, total_k, D], contiguous, overwritten; d_buffer as in mfa_attention_backward_ex.
+ * Host-readable cu_seqlens (host or managed memory) are checked (MFA_ERROR_INVALID_ARGS when malformed); device-resident ones
+ * are not read by the host, and the kernels clamp every bound they derive from them, so a malformed array gives wrong numbers
+ * but no access out of bounds.  stream as in mfa_attention_forward_ex. */
+mfa_error_t mfa_attention_forward_varlen(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k, mfa_buffer_t v, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cu_seqlens_k, uint32_t num_seqs, uint32_t total_q, uint32_t total_k,
+    uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim, float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream);
+
+mfa_error_t mfa_attention_backward_varlen(
+    mfa_context_t context, mfa_buffer_t dout, mfa_buffer_t q, mfa_buffer_t k, mfa_buffer_t v, mfa_buffer_t out,
+    mfa_buffer_t softmax_lse, mfa_buffer_t dq, mfa_buffer_t dk, mfa_buffer_t dv, mfa_buffer_t d_buffer,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cu_seqlens_k, uint32_t num_seqs, uint32_t total_q, uint32_t total_k,
+    uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim, float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, void* stream);
+
 /* Device quantiser (GEMMQuantization.swift:305-623 / GEMMRuntimeQuantization.swift:80-181 contract):
  * src is a row-major [rows, cols] matrix of src_precision; scale[b] = absmax(block b) / 127 (int8) or / 7
  * (int4), floored at scale_floor when scale_floor > 0 (the reference GPU path uses 1e-8); codes =

@@ -64,6 +64,9 @@ struct BwdTcParams {
   const int* ktiles; const int* kcounts;
   const int* qtiles; const int* qcounts;
   int m_nqb, m_nkt;
+  const int* cu_q;             // packed variable-length sequences (AttnParams::cu_q / cu_k / nseq), or null
+  const int* cu_k;
+  int nseq;
 };
 constexpr int kTileNoMask = 1 << 30;          // list entry flag: the mask is a no-op on this tile (no loads needed)
 
@@ -251,11 +254,14 @@ __global__ void __launch_bounds__(kThreads, 1) bwd_dkv_tc_kernel(const __grid_co
   const uint32_t mk_full = sBar + 184, mk_empty = sBar + 192;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for ptxas
+  // packed variable-length sequences (common.h): unmasked instantiations only -- segments do not combine with external masks
+  const int* const seg_q = MASKED ? nullptr : p.cu_q;
+  const int* const seg_k = MASKED ? nullptr : p.cu_k;
   const int jt = blockIdx.x, hk = blockIdx.y, b = blockIdx.z;
   const int c0 = jt * 128;
   const int group = p.H / p.Hkv;
   int qlo, qhi;
-  visible_query_range(p.causal, p.window, p.Sq, c0, min(c0 + 128, p.Skv), qlo, qhi);
+  block_query_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, c0, min(c0 + 128, p.Skv), qlo, qhi);
   const int i_lo = qlo >> 7;
   int nq = qhi > qlo ? ((qhi + 127) >> 7) - i_lo : 0;
   const int* qlist = nullptr;                 // visible query tiles of this KV tile under the external mask
@@ -413,8 +419,9 @@ __global__ void __launch_bounds__(kThreads, 1) bwd_dkv_tc_kernel(const __grid_co
     const uint32_t tS = tmem + lane_base + T_S + half * 64;
     const uint32_t tDP = tmem + lane_base + T_DP + half * 64;
     const float c = p.c, scale = p.scale;
-    const int qlo_r = p.causal ? key : 0;
-    const int qhi_r = p.window >= 0 ? min(key + p.window, 1 << 30) : (1 << 30);
+    int qlo_r, qhi_r;                                      // queries visible to this key: [qlo_r, qhi_r]
+    key_query_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, key, qlo_r, qhi_r);
+    --qhi_r;
     int mkc = 0;                                           // staged mask tiles consumed
     for (int it = 0; it < n_it; ++it) {
       const int s = it & 1;
@@ -595,12 +602,15 @@ __global__ void __launch_bounds__(kThreads, 1) bwd_dq_tc_kernel(const __grid_con
   const uint32_t mk_full = sBar + 152, mk_empty = sBar + 160;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for ptxas
+  // packed variable-length sequences (common.h): unmasked instantiations only -- segments do not combine with external masks
+  const int* const seg_q = MASKED ? nullptr : p.cu_q;
+  const int* const seg_k = MASKED ? nullptr : p.cu_k;
   const int it_q = p.causal ? (int)(gridDim.x - 1 - blockIdx.x) : (int)blockIdx.x;     // heavy tiles first
   const int h = blockIdx.y, b = blockIdx.z;
   const int hk = h / (p.H / p.Hkv);
   const int r0 = it_q * 128;
   int klo, khi;
-  visible_key_range(p.causal, p.window, p.Skv, r0, min(r0 + 128, p.Sq), klo, khi);
+  block_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r0, min(r0 + 128, p.Sq), klo, khi);
   const int j_lo = klo >> 7;
   int n = khi > klo ? ((khi + 127) >> 7) - j_lo : 0;
   const int* klist = nullptr;                 // visible KV tiles of this tile's 256-row query block under the external mask
@@ -727,8 +737,9 @@ __global__ void __launch_bounds__(kThreads, 1) bwd_dq_tc_kernel(const __grid_con
       L = p.lse[ri]; Dt = p.dterm[ri];
       if (L == -CUDART_INF_F) L = CUDART_INF_F;
     }
-    const int chi = p.causal ? min(p.Skv - 1, r) : p.Skv - 1;      // visible keys of this row: [clo, chi]
-    const int clo = p.window >= 0 ? max(0, r - p.window) : 0;
+    int clo, chi;                                          // visible keys of this row: [clo, chi]
+    row_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r, clo, chi);
+    --chi;
     int mkc = 0;                                           // staged mask tiles consumed
     for (int it = 0; it < n; ++it) {
       const int u = it & 1;
@@ -967,6 +978,7 @@ cudaError_t launch_bwd_tc(const AttnParams& p, cudaStream_t st) {
   prm.H = p.H; prm.Hkv = p.Hkv; prm.Sq = p.Sq; prm.Skv = p.Skv;
   prm.c = p.scale * kLog2e; prm.scale = p.scale;
   prm.causal = p.causal; prm.window = p.window;
+  prm.cu_q = p.cu_q; prm.cu_k = p.cu_k; prm.nseq = p.nseq;
   prm.mask = nullptr; prm.mask_kind = kMaskNone; prm.mask_scalar = 0; prm.mask_sb = prm.mask_sh = prm.mask_sq = 0;
   if (p.mask_kind != kMaskNone && p.mask) {
     prm.mask = p.mask; prm.mask_kind = p.mask_kind; prm.mask_scalar = p.mask_scalar;

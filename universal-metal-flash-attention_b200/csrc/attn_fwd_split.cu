@@ -216,6 +216,7 @@ cudaError_t launch_fwd_split(const AttnParams& p, void* scratch, cudaStream_t st
   prm.dv = p.D;
   prm.c = p.scale * kLog2e;
   prm.causal = p.causal; prm.window = p.window;
+  prm.cu_q = p.cu_q; prm.cu_k = p.cu_k; prm.nseq = p.nseq;
   prm.qs = inv; prm.ks = inv + 1; prm.vs = inv + 2;          // inverse power-of-two scales, read by the softmax warps
   fwd_tc_set_out_map(prm, p);
   fwd_tc_set_mask(prm, p);

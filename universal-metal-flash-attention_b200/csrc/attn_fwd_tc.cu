@@ -244,6 +244,9 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
   const uint32_t sMask = (sBar + C::kBarBytes + 1023u) & ~1023u;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;   // warp-uniform for ptxas
+  // packed variable-length sequences (common.h): unmasked instantiations only -- segments do not combine with external masks
+  const int* const seg_q = MASKED ? nullptr : p.cu_q;
+  const int* const seg_k = MASKED ? nullptr : p.cu_k;
   // One CTA per work item = (batch, head, 256-row query block), x fastest so the CTAs of one head run together (K/V stay in L2).
   struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half; };
   auto decode = [&](int w) {
@@ -258,7 +261,7 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     it.r0 = qblk * 256;
     it.nt = (it.r0 + 128 < p.Sq) ? 2 : 1;
     int klo, khi;
-    visible_key_range(p.causal, p.window, p.Skv, it.r0, min(it.r0 + 256, p.Sq), klo, khi);
+    block_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, it.r0, min(it.r0 + 256, p.Sq), klo, khi);
     it.j_lo = klo >> 7;
     it.n = khi > klo ? ((khi + 127) >> 7) - it.j_lo : 0;
     it.lid = 0;
@@ -487,8 +490,9 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     const int r0 = im.r0, h = im.h, b = im.b, hk = im.hk, nt = im.nt, n = im.n;
     const int r = r0 + t * 128 + row;
     float m = -CUDART_INF_F, l = 0.f;                      // m in scaled log2 units (score * scale * log2 e)
-    const int chi = p.causal ? min(p.Skv - 1, r) : p.Skv - 1;
-    const int clo = p.window >= 0 ? max(0, r - p.window) : 0;
+    int clo, chi;                                          // visible keys of this row: [clo, chi]
+    row_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r, clo, chi);
+    --chi;
     // int8 mode: per-row Q scale (folded with c), per-64-key K and V block scales
     float qsc = p.c;
     const float* ksp = nullptr;
@@ -1446,6 +1450,7 @@ cudaError_t launch_fwd_tc(const AttnParams& p, cudaStream_t st) {
   prm.H = p.H; prm.Hkv = p.Hkv; prm.Sq = p.Sq; prm.Skv = p.Skv;
   prm.c = p.scale * kLog2e;
   prm.causal = p.causal; prm.window = p.window;
+  prm.cu_q = p.cu_q; prm.cu_k = p.cu_k; prm.nseq = p.nseq;
   fwd_tc_set_out_map(prm, p);
   fwd_tc_set_mask(prm, p);
   if (cudaError_t me = fwd_tc_build_mask_tiles(prm, p, st); me != cudaSuccess) return me;

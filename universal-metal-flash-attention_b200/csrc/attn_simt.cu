@@ -122,10 +122,10 @@ __device__ __forceinline__ void store_out(void* base, int dtype, int64_t idx, fl
   else reinterpret_cast<__nv_bfloat16*>(base)[idx] = __float2bfloat16_rn(x);
 }
 
-// z (log2 domain) for element (row r, key c) from the raw dot product.
-__device__ __forceinline__ float logit(const AttnParams& p, int b, int h, int r, int c, float dot) {
-  bool hidden = (r >= p.Sq) || (c >= p.Skv) || (p.causal && c > r) || (p.window >= 0 && r > c + p.window);
-  if (hidden) return -CUDART_INF_F;
+// z (log2 domain) for element (row r, key c) from the raw dot product; `visible` comes from the causal / window / segment rule
+// (row_key_range / key_query_range).
+__device__ __forceinline__ float logit(const AttnParams& p, int b, int h, int r, int c, float dot, bool visible) {
+  if (!visible || r >= p.Sq || c >= p.Skv) return -CUDART_INF_F;
   float z = dot * p.scale;
   if (p.mask_kind != kMaskNone) z += mask_value(p, b, h, r, c);
   return z * kLog2e;
@@ -159,8 +159,10 @@ __global__ void __launch_bounds__(NT) fwd_simt_kernel(AttnParams p) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) acc[j][i] = 0.f;
 
+  __shared__ int rlo[TR], rhi[TR];      // visible keys of each row
+  if (threadIdx.x < TR) row_key_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, r0 + threadIdx.x, rlo[threadIdx.x], rhi[threadIdx.x]);
   int klo, khi;
-  visible_key_range(p.causal, p.window, p.Skv, r0, min(r0 + TR, p.Sq), klo, khi);
+  block_key_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, r0, min(r0 + TR, p.Sq), klo, khi);
   klo = (klo / TC) * TC;
   for (int c0 = klo; c0 < khi; c0 += TC) {
     __syncthreads();
@@ -172,7 +174,7 @@ __global__ void __launch_bounds__(NT) fwd_simt_kernel(AttnParams p) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       int r = ty * 4 + j;
-      float z = logit(p, b, h, r0 + r, c0 + tx, s[j]);
+      float z = logit(p, b, h, r0 + r, c0 + tx, s[j], c0 + tx >= rlo[r] && c0 + tx < rhi[r]);
       // row max across the warp (all 32 lanes share row r)
       float mx = z;
 #pragma unroll
@@ -270,8 +272,10 @@ __global__ void __launch_bounds__(NT) bwd_dq_simt_kernel(AttnParams p) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) acc[j][i] = 0.f;
 
+  __shared__ int rlo[TR], rhi[TR];      // visible keys of each row
+  if (threadIdx.x < TR) row_key_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, r0 + threadIdx.x, rlo[threadIdx.x], rhi[threadIdx.x]);
   int klo, khi;
-  visible_key_range(p.causal, p.window, p.Skv, r0, min(r0 + TR, p.Sq), klo, khi);
+  block_key_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, r0, min(r0 + TR, p.Sq), klo, khi);
   klo = (klo / TC) * TC;
   for (int c0 = klo; c0 < khi; c0 += TC) {
     __syncthreads();
@@ -284,7 +288,7 @@ __global__ void __launch_bounds__(NT) bwd_dq_simt_kernel(AttnParams p) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
       int r = ty * 4 + j;
-      float z = logit(p, b, h, r0 + r, c0 + tx, s[j]);
+      float z = logit(p, b, h, r0 + r, c0 + tx, s[j], c0 + tx >= rlo[r] && c0 + tx < rhi[r]);
       float L = row_L[r];
       float pv = (L == -CUDART_INF_F) ? 0.f : exp2f(z - L);
       Ss[r * (TC + 1) + tx] = pv * (dp[j] * p.scale - row_D[r]);
@@ -336,8 +340,10 @@ __global__ void __launch_bounds__(NT) bwd_dkv_simt_kernel(AttnParams p) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) { dk[j][i] = 0.f; dv[j][i] = 0.f; }
 
+  __shared__ int kqlo[TR], kqhi[TR];    // query rows that see each key
+  if (threadIdx.x < TR) key_query_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, c0 + threadIdx.x, kqlo[threadIdx.x], kqhi[threadIdx.x]);
   int qlo, qhi;
-  visible_query_range(p.causal, p.window, p.Sq, c0, min(c0 + TR, p.Skv), qlo, qhi);
+  block_query_range(p.causal, p.window, p.Sq, p.Skv, p.cu_q, p.cu_k, p.nseq, c0, min(c0 + TR, p.Skv), qlo, qhi);
   qlo = (qlo / TC) * TC;
   for (int g = 0; g < group; ++g) {
     const int h = hk * group + g;
@@ -359,7 +365,7 @@ __global__ void __launch_bounds__(NT) bwd_dkv_simt_kernel(AttnParams p) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
         int kc = ty * 4 + j;
-        float z = logit(p, b, h, r0 + tx, c0 + kc, s[j]);
+        float z = logit(p, b, h, r0 + tx, c0 + kc, s[j], r0 + tx >= kqlo[kc] && r0 + tx < kqhi[kc]);
         float L = row_L[tx];
         float pv = (L == -CUDART_INF_F) ? 0.f : exp2f(z - L);
         Ps[kc * (TC + 1) + tx] = pv;

@@ -56,6 +56,11 @@ struct AttnParams {
   int* mask_tile_scratch;
   int in_dtype, o_dtype, do_dtype;
   QuantView qq, qk, qv;     // used when in_dtype is kI8 / kI4
+  // packed variable-length sequences (B == 1): device int32 offsets [nseq + 1] of the segments along the query / key axis;
+  // null = dense.  See row_key_range.
+  const int* cu_q;
+  const int* cu_k;
+  int nseq;
 };
 
 // Visible key range [lo, hi) for query rows [r0, r1) under causal/window rules (used for tile skipping).
@@ -71,6 +76,88 @@ __host__ __device__ inline void visible_query_range(int causal, int window, int 
   lo = 0; hi = Sq;
   if (causal) { if (c0 > lo) lo = c0; }                        // rows >= c0
   if (window >= 0) { long h = (long)c1 - 1 + window + 1; if (h < hi) hi = (int)h; } // rows <= c1-1+window
+  if (hi < lo) hi = lo;
+}
+
+// ---- packed variable-length sequences.  Segment s holds query rows [cu_q[s], cu_q[s+1]) and keys [cu_k[s], cu_k[s+1]); a row
+// sees the keys of its own segment only, and causal / window apply to the offsets inside the segment (top-left aligned):
+// row i' = r - cu_q[s] hides key j' = c - cu_k[s] iff (causal && j' > i') || (window >= 0 && i' > j' + window).
+// Offsets come from device memory the host has not checked: every bound derived from them is clamped to [0, total], so a
+// malformed array gives wrong numbers but no access out of bounds.  cu == null is the dense problem (one segment, no clamps
+// needed).  Per-row lower and upper key bounds never decrease with the row (and per-key query bounds with the key), so the
+// range of a block of rows / keys is the lower bound of its first and the upper bound of its last.
+
+__host__ __device__ inline int seg_offset(const int* cu, int s, int total) {
+  const int v = cu[s];
+  return v < 0 ? 0 : v > total ? total : v;
+}
+
+// s in [0, nseq) with cu[s] <= t < cu[s+1] (binary search; 0 / nseq - 1 past either end)
+__host__ __device__ inline int segment_of(const int* cu, int nseq, int t) {
+  int lo = 0, hi = nseq - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (cu[mid] <= t) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// Visible keys [lo, hi) of query row r.
+__host__ __device__ inline void row_key_range(int causal, int window, int Sq, int Skv, const int* cu_q, const int* cu_k, int nseq,
+                                              int r, int& lo, int& hi) {
+  if (!cu_q) {
+    lo = window >= 0 ? max(0, r - window) : 0;
+    hi = (causal ? min(Skv - 1, r) : Skv - 1) + 1;
+    return;
+  }
+  const int s = segment_of(cu_q, nseq, r);
+  const int i = r - seg_offset(cu_q, s, Sq);
+  const int kb = seg_offset(cu_k, s, Skv);
+  int ke = seg_offset(cu_k, s + 1, Skv);
+  if (ke < kb) ke = kb;
+  lo = kb; hi = ke;
+  if (causal && i < ke - kb) hi = kb + (i < 0 ? 0 : i + 1);             // j' <= i'
+  if (window >= 0 && i > window) lo = i - window < ke - kb ? kb + (i - window) : ke;   // j' >= i' - window
+  if (hi < lo) hi = lo;
+}
+
+// Query rows [lo, hi) that see key c.  Dense: not clipped at Sq (rows past Sq carry L = +inf, P = 0).
+__host__ __device__ inline void key_query_range(int causal, int window, int Sq, int Skv, const int* cu_q, const int* cu_k, int nseq,
+                                                int c, int& lo, int& hi) {
+  if (!cu_k) {
+    lo = causal ? c : 0;
+    hi = (window >= 0 ? min(c + window, 1 << 30) : (1 << 30)) + 1;
+    return;
+  }
+  const int s = segment_of(cu_k, nseq, c);
+  int j = c - seg_offset(cu_k, s, Skv);
+  const int qb = seg_offset(cu_q, s, Sq);
+  int qe = seg_offset(cu_q, s + 1, Sq);
+  if (qe < qb) qe = qb;
+  if (j < 0) j = 0;
+  lo = qb; hi = qe;
+  if (causal) lo = j < qe - qb ? qb + j : qe;                            // i' >= j'
+  if (window >= 0 && (long long)j + window + 1 < qe - qb) hi = qb + j + window + 1;   // i' <= j' + window
+  if (hi < lo) hi = lo;
+}
+
+// Visible keys [lo, hi) of query rows [r0, r1), r1 > r0.
+__host__ __device__ inline void block_key_range(int causal, int window, int Sq, int Skv, const int* cu_q, const int* cu_k, int nseq,
+                                                int r0, int r1, int& lo, int& hi) {
+  if (!cu_q) { visible_key_range(causal, window, Skv, r0, r1, lo, hi); return; }
+  int l2, h2;
+  row_key_range(causal, window, Sq, Skv, cu_q, cu_k, nseq, r0, lo, h2);
+  row_key_range(causal, window, Sq, Skv, cu_q, cu_k, nseq, r1 - 1, l2, hi);
+  if (hi < lo) hi = lo;
+}
+
+// Query rows [lo, hi) that see any of the keys [c0, c1), c1 > c0.
+__host__ __device__ inline void block_query_range(int causal, int window, int Sq, int Skv, const int* cu_q, const int* cu_k, int nseq,
+                                                  int c0, int c1, int& lo, int& hi) {
+  if (!cu_k) { visible_query_range(causal, window, Sq, c0, c1, lo, hi); return; }
+  int l2, h2;
+  key_query_range(causal, window, Sq, Skv, cu_q, cu_k, nseq, c0, lo, h2);
+  key_query_range(causal, window, Sq, Skv, cu_q, cu_k, nseq, c1 - 1, l2, hi);
   if (hi < lo) hi = lo;
 }
 

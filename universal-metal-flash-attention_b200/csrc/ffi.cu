@@ -344,6 +344,34 @@ void init_params(AttnParams& p, uint32_t B, uint32_t H, uint32_t Sq, uint32_t Sk
   p.o_dtype = kF32; p.do_dtype = kF32;
 }
 
+// Packed variable-length sequences: the device offsets the kernels read (null buffers = dense).
+void set_segments(AttnParams& p, const Buffer* cu_q, const Buffer* cu_k, uint32_t nseq) {
+  if (!cu_q || !cu_k) return;
+  p.cu_q = reinterpret_cast<const int*>(cu_q->dev);
+  p.cu_k = reinterpret_cast<const int*>(cu_k->dev);
+  p.nseq = (int)nseq;
+}
+
+// Arguments every varlen entry point checks before any device work: handles and num_seqs, then (with a device) sizes and --
+// where the host can read them (host mirrors, managed memory) -- the offsets themselves: 0, non-decreasing, ending at the total.  Device-resident offsets are left to
+// the kernels, which clamp every bound they derive from them (common.h).
+mfa_error_t check_segments(const Buffer* cu_q, const Buffer* cu_k, uint32_t nseq, uint32_t total_q, uint32_t total_k) {
+  if (!cu_q || !cu_k || nseq == 0 || nseq > 0x7ffffffeu) return MFA_ERROR_INVALID_ARGS;
+  if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
+  const size_t bytes = ((size_t)nseq + 1) * sizeof(int32_t);
+  if (cu_q->bytes < bytes || cu_k->bytes < bytes || cu_q->ndim || cu_k->ndim) return MFA_ERROR_INVALID_ARGS;
+  if (total_q > 0x7fffffffu || total_k > 0x7fffffffu) return MFA_ERROR_INVALID_ARGS;
+  const struct { const Buffer* b; uint32_t total; } arrays[2] = {{cu_q, total_q}, {cu_k, total_k}};
+  for (const auto& a : arrays) {
+    if (!a.b->host) continue;
+    const int32_t* cu = reinterpret_cast<const int32_t*>(a.b->host);
+    if (cu[0] != 0 || cu[nseq] != (int64_t)a.total) return MFA_ERROR_INVALID_ARGS;
+    for (uint32_t s = 0; s < nseq; ++s)
+      if (cu[s + 1] < cu[s]) return MFA_ERROR_INVALID_ARGS;
+  }
+  return MFA_SUCCESS;
+}
+
 struct Timer {
   Context* ctx; cudaStream_t st; bool on;
   Timer(Context* c, cudaStream_t s, bool enable) : ctx(c), st(s), on(enable) { if (on) cudaEventRecord(ctx->ev0, st); }
@@ -365,6 +393,9 @@ struct FwdArgs {
   bool tq, tk, tv, to;
   MaskArgs mask;
   cudaStream_t user_stream; bool async;
+  // packed variable-length sequences (mfa_attention_forward_varlen): K / V heads (0 = H) and the segment offsets
+  uint32_t Hkv;
+  Buffer *cu_q, *cu_k; uint32_t nseq;
 };
 
 bool valid_float_dtype(int d) { return d == kF16 || d == kBF16 || d == kF32; }
@@ -395,7 +426,7 @@ size_t pipeline_chunk_bytes() {
 }
 
 bool forward_pipeline_ok(const FwdArgs& a, int o_dtype) {
-  if (a.async || getenv("MFA_DISABLE_PIPELINE")) return false;
+  if (a.async || a.cu_q || getenv("MFA_DISABLE_PIPELINE")) return false;
   if (!a.q->mirrored || !a.k->mirrored || !a.v->mirrored || !a.out->mirrored || (a.lse && !a.lse->mirrored)) return false;
   if (a.q->ndim || a.k->ndim || a.v->ndim || a.out->ndim) return false;
   if (a.tq || a.tk || a.tv || a.to) return false;
@@ -464,11 +495,13 @@ mfa_error_t forward_core(Context* ctx, const FwdArgs& a) {
   if (!ctx || !a.q || !a.k || !a.v || !a.out) return MFA_ERROR_INVALID_ARGS;
   if (!valid_float_dtype(a.in_dtype)) return MFA_ERROR_INVALID_ARGS;
   if (a.D == 0 || a.D > 256 || a.H == 0) return MFA_ERROR_INVALID_ARGS;
+  const uint32_t Hkv = a.Hkv ? a.Hkv : a.H;
+  if (a.H % Hkv) return MFA_ERROR_INVALID_ARGS;
   if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
-  const size_t nq = elems(a.B, a.H, a.Sq, a.D), nkv = elems(a.B, a.H, a.Skv, a.D);
+  const size_t nq = elems(a.B, a.H, a.Sq, a.D), nkv = elems(a.B, Hkv, a.Skv, a.D);
   const size_t esz = dtype_bytes(a.in_dtype);
-  if (!view_fits(a.q, a.B, a.H, a.Sq, a.D, esz) || !view_fits(a.k, a.B, a.H, a.Skv, a.D, esz) ||
-      !view_fits(a.v, a.B, a.H, a.Skv, a.D, esz))
+  if (!view_fits(a.q, a.B, a.H, a.Sq, a.D, esz) || !view_fits(a.k, a.B, Hkv, a.Skv, a.D, esz) ||
+      !view_fits(a.v, a.B, Hkv, a.Skv, a.D, esz))
     return MFA_ERROR_INVALID_ARGS;
   // O is fp32 (reference contract) unless the handle only fits the requested lower precision.
   int o_dtype = kF32;
@@ -477,7 +510,8 @@ mfa_error_t forward_core(Context* ctx, const FwdArgs& a) {
     else return MFA_ERROR_INVALID_ARGS;
   }
   if (a.lse && a.lse->bytes < (size_t)a.B * a.H * a.Sq * 4) return MFA_ERROR_INVALID_ARGS;
-  if (a.async && (a.q->mirrored || a.k->mirrored || a.v->mirrored || a.out->mirrored || (a.lse && a.lse->mirrored)))
+  if (a.async && (a.q->mirrored || a.k->mirrored || a.v->mirrored || a.out->mirrored || (a.lse && a.lse->mirrored) ||
+                  (a.cu_q && (a.cu_q->mirrored || a.cu_k->mirrored))))
     return MFA_ERROR_INVALID_ARGS;
 
   std::lock_guard<std::recursive_mutex> lock(ctx->mu);
@@ -498,18 +532,21 @@ mfa_error_t forward_core(Context* ctx, const FwdArgs& a) {
   ScratchScope scope(ctx, st);
   Sync sync{ctx, st, a.async, {}};
   cudaError_t e;
-  if ((e = sync.in(a.q)) != cudaSuccess || (e = sync.in(a.k)) != cudaSuccess || (e = sync.in(a.v)) != cudaSuccess)
+  if ((e = sync.in(a.q)) != cudaSuccess || (e = sync.in(a.k)) != cudaSuccess || (e = sync.in(a.v)) != cudaSuccess ||
+      (e = sync.in(a.cu_q)) != cudaSuccess || (e = sync.in(a.cu_k)) != cudaSuccess)
     return cuda_fail(e, "h2d");
   if (nq == 0) { return sync.finish() == cudaSuccess ? MFA_SUCCESS : MFA_ERROR_EXECUTION_FAILED; }
 
   AttnParams p;
   init_params(p, a.B, a.H, a.Sq, a.Skv, a.D, a.scale, a.causal, a.window);
+  p.Hkv = (int)Hkv;
   p.q = view_of(a.q, a.H, a.Sq, a.D, a.tq);
-  p.k = view_of(a.k, a.H, a.Skv, a.D, a.tk);
-  p.v = view_of(a.v, a.H, a.Skv, a.D, a.tv);
+  p.k = view_of(a.k, Hkv, a.Skv, a.D, a.tk);
+  p.v = view_of(a.v, Hkv, a.Skv, a.D, a.tv);
   p.o = view_of(a.out, a.H, a.Sq, a.D, a.to);
   p.lse = a.lse ? reinterpret_cast<float*>(a.lse->dev) : nullptr;
   p.in_dtype = a.in_dtype; p.o_dtype = o_dtype;
+  set_segments(p, a.cu_q, a.cu_k, a.nseq);
   mfa_error_t me = setup_mask(scope, st, a.mask, p);
   if (me != MFA_SUCCESS) return me;
 
@@ -547,6 +584,7 @@ struct BwdArgs {
   QuantView qq, qk, qv;
   cudaStream_t user_stream; bool async;
   bool want_dq, want_dkv;
+  Buffer *cu_q, *cu_k; uint32_t nseq;         // packed variable-length sequences (mfa_attention_backward_varlen)
 };
 
 mfa_error_t backward_core(Context* ctx, const BwdArgs& a) {
@@ -570,8 +608,9 @@ mfa_error_t backward_core(Context* ctx, const BwdArgs& a) {
   cudaStream_t st = a.async ? a.user_stream : ctx->stream;
   ScratchScope scope(ctx, st);
   Sync sync{ctx, st, a.async, {}};
-  Buffer* ins[] = {a.dout, a.q, a.k, a.v, a.out, a.lse};
+  Buffer* ins[] = {a.dout, a.q, a.k, a.v, a.out, a.lse, a.cu_q, a.cu_k};
   for (Buffer* b : ins) {
+    if (!b) continue;
     if (a.async && b->mirrored) return MFA_ERROR_INVALID_ARGS;
     cudaError_t e = sync.in(b);
     if (e != cudaSuccess) return cuda_fail(e, "h2d");
@@ -589,6 +628,7 @@ mfa_error_t backward_core(Context* ctx, const BwdArgs& a) {
   p.lse = reinterpret_cast<float*>(a.lse->dev);
   p.in_dtype = a.in_dtype; p.o_dtype = kF32; p.do_dtype = a.do_dtype;
   p.qq = a.qq; p.qk = a.qk; p.qv = a.qv;
+  set_segments(p, a.cu_q, a.cu_k, a.nseq);
   p.dq = a.want_dq ? reinterpret_cast<float*>(a.dq->dev) : nullptr;
   p.dk = a.want_dkv ? reinterpret_cast<float*>(a.dk->dev) : nullptr;
   p.dv = a.want_dkv ? reinterpret_cast<float*>(a.dv->dev) : nullptr;
@@ -1179,6 +1219,40 @@ mfa_error_t mfa_attention_backward_ex(
             window_size < 0 ? -1 : window_size, dt, dt, false, false, false, false,
             MaskArgs{mask_ptr, mask_size_bytes, mask_shape, mask_strides, mask_ndim, mask_type, mask_scalar_type},
             none, none, none, reinterpret_cast<cudaStream_t>(stream), stream != nullptr, true, true};
+  return backward_core(C_(context), a);
+}
+
+mfa_error_t mfa_attention_forward_varlen(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k, mfa_buffer_t v, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cu_seqlens_k, uint32_t num_seqs, uint32_t total_q, uint32_t total_k,
+    uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim, float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream) {
+  if (!context || !q || !k || !v || !out) return MFA_ERROR_INVALID_ARGS;
+  if (mfa_error_t e = check_segments(B_(cu_seqlens_q), B_(cu_seqlens_k), num_seqs, total_q, total_k); e != MFA_SUCCESS) return e;
+  FwdArgs a{B_(q), B_(k), B_(v), B_(out), B_(lse), 1, total_q, total_k, num_heads, head_dim,
+            softmax_scale, causal, window_size < 0 ? -1 : window_size, header_precision_to_dtype(input_precision),
+            header_precision_to_dtype(output_precision), false, false, false, false,
+            MaskArgs{nullptr, 0, nullptr, nullptr, 0, 0, 0}, reinterpret_cast<cudaStream_t>(stream), stream != nullptr,
+            num_kv_heads, B_(cu_seqlens_q), B_(cu_seqlens_k), num_seqs};
+  return forward_core(C_(context), a);
+}
+
+mfa_error_t mfa_attention_backward_varlen(
+    mfa_context_t context, mfa_buffer_t dout, mfa_buffer_t q, mfa_buffer_t k, mfa_buffer_t v, mfa_buffer_t out,
+    mfa_buffer_t softmax_lse, mfa_buffer_t dq, mfa_buffer_t dk, mfa_buffer_t dv, mfa_buffer_t d_buffer,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cu_seqlens_k, uint32_t num_seqs, uint32_t total_q, uint32_t total_k,
+    uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim, float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, void* stream) {
+  if (!context || !dout || !q || !k || !v || !out || !softmax_lse || !dq || !dk || !dv) return MFA_ERROR_INVALID_ARGS;
+  if (mfa_error_t e = check_segments(B_(cu_seqlens_q), B_(cu_seqlens_k), num_seqs, total_q, total_k); e != MFA_SUCCESS) return e;
+  const int dt = header_precision_to_dtype(input_precision);
+  if (!valid_float_dtype(dt)) return MFA_ERROR_INVALID_ARGS;
+  QuantView none{nullptr, 1.f, 0, 0};
+  BwdArgs a{B_(dout), B_(q), B_(k), B_(v), B_(out), B_(softmax_lse), B_(dq), B_(dk), B_(dv), B_(d_buffer),
+            1, total_q, total_k, num_heads, num_kv_heads ? num_kv_heads : num_heads, head_dim, softmax_scale, causal,
+            window_size < 0 ? -1 : window_size, dt, dt, false, false, false, false,
+            MaskArgs{nullptr, 0, nullptr, nullptr, 0, 0, 0}, none, none, none, reinterpret_cast<cudaStream_t>(stream),
+            stream != nullptr, true, true, B_(cu_seqlens_q), B_(cu_seqlens_k), num_seqs};
   return backward_core(C_(context), a);
 }
 

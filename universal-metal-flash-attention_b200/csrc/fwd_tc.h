@@ -55,6 +55,9 @@ struct FwdTcParams {
   const int* mtiles;       // [lists][m_nkt]
   const int* mcounts;      // [lists]
   int m_nkt;
+  const int* cu_q;         // packed variable-length sequences (AttnParams::cu_q / cu_k / nseq), or null
+  const int* cu_k;
+  int nseq;
 };
 
 bool fwd_tc_mask_ok(const AttnParams& p);

@@ -225,6 +225,93 @@ def metal_flash_attention_autograd(query, key, value, is_causal=False, scale=0.0
     return MetalFlashAttentionFn.apply(query, key, value, is_causal, scale, attn_mask)
 
 
+def _thd_handle(bind, t):
+    """[total, heads, D] tensor (unit stride along D) -> a [1, heads, total, D] strided handle over the same memory."""
+    T, Hn, D = t.shape
+    shape = (ctypes.c_int64 * 4)(1, Hn, T, D)
+    strides = (ctypes.c_int64 * 4)(T * t.stride(0), t.stride(1), t.stride(0), t.stride(2))
+    h = _ffi.mfa_buffer_t()
+    nbytes = max(((T - 1) * t.stride(0) + (Hn - 1) * t.stride(1) + D) * t.element_size(), 1)
+    _ffi._check_error(_lib.mfa_buffer_from_mtl_buffer_with_strides(bind.ctx.handle, ctypes.c_void_p(t.data_ptr()), nbytes,
+                                                                   shape, strides, 4, ctypes.byref(h)))
+    bind.handles.append(h)
+    return h
+
+
+class MetalFlashAttentionVarlenFn(torch.autograd.Function):
+    """Packed variable-length attention: forward saves (q, k, v, O fp32 [Hq, total_q, D], L); dK / dV come back per KV head."""
+
+    @staticmethod
+    def forward(ctx, query, key, value, cu_q, cu_k, is_causal, scale, window):
+        dev = query.device
+        T, H, D = query.shape
+        Tk, Hkv = key.shape[0], key.shape[1]
+        out32 = torch.empty((H, T, D), device=dev, dtype=torch.float32)
+        lse = torch.empty((H, T), device=dev, dtype=torch.float32)
+        lib_ctx = _context(dev)
+        stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream or 0), query)
+        with _Bound(lib_ctx) as bind:
+            rc = _lib.mfa_attention_forward_varlen(
+                lib_ctx.handle, _thd_handle(bind, query), _thd_handle(bind, key), _thd_handle(bind, value), bind(out32),
+                bind(lse), bind(cu_q), bind(cu_k), cu_q.numel() - 1, T, Tk, H, Hkv, D, float(scale), bool(is_causal),
+                int(window), _PREC[query.dtype], _ffi.MFA_PRECISION_FP32, stream)
+        if rc != 0:
+            raise RuntimeError(f"Metal Flash Attention varlen forward failed with code {rc}: {_ffi._get_error_string(rc)}")
+        ctx.save_for_backward(query, key, value, out32, lse, cu_q, cu_k)
+        ctx.is_causal, ctx.scale, ctx.window = bool(is_causal), float(scale), int(window)
+        out = out32.transpose(0, 1)
+        return out.contiguous() if query.dtype == torch.float32 else out.to(query.dtype)
+
+    @staticmethod
+    def backward(ctx, d_output):
+        query, key, value, out32, lse, cu_q, cu_k = ctx.saved_tensors
+        dev = query.device
+        T, H, D = query.shape
+        Tk, Hkv = key.shape[0], key.shape[1]
+        d_out = d_output.to(query.dtype).transpose(0, 1).contiguous()          # [H, total_q, D]
+        dq = torch.empty((H, T, D), device=dev, dtype=torch.float32)
+        dk = torch.empty((Hkv, Tk, D), device=dev, dtype=torch.float32)
+        dv = torch.empty((Hkv, Tk, D), device=dev, dtype=torch.float32)
+        dbuf = torch.empty((H * T,), device=dev, dtype=torch.float32)
+        lib_ctx = _context(dev)
+        stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream or 0), query)
+        with _Bound(lib_ctx) as bind:
+            rc = _lib.mfa_attention_backward_varlen(
+                lib_ctx.handle, bind(d_out), _thd_handle(bind, query), _thd_handle(bind, key), _thd_handle(bind, value),
+                bind(out32), bind(lse), bind(dq), bind(dk), bind(dv), bind(dbuf), bind(cu_q), bind(cu_k), cu_q.numel() - 1,
+                T, Tk, H, Hkv, D, ctx.scale, ctx.is_causal, ctx.window, _PREC[query.dtype], stream)
+        if rc != 0:
+            raise RuntimeError(f"Metal Flash Attention varlen backward failed with code {rc}: {_ffi._get_error_string(rc)}")
+        dq, dk, dv = (g.transpose(0, 1).to(query.dtype).contiguous() for g in (dq, dk, dv))
+        return dq, dk, dv, None, None, None, None, None
+
+
+def metal_flash_attention_varlen(q, k, v, cu_seqlens_q, cu_seqlens_k, is_causal=False, scale=None, window=-1):
+    """Attention over sequences packed along the token axis, without a dense mask.  q is [total_q, Hq, D], k / v
+    [total_k, Hkv, D] (Hkv divides Hq: grouped-query attention without copies of K / V); cu_seqlens_q / cu_seqlens_k are int32
+    CUDA tensors of num_seqs + 1 offsets (0, non-decreasing, ending at total_q / total_k).  Query row i of segment s sees the keys
+    of segment s only; is_causal and window (>= 0: keys more than `window` positions behind are hidden) apply to the positions
+    inside the segment, top-left aligned.  Returns O [total_q, Hq, D] in q's dtype; differentiable in q, k, v.  Enqueued on
+    torch's current stream.  A row that sees no key gets O = 0."""
+    for t in (q, k, v):
+        if not t.is_cuda or t.dim() != 3 or t.stride(-1) != 1:
+            raise RuntimeError("metal_flash_attention_varlen: q, k, v must be 3-D CUDA tensors [total, heads, head_dim] "
+                               "with unit stride along head_dim")
+    if q.dtype not in _PREC or k.dtype != q.dtype or v.dtype != q.dtype:
+        raise RuntimeError("metal_flash_attention_varlen: q, k, v must share one of float16, bfloat16, float32")
+    if k.shape != v.shape or k.size(2) != q.size(2) or q.size(1) % k.size(1):
+        raise RuntimeError(f"metal_flash_attention_varlen: shapes q={tuple(q.shape)} k={tuple(k.shape)} v={tuple(v.shape)}")
+    for c in (cu_seqlens_q, cu_seqlens_k):
+        if c.dtype != torch.int32 or c.dim() != 1 or c.device != q.device or not c.is_contiguous():
+            raise RuntimeError("metal_flash_attention_varlen: cu_seqlens must be contiguous 1-D int32 tensors on q's device")
+    if cu_seqlens_q.numel() != cu_seqlens_k.numel() or cu_seqlens_q.numel() < 2:
+        raise RuntimeError("metal_flash_attention_varlen: cu_seqlens_q / cu_seqlens_k need the same num_seqs + 1 >= 2 entries")
+    if scale is None or scale <= 0.0:
+        scale = 1.0 / math.sqrt(q.size(-1))
+    return MetalFlashAttentionVarlenFn.apply(q, k, v, cu_seqlens_q, cu_seqlens_k, is_causal, scale,
+                                             -1 if window is None or window < 0 else int(window))
+
+
 def _dense_mask_f32(mask, query, Skv):
     """The quantised entry points take NULL or a dense fp32 additive [B,H,Sq,Skv] mask (metal_sdpa_backend.cpp:3210-3231)."""
     if mask is None:

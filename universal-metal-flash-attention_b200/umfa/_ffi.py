@@ -62,6 +62,7 @@ _ctx, _buf, _u32, _u16, _i32, _f32, _b, _sz, _vp, _i64, _u64 = (
 _pi64 = _c.POINTER(_c.c_int64)
 _DIMS = [_u32, _u32, _u32, _u32, _u16]                  # batch, seq_q, seq_kv, heads, head_dim
 _MASK = [_vp, _sz, _pi64, _pi64, _u32, _i32, _i32]     # ptr, bytes, shape, strides, ndim, type, scalar
+_VARLEN = [_u32, _u32, _u32, _u32, _u32, _u16]         # num_seqs, total_q, total_k, heads, kv heads, head_dim
 _QPARAMS = [_f32, _i32, _f32, _i32, _f32, _i32]
 _T4 = [_b, _b, _b, _b]
 
@@ -128,6 +129,8 @@ SIGNATURES = {
                                  _MASK + [_vp]),
     "mfa_attention_forward_accumulate": (_i32, [_ctx, _buf, _buf, _buf, _buf, _buf] + _DIMS + [_f32, _b, _i32, _i32, _u32, _u32, _vp]),
     "mfa_attention_backward_ex": (_i32, [_ctx] + [_buf] * 10 + _DIMS + [_f32, _b, _i32, _i32] + _MASK + [_vp]),
+    "mfa_attention_forward_varlen": (_i32, [_ctx] + [_buf] * 7 + _VARLEN + [_f32, _b, _i32, _i32, _i32, _vp]),
+    "mfa_attention_backward_varlen": (_i32, [_ctx] + [_buf] * 12 + _VARLEN + [_f32, _b, _i32, _i32, _vp]),
     "mfa_quantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _i32, _f32, _vp]),
     "mfa_dequantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _vp]),
     "mfa_merge_partials": (_i32, [_ctx, _buf, _buf, _buf, _buf, _u64, _u32, _vp]),

@@ -362,6 +362,100 @@ def flash_attention_backward(context: MFAContext, d_out, q, k, v, out, lse, *, a
     return dq, dk, dv, (dterm.reshape(d.Sq) if q.ndim == 2 else dterm)
 
 
+def _varlen_dims(q, k, v, cu_seqlens_q, cu_seqlens_k, layout: str):
+    """(H, Hkv, total_q, total_k, D, cu_q, cu_k) of packed [total, heads, D] ("thd") or [heads, total, D] ("hsd") operands."""
+    if not all(isinstance(x, np.ndarray) and x.ndim == 3 for x in (q, k, v)):
+        raise ValueError("varlen q, k, v must be 3-D numpy arrays")
+    if layout == "thd":
+        (Tq, H, D), (Tk, Hkv, Dk) = q.shape, k.shape
+    elif layout == "hsd":
+        (H, Tq, D), (Hkv, Tk, Dk) = q.shape, k.shape
+    else:
+        raise ValueError("layout must be 'thd' or 'hsd'")
+    if v.shape != k.shape or Dk != D or Hkv == 0 or H % Hkv:
+        raise ValueError(f"Shape mismatch: q={q.shape}, k={k.shape}, v={v.shape}")
+    cu_q = np.ascontiguousarray(cu_seqlens_q, np.int32)
+    cu_k = np.ascontiguousarray(cu_seqlens_k, np.int32)
+    if cu_q.ndim != 1 or cu_q.shape != cu_k.shape or cu_q.size < 2:
+        raise ValueError("cu_seqlens_q / cu_seqlens_k must be 1-D int32 arrays of num_seqs + 1 offsets")
+    return H, Hkv, Tq, Tk, D, cu_q, cu_k
+
+
+def _varlen_operand(ctx, arr, heads: int, total: int, D: int, layout: str):
+    """[total, heads, D] arrays travel as [1, heads, total, D] element strides; [heads, total, D] as they are."""
+    if layout == "thd":
+        return MFABuffer(ctx, arr, shape=(1, heads, total, D), strides=(total * heads * D, D, heads * D, 1))
+    return MFABuffer(ctx, arr)
+
+
+def flash_attention_varlen_forward(context: MFAContext, q, k, v, cu_seqlens_q, cu_seqlens_k, *, causal: bool = False,
+                                   softmax_scale: Optional[float] = None, input_precision: Precision = "fp16",
+                                   window_size: Optional[int] = None, layout: str = "thd"):
+    """Attention over sequences packed along the token axis (mfa_attention_forward_varlen): segment s holds query rows
+    cu_seqlens_q[s]:cu_seqlens_q[s+1] and keys cu_seqlens_k[s]:cu_seqlens_k[s+1]; a row sees only its own segment's keys, causal /
+    window_size apply inside the segment (top-left aligned).  q is [total_q, H, D], k / v [total_k, Hkv, D] (layout="hsd":
+    [H, total, D]); Hkv divides H (grouped-query attention).  bf16 inputs are uint16 bit patterns with input_precision="bf16".
+    Returns (O fp32 shaped like q, L fp32 [H, total_q] in log2 units; rows that see no key: O = 0, L = -inf)."""
+    H, Hkv, Tq, Tk, D, cu_q, cu_k = _varlen_dims(q, k, v, cu_seqlens_q, cu_seqlens_k, layout)
+    if softmax_scale is None:
+        softmax_scale = 1.0 / np.sqrt(D)
+    in_prec = _parse_precision(input_precision)
+    for name, x in (("q", q), ("k", k), ("v", v)):
+        _check_input_dtype(x, in_prec, name)
+    out = np.zeros(q.shape, np.float32)
+    lse = np.zeros((H, Tq), np.float32)
+    bufs = [_varlen_operand(context, np.ascontiguousarray(q), H, Tq, D, layout),
+            _varlen_operand(context, np.ascontiguousarray(k), Hkv, Tk, D, layout),
+            _varlen_operand(context, np.ascontiguousarray(v), Hkv, Tk, D, layout),
+            _varlen_operand(context, out, H, Tq, D, layout), MFABuffer(context, lse),
+            MFABuffer(context, cu_q), MFABuffer(context, cu_k)]
+    try:
+        _check_error(_lib.mfa_attention_forward_varlen(
+            context.handle, *[b.handle for b in bufs], cu_q.size - 1, Tq, Tk, H, Hkv, D, softmax_scale, causal,
+            -1 if window_size is None else int(window_size), in_prec, MFA_PRECISION_FP32, None))
+    finally:
+        for b in bufs:
+            b.close()
+    return out, lse
+
+
+def flash_attention_varlen_backward(context: MFAContext, d_out, q, k, v, out, lse, cu_seqlens_q, cu_seqlens_k, *,
+                                    causal: bool = False, softmax_scale: Optional[float] = None,
+                                    input_precision: Precision = "fp32", window_size: Optional[int] = None,
+                                    layout: str = "thd"):
+    """dQ, dK, dV (fp32, shaped like q / k / v) and D ([H, total_q]) of flash_attention_varlen_forward
+    (mfa_attention_backward_varlen).  d_out, q, k, v share input_precision; out / lse are the forward's fp32 results.
+    With Hkv < H, dK / dV hold the sums over each group of query heads."""
+    H, Hkv, Tq, Tk, D, cu_q, cu_k = _varlen_dims(q, k, v, cu_seqlens_q, cu_seqlens_k, layout)
+    if softmax_scale is None:
+        softmax_scale = 1.0 / np.sqrt(D)
+    in_prec = _parse_precision(input_precision)
+    for name, x in (("q", q), ("k", k), ("v", v), ("d_out", d_out)):
+        _check_input_dtype(x, in_prec, name)
+    hsd = (lambda x: np.ascontiguousarray(x.transpose(1, 0, 2))) if layout == "thd" else np.ascontiguousarray
+    dq = np.zeros((H, Tq, D), np.float32)
+    dk = np.zeros((Hkv, Tk, D), np.float32)
+    dv = np.zeros((Hkv, Tk, D), np.float32)
+    dterm = np.zeros((H, Tq), np.float32)
+    bufs = [MFABuffer(context, hsd(d_out)),
+            _varlen_operand(context, np.ascontiguousarray(q), H, Tq, D, layout),
+            _varlen_operand(context, np.ascontiguousarray(k), Hkv, Tk, D, layout),
+            _varlen_operand(context, np.ascontiguousarray(v), Hkv, Tk, D, layout),
+            MFABuffer(context, hsd(np.asarray(out, np.float32))), MFABuffer(context, np.ascontiguousarray(lse, np.float32)),
+            MFABuffer(context, dq), MFABuffer(context, dk), MFABuffer(context, dv), MFABuffer(context, dterm),
+            MFABuffer(context, cu_q), MFABuffer(context, cu_k)]
+    try:
+        _check_error(_lib.mfa_attention_backward_varlen(
+            context.handle, *[b.handle for b in bufs], cu_q.size - 1, Tq, Tk, H, Hkv, D, softmax_scale, causal,
+            -1 if window_size is None else int(window_size), in_prec, None))
+    finally:
+        for b in bufs:
+            b.close()
+    if layout == "thd":
+        dq, dk, dv = (np.ascontiguousarray(x.transpose(1, 0, 2)) for x in (dq, dk, dv))
+    return dq, dk, dv, dterm
+
+
 def attention(q, k, v, context: Optional[MFAContext] = None, **kwargs):
     """flash_attention_forward with automatic context management."""
     if context is not None:
