@@ -239,6 +239,39 @@ mfa_error_t mfa_attention_backward_varlen(
     uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim, float softmax_scale, bool causal, int32_t window_size,
     mfa_precision_t input_precision, void* stream);
 
+/* Attention of seq_len_q new query tokens per sequence against that sequence's K/V cache (decode, speculative decode,
+ * chunked prefill).  Forward only.
+ * q is a [batch_size, num_heads, seq_len_q, D] view (strided handles give [B, Sq, H, D]); out has the same shape in
+ * output_precision (fp32, bf16 or fp16, may be strided); lse fp32 [B, num_heads, seq_len_q] (log2 units) or NULL.
+ * Contiguous cache (page_size == 0, block_table NULL): k_cache / v_cache are [B, num_kv_heads, cache_capacity, D] views (strided
+ * handles give [B, cache_capacity, num_kv_heads, D]).  Paged cache (page_size > 0): k_cache / v_cache are contiguous
+ * [num_pages, page_size, num_kv_heads, D] pools and block_table is int32 [B, cache_capacity / page_size], row-major: key j of
+ * sequence b is row j % page_size of page block_table[b][j / page_size].  page_size is a multiple of 16 and divides
+ * cache_capacity.
+ * cache_seqlens is int32 [B]: L_b valid keys of sequence b, the seq_len_q new tokens included (the caller writes their K / V into
+ * the cache first).  Query row s sits at position p = L_b - seq_len_q + s and sees key j < L_b iff (!causal || j <= p) &&
+ * (window_size < 0 || p - j <= window_size) (bottom-right alignment).  A row that sees no key (L_b = 0, or L_b < seq_len_q under
+ * causal) gets O = 0, L = -inf.  Cache rows past L_b are read as part of their 128-key tile and must hold finite values.
+ * num_kv_heads divides num_heads (0 = num_heads), num_heads / num_kv_heads <= 128; bf16 / fp16 operands, head_dim a multiple of 8
+ * up to 128.  Anything else returns MFA_ERROR_INVALID_ARGS.
+ * Host-readable cache_seqlens / block_table (host or managed memory) are checked: lengths in [0, cache_capacity], page ids in
+ * [0, num_pages).  Device-resident ones are not read by the host; the kernels clamp lengths to [0, cache_capacity] and page ids
+ * to [0, num_pages), so malformed arrays give wrong numbers but no access out of bounds.
+ * The keys of long caches are split over several work items whose partials a second kernel merges; how many depends on the
+ * shape and the GPU only, never on the lengths, so results are deterministic.  With stream != NULL the call only enqueues work:
+ * no host synchronisation, no host read of device memory, and no allocation once the context's scratch has been sized for the
+ * shape by an earlier call.  Such a call can be captured in a CUDA graph and replayed with new cache_seqlens and cache contents;
+ * make one call of the shape outside the capture first (during capture a call that would have to grow the scratch returns
+ * MFA_ERROR_MEMORY_ALLOCATION).  A scratch block a graph has captured is never freed before the context: a later call that needs
+ * more scratch gets a new block.  Replays and other calls on the context order themselves through an event, on any stream. */
+mfa_error_t mfa_attention_forward_kvcache(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t batch_size, uint32_t seq_len_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream);
+
 /* Device quantiser (GEMMQuantization.swift:305-623 / GEMMRuntimeQuantization.swift:80-181 contract):
  * src is a row-major [rows, cols] matrix of src_precision; scale[b] = absmax(block b) / 127 (int8) or / 7
  * (int4), floored at scale_floor when scale_floor > 0 (the reference GPU path uses 1e-8); codes =

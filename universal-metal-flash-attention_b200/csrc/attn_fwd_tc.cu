@@ -33,7 +33,9 @@
 #include <cuda_fp16.h>
 #include <math_constants.h>
 
+#include <algorithm>
 #include <mutex>
+#include <numeric>
 #include <type_traits>
 
 #include "common.h"
@@ -247,11 +249,32 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
   // packed variable-length sequences (common.h): unmasked instantiations only -- segments do not combine with external masks
   const int* const seg_q = MASKED ? nullptr : p.cu_q;
   const int* const seg_k = MASKED ? nullptr : p.cu_k;
+  // decode over a K/V cache (FwdTcParams::kv_len): the 16-bit unmasked instantiations serve it
+  constexpr bool KVC = (MODE == kFwdF16 || MODE == kFwdBF16) && MASKED == 0;
   // One CTA per work item = (batch, head, 256-row query block), x fastest so the CTAs of one head run together (K/V stay in L2).
-  struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half; };
+  struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half, L; };
   auto decode = [&](int w) {
-    const int nqb = (p.Sq + 255) / 256;
     Item it;
+    if constexpr (KVC) {
+      if (p.kv_len) {        // (query item, split, KV head, sequence), query items fastest: they read the same keys
+        it.half = 0; it.lid = 0;
+        const int qi = w % p.kv_nqi;
+        w /= p.kv_nqi;
+        const int split = w % p.kv_nsplit;
+        w /= p.kv_nsplit;
+        it.hk = w % p.Hkv; it.b = w / p.Hkv; it.h = it.hk * p.kv_g;
+        it.r0 = 2 * qi * p.kv_sqb;                                         // first token of the item
+        it.nt = it.r0 + p.kv_sqb < p.Sq ? 2 : 1;
+        it.L = kvc_len(p.kv_len, it.b, p.kv_cap);
+        int klo, khi, t0, t1;
+        kvc_block_key_range(p.causal, p.window, it.L, p.Sq, it.r0, min(it.r0 + it.nt * p.kv_sqb, p.Sq), klo, khi);
+        kvc_split_tiles((p.kv_cap + 127) >> 7, p.kv_nsplit, split, t0, t1);
+        it.j_lo = max(klo >> 7, t0);
+        it.n = khi > klo ? max(0, min((khi + 127) >> 7, t1) - it.j_lo) : 0;
+        return it;
+      }
+    }
+    const int nqb = (p.Sq + 255) / 256;
     it.half = 0;
     if constexpr (WIDE) { it.half = w & 1; w >>= 1; }           // the two O halves of a query block run next to each other
     const int x = w % nqb, hb = w / nqb;
@@ -327,6 +350,14 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
           ++nqraw;
           return;
         }
+        if constexpr (KVC) {
+          if (p.kv_len) {      // GQA-packed tile: box (64, kv_sqb, G) of the (D, Sq, G, Hkv, B) map lands as rows g * kv_sqb + s
+            mbar_arrive_expect_tx(q_full(t2), p.kv_qbytes);
+#pragma unroll
+            for (int c = 0; c < C::kQChunks; ++c) tma_load_5d(sQ + t2 * QT + c * CHB, &p.tq, q_full(t2), c * 64, r0 + t2 * p.kv_sqb, 0, hk, b);
+            return;
+          }
+        }
         mbar_arrive_expect_tx(q_full(t2), QT);
         load_half(sQ + t2 * QT, &p.tq, q_full(t2), r0 + t2 * 128, h);
         if constexpr (SPLIT) load_half(sQ + t2 * QT + HT, &p.tq2, q_full(t2), r0 + t2 * 128, h);
@@ -355,8 +386,48 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         for (int c = 0; c < C::kVChunks; ++c) tma_load_4d(sKV + s * STG + c * CHB, m, kv_full(s), col0 + c * 64, row, hk, b);
         ++kvi;
       };
-      if (n > 0) load_q(0);
-      for (int it = 0; it < n; ++it) {
+      bool paged = false;
+      if constexpr (KVC) paged = p.kv_pages != nullptr;
+      if (paged) {
+        // paged K / V cache: the pools are mapped as [num_pages, page_size, Hkv, D], and a 128-key tile arrives as 128 / kv_box boxes
+        // of kv_box = gcd(page_size, 128) rows, each inside one page.  Box rows are a multiple of 16, so the boxes together leave
+        // the same 128-byte-swizzled image as one 128-row box.  The page ids of the next tile are read right after this tile's loads
+        // are issued, so their L2 round trip overlaps the wait for a free stage.
+        const int br = p.kv_box, nb = 128 / br;
+        const int* bt = p.kv_pages + (size_t)b * p.kv_npb;
+        int pg[8];
+        auto fetch_pages = [&](int j) {
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const int key = j * 128 + i * br;
+            pg[i] = p.kv_npages;               // past the capacity: a box wholly outside the pool, which TMA fills with zeros
+            if (i < nb && key < p.kv_cap) pg[i] = min(max(__ldg(bt + key / p.kv_page), 0), p.kv_npages - 1);
+          }
+        };
+        auto load_paged = [&](const CUtensorMap* m, uint32_t bytes, int nch, int j) {
+          const int s = kvi % NS;
+          mbar_wait(kv_empty(s), ((kvi / NS) & 1) ^ 1);
+          mbar_arrive_expect_tx(kv_full(s), bytes);
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            if (i < nb) {
+              const int prow = (j * 128 + i * br) % p.kv_page;
+              for (int c = 0; c < nch; ++c)
+                tma_load_4d(sKV + s * STG + c * CHB + i * br * 128, m, kv_full(s), c * 64, prow, hk, pg[i]);
+            }
+          }
+          ++kvi;
+        };
+        if (n > 0) { fetch_pages(im.j_lo); load_q(0); }
+        for (int it = 0; it < n; ++it) {
+          load_paged(&p.tk, HT, C::kQChunks, im.j_lo + it);
+          if (it == 0 && nt == 2) load_q(1);
+          load_paged(&p.tv, VT, C::kVChunks, im.j_lo + it);
+          if (it + 1 < n) fetch_pages(im.j_lo + it + 1);
+        }
+      }
+      if (!paged && n > 0) load_q(0);
+      for (int it = 0; it < n && !paged; ++it) {
         const int row = (tile_of(im, it) & (kTileNoMask - 1)) * 128;
         if constexpr (SPLIT) load_k(&p.tk2, row);         // K_lo first: its stage is released after the first MMA group
         load_k(&p.tk, row);
@@ -491,7 +562,16 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     const int r = r0 + t * 128 + row;
     float m = -CUDART_INF_F, l = 0.f;                      // m in scaled log2 units (score * scale * log2 e)
     int clo, chi;                                          // visible keys of this row: [clo, chi]
-    row_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r, clo, chi);
+    bool kvc = false;
+    if constexpr (KVC) kvc = p.kv_len != nullptr;
+    if (kvc) {
+      // token s of query head g = row / kv_sqb; rows past G * kv_sqb (stale shared memory) and tokens past Sq (zero-filled) see no key
+      const int s = r0 + t * p.kv_sqb + row % p.kv_sqb;
+      clo = chi = 0;
+      if (row < p.kv_rows && s < p.Sq) kvc_row_key_range(p.causal, p.window, im.L, p.Sq, s, clo, chi);
+    } else {
+      row_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r, clo, chi);
+    }
     --chi;
     // int8 mode: per-row Q scale (folded with c), per-64-key K and V block scales
     float qsc = p.c;
@@ -833,12 +913,12 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
       float inv = (l > 0.f ? 1.f / l : 0.f) * ((I8 && !v_blocks) ? p.vs1 : 1.f);
       if constexpr (F8) { if (p.vs) inv = (l > 0.f ? 1.f / l : 0.f) * __ldg(p.vs + (size_t)b * p.Hkv + hk); }     // per-(b, head) scale of the e4m3 V
       if constexpr (SPLIT) inv *= __ldg(p.vs);
-      const bool live = r < p.Sq;
+      const bool live = kvc ? row < p.kv_rows : r < p.Sq;
       // zero-padded head dims: the columns past the true head dim p.dv are not written
       const bool padded_d = p.dv > 0 && p.dv < (WIDE ? 256 : D);
       const int dv_tile = p.dv - (WIDE ? 128 * im.half : 0);
       const size_t orow = (size_t)b * p.o_sb + (size_t)h * p.o_sh + (size_t)r * p.o_ss + (WIDE ? 128 * im.half : 0);   // wide: this CTA's half of O
-      const size_t lrow = ((size_t)b * p.H + h) * p.lse_sh + r;
+      const size_t lrow = kvc ? ((size_t)blockIdx.x * 2 + t) * p.kv_rows + row : ((size_t)b * p.H + h) * p.lse_sh + r;
       float l_out = l > 0.f ? m + log2f(l) - kShift : -CUDART_INF_F;
       // accumulate mode (ring attention): the partial of this launch is merged in place with the (O, L) already there,
       //   L = log2(2^L_old + 2^L_new),  O = O_old 2^(L_old - L) + O_new 2^(L_new - L)      (fp32 O only)
@@ -975,9 +1055,11 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         named_bar_sync(4 + t, 128);
         if ((threadIdx.x & 127) == 0) {
           if (p.o_dtype == kF32) {
+            // K/V-cache partials go to the scratch tile (tile t, item) of the [items, 2, kv_rows, D] map
+            const int y = kvc ? 0 : r0 + t * 128, z = kvc ? t : h, w = kvc ? (int)blockIdx.x : b;
 #pragma unroll
             for (int ch = 0; ch < D / 32; ++ch)
-              tma_store_4d(&p.to, base + (uint32_t)(t * (D / 32) + ch) * (128u * 128u), ch * 32 + (WIDE ? 128 * im.half : 0), r0 + t * 128, h, b);
+              tma_store_4d(&p.to, base + (uint32_t)(t * (D / 32) + ch) * (128u * 128u), ch * 32 + (WIDE ? 128 * im.half : 0), y, z, w);
           } else {
 #pragma unroll
             for (int ch = 0; ch < D / 64; ++ch)
@@ -1308,7 +1390,8 @@ cudaError_t launch_fwd_tc_kernel(const FwdTcParams& prm_in, int D, int mode, cud
   prm.nbatch = B;
   ptx::watchdog_bind();
   const bool wide = mode == kFwdWideF16 || mode == kFwdWideBF16;
-  const long long items = (long long)((prm.Sq + 255) / 256) * prm.H * B * (wide ? 2 : 1);
+  const long long items = prm.kv_len ? (long long)prm.kv_nqi * prm.kv_nsplit * prm.Hkv * B
+                                     : (long long)((prm.Sq + 255) / 256) * prm.H * B * (wide ? 2 : 1);
   if (items <= 0 || items > 0x7fffffffLL) return cudaErrorInvalidValue;
   const dim3 grid((unsigned)items, 1, 1);        // one CTA per work item
   if (wide) {                                    // D is the head dim of the problem (256); the kernel's tiles are 128 wide
@@ -1470,6 +1553,134 @@ cudaError_t launch_fwd_tc(const AttnParams& p, cudaStream_t st) {
   else g_last_kernel = prm.mask ? (bf ? "fwd_tc_bf16_d64_mask" : "fwd_tc_fp16_d64_mask") : (bf ? "fwd_tc_bf16_d64" : "fwd_tc_fp16_d64");
   ++g_launch_count;
   return e;
+}
+
+// ------------------------------------------------------------------------------------------------ decode over a K/V cache
+namespace {
+
+struct KvcCombine {
+  const float* o_part;       // [items][2][rows][D]
+  const float* l_part;       // [items][2][rows]
+  void* o;
+  long long o_sb, o_sh, o_ss;
+  int o_dtype;
+  float* lse;                // [B, H, Sq] or null
+  int H, Hkv, Sq, D, G, sqb, rows, nqi, nsplit;
+};
+
+// One warp per query row (b, h, s), grid (Sq / 8, H, B): merges the row's partials of every split (lse_merge_*), writes O in the output's type and
+// stride and L.  Splits without a visible key (L_k = -inf) are not read.  Lane i holds head dims [4i, 4i + 4).
+__global__ void __launch_bounds__(256) kvcache_combine_kernel(const KvcCombine c) {
+  const int s = blockIdx.x * 8 + (threadIdx.x >> 5), h = blockIdx.y, b = blockIdx.z;
+  const int lane = threadIdx.x & 31;
+  if (s >= c.Sq) return;
+  const long long rid = ((long long)b * c.H + h) * c.Sq + s;
+  const int hk = h / c.G, chunk = s / c.sqb;
+  const int r = (h % c.G) * c.sqb + s % c.sqb;
+  const long long item0 = ((long long)b * c.Hkv + hk) * c.nsplit * c.nqi + (chunk >> 1);     // split k: item0 + k * nqi
+  auto slot = [&](int k) { return ((item0 + (long long)k * c.nqi) * 2 + (chunk & 1)) * c.rows + r; };
+  float m = -CUDART_INF_F;
+  for (int k = lane; k < c.nsplit; k += 32) m = fmaxf(m, __ldg(c.l_part + slot(k)));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
+  float4 acc = make_float4(-0.f, -0.f, -0.f, -0.f);       // -0 + x == x for every x: one split passes through unchanged
+  float L = -CUDART_INF_F;
+  const int c0 = lane * 4;
+  if (m != -CUDART_INF_F) {
+    float wsum = 0.f;
+    for (int k = lane; k < c.nsplit; k += 32) wsum += lse_merge_weight(__ldg(c.l_part + slot(k)), m);
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
+    L = lse_merge_total(m, wsum);
+    for (int k = 0; k < c.nsplit; ++k) {
+      const float lk = __ldg(c.l_part + slot(k));
+      if (lk == -CUDART_INF_F || c0 >= c.D) continue;
+      const float wk = lse_merge_weight(lk, m) / wsum;
+      const float4 ok = __ldg(reinterpret_cast<const float4*>(c.o_part + slot(k) * c.D + c0));
+      acc = make_float4(fmaf(wk, ok.x, acc.x), fmaf(wk, ok.y, acc.y), fmaf(wk, ok.z, acc.z), fmaf(wk, ok.w, acc.w));
+    }
+  }
+  if (m == -CUDART_INF_F) acc = make_float4(0.f, 0.f, 0.f, 0.f);   // a row without keys: O = +0
+  if (c0 < c.D) {
+    const long long off = (long long)b * c.o_sb + (long long)h * c.o_sh + (long long)s * c.o_ss + c0;
+    auto put = [&](int i, float x) {
+      if (c.o_dtype == kF32) reinterpret_cast<float*>(c.o)[off + i] = x;
+      else reinterpret_cast<uint16_t*>(c.o)[off + i] = (uint16_t)((c.o_dtype == kBF16 ? pack_bf16(x, 0.f) : pack_f16(x, 0.f)) & 0xffffu);
+    };
+    put(0, acc.x); put(1, acc.y); put(2, acc.z); put(3, acc.w);
+  }
+  if (lane == 0 && c.lse) c.lse[rid] = L;
+}
+
+}  // namespace
+
+KvCachePlan kvcache_plan(const KvCacheParams& p, int sm_count) {
+  KvCachePlan k;
+  k.G = p.H / p.Hkv;
+  k.sqb = std::min(p.Sq, 128 / k.G);
+  k.rows = k.G * k.sqb;
+  const int chunks = (p.Sq + k.sqb - 1) / k.sqb;
+  k.nqi = (chunks + 1) / 2;
+  // split the keys when the items of the call leave SMs idle: about one wave of CTAs, each split at least two 128-key tiles
+  const long long base = (long long)p.B * p.Hkv * k.nqi;
+  const int ntiles = (p.cap + 127) / 128;
+  long long ns = base < sm_count ? sm_count / base : 1;
+  ns = std::max(1LL, std::min(ns, (long long)ntiles / 2));
+  const int per = (int)((ntiles + ns - 1) / ns);
+  k.nsplit = (ntiles + per - 1) / per;                   // no split is left without tiles
+  k.items = base * k.nsplit;
+  k.o_bytes = ((size_t)k.items * 2 * k.rows * p.D * sizeof(float) + 255) & ~(size_t)255;
+  k.l_bytes = (size_t)k.items * 2 * k.rows * sizeof(float);
+  return k;
+}
+
+cudaError_t launch_fwd_kvcache(const KvCacheParams& p, const KvCachePlan& k, void* scratch, cudaStream_t st) {
+  if (k.items <= 0 || k.items > 0x7fffffffLL || p.H > 65535 || p.B > 65535) return cudaErrorInvalidValue;   // (combine grid y / z)
+  float* o_part = reinterpret_cast<float*>(scratch);
+  float* l_part = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(scratch) + k.o_bytes);
+  FwdTcParams prm = {};
+  const int Dk = p.D <= 64 ? 64 : 128;
+  const bool paged = p.block_table != nullptr;
+  TensorView kv[2] = {p.k, p.v};
+  int kB = p.B, kS = p.cap, box = 128;
+  if (paged) {                                 // [num_pages, page_size, Hkv, D] pools seen as [B = pages, H = Hkv, S = page, D]
+    for (TensorView& t : kv) { t.sb = (int64_t)p.page_size * p.Hkv * p.D; t.sh = p.D; t.ss = (int64_t)p.Hkv * p.D; t.sd = 1; }
+    kB = p.num_pages; kS = p.page_size;
+    box = std::gcd(p.page_size, 128);
+  }
+  const TensorView ov = {o_part, 2LL * k.rows * p.D, (int64_t)k.rows * p.D, p.D, 1};
+  if (!tc::make_map_gqa(&prm.tq, p.q, p.in_dtype, p.B, p.Hkv, k.G, p.Sq, p.D, k.sqb) ||
+      !make_map(&prm.tk, kv[0], p.in_dtype, kB, p.Hkv, kS, p.D, box) || !make_map(&prm.tv, kv[1], p.in_dtype, kB, p.Hkv, kS, p.D, box) ||
+      !make_map(&prm.to, ov, kF32, (int)k.items, 2, k.rows, p.D, k.rows))
+    return cudaErrorInvalidValue;
+  prm.o_tma = 1;
+  prm.o_dtype = kF32;
+  prm.lse = l_part;
+  prm.H = p.H; prm.Hkv = p.Hkv; prm.Sq = p.Sq; prm.Skv = p.cap;
+  prm.dv = p.D;
+  prm.c = p.scale * kLog2e;
+  prm.causal = p.causal; prm.window = p.window;
+  prm.kv_len = p.seqlens; prm.kv_pages = p.block_table;
+  prm.kv_cap = p.cap; prm.kv_page = p.page_size; prm.kv_npages = p.num_pages;
+  prm.kv_npb = paged ? p.cap / p.page_size : 0; prm.kv_box = box;
+  prm.kv_g = k.G; prm.kv_sqb = k.sqb; prm.kv_rows = k.rows; prm.kv_nqi = k.nqi; prm.kv_nsplit = k.nsplit;
+  prm.kv_qbytes = (Dk / 64) * 128 * k.rows;
+  const bool bf = p.in_dtype == kBF16;
+  cudaError_t e = launch_fwd_tc_kernel(prm, Dk, bf ? kFwdBF16 : kFwdF16, st, p.B);
+  if (e != cudaSuccess) return e;
+  KvcCombine c;
+  c.o_part = o_part; c.l_part = l_part;
+  c.o = const_cast<void*>(p.o.ptr); c.o_sb = p.o.sb; c.o_sh = p.o.sh; c.o_ss = p.o.ss; c.o_dtype = p.o_dtype;
+  c.lse = p.lse;
+  c.H = p.H; c.Hkv = p.Hkv; c.Sq = p.Sq; c.D = p.D; c.G = k.G; c.sqb = k.sqb; c.rows = k.rows; c.nqi = k.nqi; c.nsplit = k.nsplit;
+  kvcache_combine_kernel<<<dim3((unsigned)((p.Sq + 7) / 8), (unsigned)p.H, (unsigned)p.B), 256, 0, st>>>(c);
+  static const char* names[2][2][2] = {{{"fwd_tc_fp16_d64_kvcache", "fwd_tc_fp16_d64_kvcache_split"},
+                                        {"fwd_tc_fp16_d128_kvcache", "fwd_tc_fp16_d128_kvcache_split"}},
+                                       {{"fwd_tc_bf16_d64_kvcache", "fwd_tc_bf16_d64_kvcache_split"},
+                                        {"fwd_tc_bf16_d128_kvcache", "fwd_tc_bf16_d128_kvcache_split"}}};
+  g_last_kernel = names[bf][Dk == 128][k.nsplit > 1];
+  g_launch_count += 2;
+  return cudaGetLastError();
 }
 
 }  // namespace mfa

@@ -161,6 +161,67 @@ __host__ __device__ inline void block_query_range(int causal, int window, int Sq
   if (hi < lo) hi = lo;
 }
 
+// ---- decode over a K/V cache.  Sequence b holds L_b valid keys, the last Sq of them the new tokens: query row s sits at position
+// p = L_b - Sq + s and sees key j < L_b iff (!causal || j <= p) && (window < 0 || p - j <= window) (bottom-right alignment).
+// L_b comes from device memory the host has not checked: kvc_len clamps it to [0, capacity].  Per-row bounds never decrease with
+// s, so the range of a block of rows is the lower bound of its first and the upper bound of its last.
+
+__host__ __device__ inline int kvc_len(const int* lens, int b, int cap) {
+  const int v = lens[b];
+  return v < 0 ? 0 : v > cap ? cap : v;
+}
+
+// Visible keys [lo, hi) of query row s (lo == hi: none).
+__host__ __device__ inline void kvc_row_key_range(int causal, int window, int L, int Sq, int s, int& lo, int& hi) {
+  const int p = L - Sq + s;
+  lo = window >= 0 ? max(0, p - window) : 0;
+  hi = causal ? min(L, p + 1) : L;
+  if (hi < lo) hi = lo;
+}
+
+// Visible keys [lo, hi) of query rows [s0, s1), s1 > s0.
+__host__ __device__ inline void kvc_block_key_range(int causal, int window, int L, int Sq, int s0, int s1, int& lo, int& hi) {
+  int l2, h2;
+  kvc_row_key_range(causal, window, L, Sq, s0, lo, h2);
+  kvc_row_key_range(causal, window, L, Sq, s1 - 1, l2, hi);
+  if (hi < lo) hi = lo;
+}
+
+// Key tiles [t0, t1) of split k when the ntiles 128-key tiles of the capacity are shared by nsplit splits.
+__host__ __device__ inline void kvc_split_tiles(int ntiles, int nsplit, int k, int& t0, int& t1) {
+  const int per = (ntiles + nsplit - 1) / nsplit;
+  t0 = min(k * per, ntiles);
+  t1 = min(t0 + per, ntiles);
+}
+
+// Log2-domain merge of attention partials over disjoint key sets (SURVEY 8e): with m = max_k L_k and w_k = 2^(L_k - m),
+//   L = m + log2(sum_k w_k),  O = sum_k O_k w_k / sum_k w_k.
+// A partial without keys (L_k = -inf) weighs 0.  With one partial, w = 1 and L = m exactly.
+__device__ __forceinline__ float lse_merge_weight(float lk, float m) { return lk == -__int_as_float(0x7f800000) ? 0.f : exp2f(lk - m); }
+__device__ __forceinline__ float lse_merge_total(float m, float wsum) { return m + log2f(wsum); }
+
+// Attention of Sq new tokens per sequence against that sequence's K/V cache (mfa_attention_forward_kvcache).
+struct KvCacheParams {
+  TensorView q, o;           // [B, H, Sq, D] views (o in o_dtype)
+  TensorView k, v;           // contiguous cache: [B, Hkv, cap, D] views; paged: base of the [num_pages, page_size, Hkv, D] pools
+  float* lse;                // [B, H, Sq] or null
+  const int* seqlens;        // [B] device
+  const int* block_table;    // [B, cap / page_size] device, or null (contiguous cache)
+  int B, H, Hkv, Sq, D, cap, page_size, num_pages;
+  float scale;
+  int causal, window, in_dtype, o_dtype;
+};
+// How a call is cut into work items: G query heads per KV head share a tile as rows g * sqb + s (rows = G * sqb live rows), a
+// work item holds two such tiles of consecutive tokens (nqi items per (b, KV head)), and the keys of the capacity are shared by
+// nsplit splits.  Chosen from the shape and the SM count only, never from the lengths.
+struct KvCachePlan {
+  int G, sqb, rows, nqi, nsplit;
+  long long items;
+  size_t o_bytes, l_bytes;   // scratch: partial O (fp32 [items][2][rows][D]) and L ([items][2][rows])
+};
+KvCachePlan kvcache_plan(const KvCacheParams& p, int sm_count);
+cudaError_t launch_fwd_kvcache(const KvCacheParams& p, const KvCachePlan& plan, void* scratch, cudaStream_t st);
+
 // ---- kernel launchers (each returns cudaGetLastError()) ----
 cudaError_t launch_fwd_simt(const AttnParams& p, cudaStream_t st);
 cudaError_t launch_bwd_simt(const AttnParams& p, cudaStream_t st);          // dterm + dQ + dK/dV

@@ -17,6 +17,7 @@
 
 #include "../../include/mfa_ffi_ext.h"
 #include "common.h"
+#include "tc_host.h"
 
 using namespace mfa;
 
@@ -52,16 +53,24 @@ struct Scratch {
   cudaEvent_t ev = nullptr;
   cudaStream_t last = nullptr;
   bool used = false;
+  // a captured CUDA graph holds the block's address: growing the block then retires it instead of freeing it, and retired blocks
+  // are freed with the context, so a graph replayed later still writes memory it owns
+  bool captured = false;
+  std::vector<void*> retired;
   void* get(size_t bytes) {
     if (bytes <= cap) return ptr;
-    if (ptr) cudaFree(ptr);            // implicitly waits for everything that may still read the old block
-    ptr = nullptr; cap = 0; used = false;
+    if (ptr && captured) retired.push_back(ptr);
+    else if (ptr) cudaFree(ptr);       // implicitly waits for everything that may still read the old block
+    ptr = nullptr; cap = 0; used = false; captured = false;
     size_t want = bytes + (bytes >> 2) + 256;
     if (cudaMalloc(&ptr, want) != cudaSuccess) { ptr = nullptr; cudaGetLastError(); return nullptr; }
     cap = want;
     return ptr;
   }
   void release() {
+    for (void* r : retired) cudaFree(r);
+    retired.clear();
+    captured = false;
     if (ptr) cudaFree(ptr);
     if (ev) cudaEventDestroy(ev);
     ptr = nullptr; cap = 0; ev = nullptr; used = false;
@@ -78,7 +87,7 @@ struct Context {
   double last_latency = 0.0;
   int refs = 0;
   std::recursive_mutex mu;          // recursive: mfa_quantized_backward holds it across quantise + backward_core
-  enum { kMask, kLse, kDterm, kQCodes, kKCodes, kVCodes, kQScales, kKScales, kVScales, kTmpO, kQTmp, kMaskTiles, kNumScratch };
+  enum { kMask, kLse, kDterm, kQCodes, kKCodes, kVCodes, kQScales, kKScales, kVScales, kTmpO, kQTmp, kMaskTiles, kKvSplit, kNumScratch };
   Scratch scratch[kNumScratch];
   std::vector<float> row_scales[3];
   const char* last_kernel = "none";
@@ -122,7 +131,8 @@ void* ScratchScope::take(int slot, size_t bytes) {
   Scratch& sc = ctx->scratch[slot];
   void* p = sc.get(bytes);
   if (!p) return nullptr;
-  if (sc.used && sc.last != st && sc.ev) cudaStreamWaitEvent(st, sc.ev, 0);
+  // (a block a captured graph writes may be in use by a replay on any stream)
+  if (sc.used && (sc.last != st || sc.captured) && sc.ev) cudaStreamWaitEvent(st, sc.ev, 0);
   slots.push_back(slot);
   return p;
 }
@@ -1254,6 +1264,113 @@ mfa_error_t mfa_attention_backward_varlen(
             MaskArgs{nullptr, 0, nullptr, nullptr, 0, 0, 0}, none, none, none, reinterpret_cast<cudaStream_t>(stream),
             stream != nullptr, true, true, B_(cu_seqlens_q), B_(cu_seqlens_k), num_seqs};
   return backward_core(C_(context), a);
+}
+
+mfa_error_t mfa_attention_forward_kvcache(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t batch_size, uint32_t seq_len_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream) {
+  if (!context || !q || !k_cache || !v_cache || !out || !cache_seqlens) return MFA_ERROR_INVALID_ARGS;
+  const uint32_t B = batch_size, Sq = seq_len_q, H = num_heads, Hkv = num_kv_heads ? num_kv_heads : num_heads, D = head_dim;
+  const uint32_t cap = cache_capacity;
+  const int dt = header_precision_to_dtype(input_precision), odt = header_precision_to_dtype(output_precision);
+  if ((dt != kBF16 && dt != kF16) || !valid_float_dtype(odt)) return MFA_ERROR_INVALID_ARGS;
+  if (B == 0 || Sq == 0 || H == 0 || H % Hkv || H / Hkv > 128 || D < 8 || D > 128 || (D & 7) || cap == 0) return MFA_ERROR_INVALID_ARGS;
+  if (B > 65535 || Sq > 0x7fffffffu || H > 65535 || cap > 0x7fffff80u || !(softmax_scale > 0.f)) return MFA_ERROR_INVALID_ARGS;
+  const bool paged = page_size > 0;
+  if (paged ? (!block_table || (page_size & 15) || cap % page_size || num_pages == 0 || num_pages > 0x7fffffffu) : block_table != nullptr)
+    return MFA_ERROR_INVALID_ARGS;
+  if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
+  Buffer *bq = B_(q), *bk = B_(k_cache), *bv = B_(v_cache), *bo = B_(out), *bl = B_(lse), *bs = B_(cache_seqlens), *bt = B_(block_table);
+  if (!view_fits(bq, B, H, Sq, D, 2) || !view_fits(bo, B, H, Sq, D, dtype_bytes(odt))) return MFA_ERROR_INVALID_ARGS;
+  if (paged) {
+    const size_t pool = (size_t)num_pages * page_size * Hkv * D * 2;
+    if (bk->ndim || bv->ndim || bk->bytes < pool || bv->bytes < pool) return MFA_ERROR_INVALID_ARGS;
+    if (bt->ndim || bt->bytes < (size_t)B * (cap / page_size) * 4) return MFA_ERROR_INVALID_ARGS;
+  } else if (!view_fits(bk, B, Hkv, cap, D, 2) || !view_fits(bv, B, Hkv, cap, D, 2)) {
+    return MFA_ERROR_INVALID_ARGS;
+  }
+  if (bs->ndim || bs->bytes < (size_t)B * 4 || (bl && bl->bytes < (size_t)B * H * Sq * 4)) return MFA_ERROR_INVALID_ARGS;
+  // lengths and page ids the host can read are checked here; device-resident ones are clamped by the kernel
+  if (bs->host) {
+    const int32_t* len = reinterpret_cast<const int32_t*>(bs->host);
+    for (uint32_t b = 0; b < B; ++b)
+      if (len[b] < 0 || (uint32_t)len[b] > cap) return MFA_ERROR_INVALID_ARGS;
+  }
+  if (paged && bt->host) {
+    const int32_t* ids = reinterpret_cast<const int32_t*>(bt->host);
+    for (size_t i = 0, n = (size_t)B * (cap / page_size); i < n; ++i)
+      if (ids[i] < 0 || (uint32_t)ids[i] >= num_pages) return MFA_ERROR_INVALID_ARGS;
+  }
+  const bool async = stream != nullptr;
+  if (async && (bq->mirrored || bk->mirrored || bv->mirrored || bo->mirrored || (bl && bl->mirrored) || bs->mirrored || (bt && bt->mirrored)))
+    return MFA_ERROR_INVALID_ARGS;
+
+  Context* ctx = C_(context);
+  std::lock_guard<std::recursive_mutex> lock(ctx->mu);
+  DeviceGuard dg(ctx->device);
+  KvCacheParams p;
+  p.q = view_of(bq, H, Sq, D, false);
+  p.o = view_of(bo, H, Sq, D, false);
+  p.k = view_of(bk, Hkv, cap, D, false);
+  p.v = view_of(bv, Hkv, cap, D, false);
+  p.lse = bl ? reinterpret_cast<float*>(bl->dev) : nullptr;
+  p.seqlens = reinterpret_cast<const int*>(bs->dev);
+  p.block_table = paged ? reinterpret_cast<const int*>(bt->dev) : nullptr;
+  p.B = (int)B; p.H = (int)H; p.Hkv = (int)Hkv; p.Sq = (int)Sq; p.D = (int)D; p.cap = (int)cap;
+  p.page_size = (int)page_size; p.num_pages = (int)num_pages;
+  p.scale = softmax_scale; p.causal = causal ? 1 : 0; p.window = window_size < 0 ? -1 : window_size;
+  p.in_dtype = dt; p.o_dtype = odt;
+  // TMA: 16-byte aligned bases and outer strides; out only needs unit stride along D (the combine kernel stores elements)
+  if (!tc::view_ok(p.q, H, B) || p.o.sd != 1 || (!paged && (!tc::view_ok(p.k, Hkv, B) || !tc::view_ok(p.v, Hkv, B))) ||
+      (paged && ((reinterpret_cast<uintptr_t>(bk->dev) | reinterpret_cast<uintptr_t>(bv->dev)) & 15)))
+    return MFA_ERROR_INVALID_ARGS;
+  static int sm_count[kMaxDevices] = {0};
+  if (!sm_count[ctx->device] && cudaDeviceGetAttribute(&sm_count[ctx->device], cudaDevAttrMultiProcessorCount, ctx->device) != cudaSuccess) {
+    cudaGetLastError();
+    sm_count[ctx->device] = 148;
+  }
+  const KvCachePlan plan = kvcache_plan(p, sm_count[ctx->device]);
+  const size_t bytes = plan.o_bytes + plan.l_bytes;
+
+  cudaStream_t st = async ? reinterpret_cast<cudaStream_t>(stream) : ctx->stream;
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if (async && cudaStreamIsCapturing(st, &cs) != cudaSuccess) { cudaGetLastError(); return MFA_ERROR_EXECUTION_FAILED; }
+  ScratchScope scope(ctx, st);
+  void* scratch = nullptr;
+  Scratch& ksc = ctx->scratch[Context::kKvSplit];
+  if (cs != cudaStreamCaptureStatusNone) {
+    // inside a graph capture: no allocation.  The graph keeps the block (Scratch::captured) and orders itself against other
+    // users of it through external event nodes: a replay waits for the last use recorded before its launch and records its own.
+    if (ksc.cap < bytes) return MFA_ERROR_MEMORY_ALLOCATION;
+    if (!ksc.ev && cudaEventCreateWithFlags(&ksc.ev, cudaEventDisableTiming) != cudaSuccess) { cudaGetLastError(); return MFA_ERROR_EXECUTION_FAILED; }
+    if (ksc.used && cudaStreamWaitEvent(st, ksc.ev, cudaEventWaitExternal) != cudaSuccess) { cudaGetLastError(); return MFA_ERROR_EXECUTION_FAILED; }
+    scratch = ksc.ptr;
+  } else if (!(scratch = scope.take(Context::kKvSplit, bytes))) {
+    return MFA_ERROR_MEMORY_ALLOCATION;
+  }
+  Sync sync{ctx, st, async, {}};
+  cudaError_t e;
+  if ((e = sync.in(bq)) != cudaSuccess || (e = sync.in(bk)) != cudaSuccess || (e = sync.in(bv)) != cudaSuccess ||
+      (e = sync.in(bs)) != cudaSuccess || (e = sync.in(bt)) != cudaSuccess)
+    return cuda_fail(e, "h2d");
+  Timer tm(ctx, st, !async);
+  e = launch_fwd_kvcache(p, plan, scratch, st);
+  if (e == cudaSuccess && cs != cudaStreamCaptureStatusNone) {
+    e = cudaEventRecordWithFlags(ksc.ev, st, cudaEventRecordExternal);
+    ksc.captured = true; ksc.used = true;
+    ksc.last = nullptr;                // every later call, on any stream, waits for the replays' record
+  }
+  tm.stop();
+  ctx->last_kernel = g_last_kernel;
+  if (e != cudaSuccess) return cuda_fail(e, "kvcache forward launch");
+  sync.out(bo); sync.out(bl);
+  if ((e = sync.finish()) != cudaSuccess) return cuda_fail(e, "kvcache forward sync");
+  tm.read();
+  return MFA_SUCCESS;
 }
 
 // ---- quantised forward family ---------------------------------------------------------------------

@@ -58,6 +58,15 @@ struct FwdTcParams {
   const int* cu_q;         // packed variable-length sequences (AttnParams::cu_q / cu_k / nseq), or null
   const int* cu_k;
   int nseq;
+  // decode over a K/V cache (common.h, kvc_*) when kv_len is set; read by the unmasked 16-bit instantiations only.  A work item is
+  // (query item, split, KV head, sequence); its tiles hold the G query heads of one KV head as rows g * kv_sqb + s (tq is the 5-D
+  // (D, Sq, G, Hkv, B) map), and it leaves a normalised partial: O through `to` at (column, 0, tile, item) and L in
+  // lse[(item * 2 + tile) * kv_rows + row].
+  const int* kv_len;       // [B] valid keys per sequence
+  const int* kv_pages;     // [B][kv_npb] page table, or null (contiguous cache: tk / tv map [B, Hkv, cap, D])
+  int kv_cap, kv_page, kv_npages, kv_npb, kv_box;   // capacity, page size, pages in the pool, pages per sequence, rows per K / V box
+  int kv_g, kv_sqb, kv_rows, kv_nqi, kv_nsplit;     // see KvCachePlan
+  int kv_qbytes;           // bytes TMA writes into one Q tile
 };
 
 bool fwd_tc_mask_ok(const AttnParams& p);

@@ -447,7 +447,7 @@ __global__ void merge_partials_kernel(float* __restrict__ o_acc, float* __restri
   const float la = l_acc[row], lp = l_part[row];
   if (lp == -CUDART_INF_F) return;
   const float m = fmaxf(la, lp);
-  const float wa = (la == -CUDART_INF_F) ? 0.f : exp2f(la - m), wp = exp2f(lp - m);
+  const float wa = lse_merge_weight(la, m), wp = lse_merge_weight(lp, m);
   const float s = wa + wp;
   const float ca = wa / s, cp = wp / s;
   float* oa = o_acc + row * D;
@@ -463,7 +463,7 @@ __global__ void merge_partials_kernel(float* __restrict__ o_acc, float* __restri
     for (uint32_t d = lane; d < D; d += 32) oa[d] = oa[d] * ca + op[d] * cp;
   }
   __syncwarp();
-  if (lane == 0) l_acc[row] = m + log2f(s);
+  if (lane == 0) l_acc[row] = lse_merge_total(m, s);
 }
 
 // ---- in-place FWHT over blocks of n = 2^k <= 1024 fp32 values, scaled by 1/sqrt(n)

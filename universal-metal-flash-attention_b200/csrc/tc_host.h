@@ -88,6 +88,26 @@ inline bool make_map5(CUtensorMap* out, const void* base, int dtype, int slots, 
   return r == CUDA_SUCCESS;
 }
 
+// Q of grouped-query attention, [B, H = Hkv * G, Sq, D] view with unit inner stride -> 5-D tensor map (D, Sq, G, Hkv, B), box
+// (64, sqb, G, 1, 1), 128B swizzle: one box lands the sqb tokens of all G query heads of a KV head as rows g * sqb + s of a tile.
+inline bool make_map_gqa(CUtensorMap* out, const TensorView& t, int dtype, int B, int Hkv, int G, int Sq, int D, int sqb) {
+  EncodeTiledFn fn = encode_fn();
+  if (!fn || sqb < 1 || G < 1 || sqb * G > 128) return false;
+  const cuuint64_t eb = 2;
+  cuuint64_t dims[5] = {(cuuint64_t)D, (cuuint64_t)Sq, (cuuint64_t)G, (cuuint64_t)Hkv, (cuuint64_t)B};
+  cuuint64_t st[4] = {(cuuint64_t)t.ss * eb, (cuuint64_t)t.sh * eb, (cuuint64_t)t.sh * G * eb, (cuuint64_t)t.sb * eb};
+  if (Sq == 1) st[0] = (cuuint64_t)D * eb;              // extent-1 dims: any valid stride (the view's may be 0)
+  if (G == 1) st[1] = st[0] * (cuuint64_t)Sq;
+  if (Hkv == 1) st[2] = st[1] * (cuuint64_t)G;
+  if (B == 1) st[3] = st[2] * (cuuint64_t)Hkv;
+  cuuint32_t box[5] = {64, (cuuint32_t)sqb, (cuuint32_t)G, 1, 1};
+  cuuint32_t es[5] = {1, 1, 1, 1, 1};
+  const CUtensorMapDataType ty = dtype == kBF16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+  CUresult r = fn(out, ty, 5, const_cast<void*>(t.ptr), dims, st, box, es, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return r == CUDA_SUCCESS;
+}
+
 // TMA needs a 16-byte aligned base, unit inner stride and 16-byte multiples for the outer strides.
 inline bool view_ok(const TensorView& t, int64_t Hn, int64_t B, int elem_bytes = 2) {
   const int64_t q = 16 / elem_bytes;

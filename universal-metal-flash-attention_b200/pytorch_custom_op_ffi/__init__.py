@@ -7,8 +7,9 @@
 """
 from .backend import (MetalSDPAContext, is_metal_sdpa_available, metal_sdpa_version, register_metal_sdpa_backend,
                       unregister_metal_sdpa_backend, use_metal_sdpa)
-from .ext import metal_flash_attention_varlen
+from .ext import metal_flash_attention_varlen, metal_flash_attention_with_kvcache
 
 __version__ = "0.1.0"
 __all__ = ["register_metal_sdpa_backend", "unregister_metal_sdpa_backend", "use_metal_sdpa", "is_metal_sdpa_available",
-           "metal_sdpa_version", "MetalSDPAContext", "metal_flash_attention_varlen"]
+           "metal_sdpa_version", "MetalSDPAContext", "metal_flash_attention_varlen",
+           "metal_flash_attention_with_kvcache"]

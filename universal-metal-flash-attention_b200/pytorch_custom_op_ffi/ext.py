@@ -312,6 +312,80 @@ def metal_flash_attention_varlen(q, k, v, cu_seqlens_q, cu_seqlens_k, is_causal=
                                              -1 if window is None or window < 0 else int(window))
 
 
+def _bshd_handle(bind, t):
+    """[B, S, heads, D] tensor (unit stride along D) -> a [B, heads, S, D] strided handle over the same memory."""
+    B, S, Hn, D = t.shape
+    shape = (ctypes.c_int64 * 4)(B, Hn, S, D)
+    strides = (ctypes.c_int64 * 4)(t.stride(0), t.stride(2), t.stride(1), t.stride(3))
+    h = _ffi.mfa_buffer_t()
+    nbytes = max(((B - 1) * t.stride(0) + (S - 1) * t.stride(1) + (Hn - 1) * t.stride(2) + D) * t.element_size(), 1)
+    _ffi._check_error(_lib.mfa_buffer_from_mtl_buffer_with_strides(bind.ctx.handle, ctypes.c_void_p(t.data_ptr()), nbytes,
+                                                                   shape, strides, 4, ctypes.byref(h)))
+    bind.handles.append(h)
+    return h
+
+
+def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block_table=None, is_causal=True, scale=None,
+                                       window=-1, return_lse=False):
+    """Attention of the Sq new tokens of each sequence against that sequence's K/V cache (inference decode, speculative
+    decode, chunked prefill).  q is [B, Sq, H, D] (bf16 / fp16, D a multiple of 8 up to 128); k_cache / v_cache are
+    [B, capacity, Hkv, D], or with block_table (int32 [B, capacity / page_size] page ids) paged pools
+    [num_pages, page_size, Hkv, D] with page_size a multiple of 16.  Hkv divides H (grouped-query attention without copies).
+    cache_seqlens (int32 [B]) counts the valid keys of each sequence, the new tokens included (write their K / V into the cache
+    first); token s sits at position cache_seqlens[b] - Sq + s and is_causal / window are bottom-right aligned.  Returns O
+    [B, Sq, H, D] in q's dtype (and L fp32 [B, H, Sq] in log2 units with return_lse).  Cache rows past cache_seqlens[b] inside
+    the last 128-key tile (in a paged cache: rows of the pages that block_table points to there) are read and enter P V with
+    weight 0, so they must hold finite values: allocate pools with torch.zeros, not torch.empty.  Enqueued on torch's current
+    stream with no copies of q or the caches, so it can be captured in a CUDA graph after one call of the shape outside the
+    capture; the graph stays valid when later calls of other shapes run.  Forward only."""
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (q, k_cache, v_cache)):
+        raise RuntimeError("metal_flash_attention_with_kvcache has no backward: call it under torch.no_grad() or on "
+                           "tensors that do not require grad")
+    for t in (q, k_cache, v_cache):
+        if not t.is_cuda or t.dim() != 4 or t.stride(-1) != 1:
+            raise RuntimeError("metal_flash_attention_with_kvcache: q, k_cache, v_cache must be 4-D CUDA tensors with unit "
+                               "stride along head_dim")
+    if q.dtype not in (torch.float16, torch.bfloat16) or k_cache.dtype != q.dtype or v_cache.dtype != q.dtype:
+        raise RuntimeError("metal_flash_attention_with_kvcache: q, k_cache, v_cache must share float16 or bfloat16")
+    B, Sq, H, D = q.shape
+    if k_cache.shape != v_cache.shape or k_cache.size(3) != D or H % k_cache.size(2):
+        raise RuntimeError(f"metal_flash_attention_with_kvcache: shapes q={tuple(q.shape)} k_cache={tuple(k_cache.shape)} "
+                           f"v_cache={tuple(v_cache.shape)}")
+    Hkv = k_cache.size(2)
+    for name, t in (("cache_seqlens", cache_seqlens), ("block_table", block_table)):
+        if t is not None and (t.dtype != torch.int32 or t.device != q.device or not t.is_contiguous()):
+            raise RuntimeError(f"metal_flash_attention_with_kvcache: {name} must be a contiguous int32 tensor on q's device")
+    if cache_seqlens.shape != (B,):
+        raise RuntimeError(f"metal_flash_attention_with_kvcache: cache_seqlens must be [{B}], got {tuple(cache_seqlens.shape)}")
+    if block_table is None:
+        if k_cache.size(0) != B:
+            raise RuntimeError(f"metal_flash_attention_with_kvcache: contiguous caches need batch {B}")
+        cap, page, npages = k_cache.size(1), 0, 0
+    else:
+        if block_table.dim() != 2 or block_table.size(0) != B:
+            raise RuntimeError("metal_flash_attention_with_kvcache: block_table must be [batch, pages per sequence]")
+        if not (k_cache.is_contiguous() and v_cache.is_contiguous()):
+            raise RuntimeError("metal_flash_attention_with_kvcache: paged pools must be contiguous")
+        npages, page = k_cache.size(0), k_cache.size(1)
+        cap = block_table.size(1) * page
+    if scale is None or scale <= 0.0:
+        scale = 1.0 / math.sqrt(D)
+    out = torch.empty(q.shape, device=q.device, dtype=q.dtype)
+    lse = torch.empty((B, H, Sq), device=q.device, dtype=torch.float32) if return_lse else None
+    lib_ctx = _context(q.device)
+    stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(q.device).cuda_stream or 0), q)
+    with _Bound(lib_ctx) as bind:
+        paged = block_table is not None
+        rc = _lib.mfa_attention_forward_kvcache(
+            lib_ctx.handle, _bshd_handle(bind, q), bind(k_cache) if paged else _bshd_handle(bind, k_cache),
+            bind(v_cache) if paged else _bshd_handle(bind, v_cache), _bshd_handle(bind, out), bind(lse), bind(cache_seqlens),
+            bind(block_table), B, Sq, H, Hkv, D, cap, page, npages, float(scale), bool(is_causal),
+            -1 if window is None or window < 0 else int(window), _PREC[q.dtype], _PREC[q.dtype], stream)
+    if rc != 0:
+        raise RuntimeError(f"Metal Flash Attention kvcache forward failed with code {rc}: {_ffi._get_error_string(rc)}")
+    return (out, lse) if return_lse else out
+
+
 def _dense_mask_f32(mask, query, Skv):
     """The quantised entry points take NULL or a dense fp32 additive [B,H,Sq,Skv] mask (metal_sdpa_backend.cpp:3210-3231)."""
     if mask is None:

@@ -131,6 +131,8 @@ SIGNATURES = {
     "mfa_attention_backward_ex": (_i32, [_ctx] + [_buf] * 10 + _DIMS + [_f32, _b, _i32, _i32] + _MASK + [_vp]),
     "mfa_attention_forward_varlen": (_i32, [_ctx] + [_buf] * 7 + _VARLEN + [_f32, _b, _i32, _i32, _i32, _vp]),
     "mfa_attention_backward_varlen": (_i32, [_ctx] + [_buf] * 12 + _VARLEN + [_f32, _b, _i32, _i32, _vp]),
+    "mfa_attention_forward_kvcache": (_i32, [_ctx] + [_buf] * 7 + [_u32, _u32, _u32, _u32, _u16, _u32, _u32, _u32] +
+                                      [_f32, _b, _i32, _i32, _i32, _vp]),
     "mfa_quantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _i32, _f32, _vp]),
     "mfa_dequantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _vp]),
     "mfa_merge_partials": (_i32, [_ctx, _buf, _buf, _buf, _buf, _u64, _u32, _vp]),

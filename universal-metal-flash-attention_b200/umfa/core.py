@@ -419,6 +419,67 @@ def flash_attention_varlen_forward(context: MFAContext, q, k, v, cu_seqlens_q, c
     return out, lse
 
 
+def _kvcache_dims(q, k_cache, v_cache, cache_seqlens, block_table):
+    """(B, Sq, H, Hkv, D, capacity, page_size, num_pages, lens, table) of a K/V-cache call: q [B, Sq, H, D]; caches
+    [B, capacity, Hkv, D] (block_table None) or paged pools [num_pages, page_size, Hkv, D] with block_table [B, pages per seq]."""
+    if not all(isinstance(x, np.ndarray) and x.ndim == 4 for x in (q, k_cache, v_cache)):
+        raise ValueError("kvcache q, k_cache, v_cache must be 4-D numpy arrays")
+    B, Sq, H, D = q.shape
+    if v_cache.shape != k_cache.shape or k_cache.shape[3] != D or k_cache.shape[2] == 0 or H % k_cache.shape[2]:
+        raise ValueError(f"Shape mismatch: q={q.shape}, k_cache={k_cache.shape}, v_cache={v_cache.shape}")
+    Hkv = k_cache.shape[2]
+    lens = np.ascontiguousarray(cache_seqlens, np.int32)
+    if lens.shape != (B,):
+        raise ValueError(f"cache_seqlens must hold one length per sequence ({B}), got shape {lens.shape}")
+    if block_table is None:
+        if k_cache.shape[0] != B:
+            raise ValueError(f"contiguous caches need batch {B}, got {k_cache.shape[0]}")
+        return B, Sq, H, Hkv, D, k_cache.shape[1], 0, 0, lens, None
+    table = np.ascontiguousarray(block_table, np.int32)
+    if table.ndim != 2 or table.shape[0] != B:
+        raise ValueError(f"block_table must be [batch, pages per sequence], got shape {table.shape}")
+    num_pages, page_size = k_cache.shape[0], k_cache.shape[1]
+    return B, Sq, H, Hkv, D, table.shape[1] * page_size, page_size, num_pages, lens, table
+
+
+def flash_attention_kvcache(context: MFAContext, q, k_cache, v_cache, cache_seqlens, block_table=None, *,
+                            causal: bool = True, window_size: Optional[int] = None, softmax_scale: Optional[float] = None,
+                            input_precision: Precision = "bf16", output_precision: Precision = "fp32"):
+    """Attention of Sq new tokens per sequence against that sequence's K/V cache (mfa_attention_forward_kvcache).  q is
+    [B, Sq, H, D]; k_cache / v_cache are [B, capacity, Hkv, D], or with block_table ([B, capacity / page_size] int32 page ids)
+    paged pools [num_pages, page_size, Hkv, D].  cache_seqlens[b] = valid keys of sequence b, the Sq new tokens included; token s
+    sits at position cache_seqlens[b] - Sq + s (causal / window_size are bottom-right aligned).  bf16 data travels as uint16 bit
+    patterns.  Returns (O [B, Sq, H, D] in output_precision (fp32, or fp16 / uint16 bf16 bits), L fp32 [B, H, Sq] in log2
+    units); rows that see no key get O = 0, L = -inf.  Cache rows past cache_seqlens[b] inside the last 128-key tile are read
+    and enter P V with weight 0, so they must hold finite values (zero-initialised caches do)."""
+    B, Sq, H, Hkv, D, cap, page, npages, lens, table = _kvcache_dims(q, k_cache, v_cache, cache_seqlens, block_table)
+    if softmax_scale is None:
+        softmax_scale = 1.0 / np.sqrt(D)
+    in_prec, out_prec = _parse_precision(input_precision), _parse_precision(output_precision)
+    for name, x in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache)):
+        _check_input_dtype(x, in_prec, name)
+    out = np.zeros(q.shape, {MFA_PRECISION_FP32: np.float32, MFA_PRECISION_FP16: np.float16}.get(out_prec, np.uint16))
+    lse = np.zeros((B, H, Sq), np.float32)
+    bshd = lambda arr, S, Hn: MFABuffer(context, arr, shape=(B, Hn, S, D), strides=(S * Hn * D, D, Hn * D, 1))
+    bufs = [bshd(np.ascontiguousarray(q), Sq, H)]
+    if table is None:
+        bufs += [bshd(np.ascontiguousarray(k_cache), cap, Hkv), bshd(np.ascontiguousarray(v_cache), cap, Hkv)]
+    else:
+        bufs += [MFABuffer(context, np.ascontiguousarray(k_cache)), MFABuffer(context, np.ascontiguousarray(v_cache))]
+    bufs += [bshd(out, Sq, H), MFABuffer(context, lse), MFABuffer(context, lens)]
+    if table is not None:
+        bufs.append(MFABuffer(context, table))
+    h = [b.handle for b in bufs]
+    try:
+        _check_error(_lib.mfa_attention_forward_kvcache(
+            context.handle, *h[:6], h[6] if table is not None else None, B, Sq, H, Hkv, D, cap, page, npages, softmax_scale,
+            causal, -1 if window_size is None else int(window_size), in_prec, out_prec, None))
+    finally:
+        for b in bufs:
+            b.close()
+    return out, lse
+
+
 def flash_attention_varlen_backward(context: MFAContext, d_out, q, k, v, out, lse, cu_seqlens_q, cu_seqlens_k, *,
                                     causal: bool = False, softmax_scale: Optional[float] = None,
                                     input_precision: Precision = "fp32", window_size: Optional[int] = None,
