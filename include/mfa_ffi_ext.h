@@ -272,6 +272,33 @@ mfa_error_t mfa_attention_forward_kvcache(
     float softmax_scale, bool causal, int32_t window_size,
     mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream);
 
+/* mfa_attention_forward_kvcache with a per-sequence number of new query tokens: one call for a continuous-batching step that
+ * mixes 1-token decodes, speculative runs and prefill chunks.  Forward only.
+ * q is a [1, num_heads, total_q, D] view (strided handles give [total_q, H, D]); out has the same shape in output_precision
+ * (fp32, bf16 or fp16, may be strided); lse fp32 [num_heads, total_q] (log2 units) or NULL.
+ * cu_seqlens_q is int32 [num_seqs + 1]: 0, non-decreasing, ending at total_q.  Sequence b owns query rows [cu[b], cu[b+1]),
+ * sq_b = cu[b+1] - cu[b] of them (0 allowed, at most max_seqlen_q).  Row s of sequence b sits at position p = L_b - sq_b + s
+ * and sees key j < L_b iff (!causal || j <= p) && (window_size < 0 || p - j <= window_size).  A row that sees no key gets
+ * O = +0, L = -inf.  Caches, block_table, cache_seqlens, dtypes, head_dim, GQA and page rules are those of
+ * mfa_attention_forward_kvcache with batch_size = num_seqs.  max_seqlen_q sizes the work (1 <= max_seqlen_q <= total_q); it is
+ * never read back from the device.  With uniform segments (sq_b = max_seqlen_q) the results are bit-identical to
+ * mfa_attention_forward_kvcache with seq_len_q = max_seqlen_q.
+ * Host-readable cu_seqlens_q (host or managed memory) is checked: a first offset other than 0, a decrease, a last offset other
+ * than total_q or a segment longer than max_seqlen_q returns MFA_ERROR_INVALID_ARGS.  Device-resident offsets are not read by the
+ * host; the kernels clamp them to [0, total_q] and sq_b to [0, max_seqlen_q]: a segment longer than max_seqlen_q is served as its
+ * first max_seqlen_q rows (positions L_b - max_seqlen_q + s), and its rows past those see no key.  Rows outside every segment are
+ * not written.  Malformed arrays give wrong numbers but no access outside q, out, lse or the context's scratch.
+ * Streams, CUDA graphs and scratch behave as for mfa_attention_forward_kvcache: a replay may carry new cu_seqlens_q contents
+ * (same num_seqs, total_q and max_seqlen_q), new cache lengths and new cache contents.  The work split depends on the shape and
+ * the GPU only. */
+mfa_error_t mfa_attention_forward_kvcache_varlen(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t num_seqs, uint32_t total_q, uint32_t max_seqlen_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream);
+
 /* Device quantiser (GEMMQuantization.swift:305-623 / GEMMRuntimeQuantization.swift:80-181 contract):
  * src is a row-major [rows, cols] matrix of src_precision; scale[b] = absmax(block b) / 127 (int8) or / 7
  * (int4), floored at scale_floor when scale_floor > 0 (the reference GPU path uses 1e-8); codes =

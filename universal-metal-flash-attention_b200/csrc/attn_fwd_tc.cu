@@ -251,23 +251,40 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
   const int* const seg_k = MASKED ? nullptr : p.cu_k;
   // decode over a K/V cache (FwdTcParams::kv_len): the 16-bit unmasked instantiations serve it
   constexpr bool KVC = (MODE == kFwdF16 || MODE == kFwdBF16) && MASKED == 0;
+  // packed query-item slots: the sequence that owns this CTA's slot, found once (the int4 barrier words, unused by KVC modes)
+  int* const kv_owner = reinterpret_cast<int*>(smem_raw + (raw_full(0) - raw));
   // One CTA per work item = (batch, head, 256-row query block), x fastest so the CTAs of one head run together (K/V stay in L2).
-  struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half, L; };
+  // KVC: q0 = first query row of sequence b in the packed Q (kv_cu_q) or 0, sq = its number of new tokens
+  struct Item { int r0, h, b, hk, nt, j_lo, n, lid, half, L, q0, sq; };
   auto decode = [&](int w) {
     Item it;
     if constexpr (KVC) {
       if (p.kv_len) {        // (query item, split, KV head, sequence), query items fastest: they read the same keys
         it.half = 0; it.lid = 0;
-        const int qi = w % p.kv_nqi;
-        w /= p.kv_nqi;
-        const int split = w % p.kv_nsplit;
-        w /= p.kv_nsplit;
-        it.hk = w % p.Hkv; it.b = w / p.Hkv; it.h = it.hk * p.kv_g;
+        int qi, split;
+        if (p.kv_slots) {    // packed slots: (slot, split, KV head)
+          const int slot = w % p.kv_slots;
+          w /= p.kv_slots;
+          split = w % p.kv_nsplit;
+          it.hk = w / p.kv_nsplit;
+          it.b = *kv_owner;
+          qi = slot - kvc_first_slot(p.kv_cu_q, it.b, p.kv_total, 2 * p.kv_sqb);
+        } else {
+          qi = w % p.kv_nqi;
+          w /= p.kv_nqi;
+          split = w % p.kv_nsplit;
+          w /= p.kv_nsplit;
+          it.hk = w % p.Hkv; it.b = w / p.Hkv;
+        }
+        it.h = it.hk * p.kv_g;
+        it.q0 = p.kv_cu_q ? seg_offset(p.kv_cu_q, it.b, p.kv_total) : 0;
+        it.sq = p.kv_cu_q ? kvc_seq_len(p.kv_cu_q, it.b, p.kv_total, p.Sq) : p.Sq;
         it.r0 = 2 * qi * p.kv_sqb;                                         // first token of the item
-        it.nt = it.r0 + p.kv_sqb < p.Sq ? 2 : 1;
+        it.nt = it.r0 + p.kv_sqb < it.sq ? 2 : 1;
+        if (qi < 0 || it.r0 >= it.sq) { it.nt = 0; it.n = 0; return it; } // a slot past its sequence's rows
         it.L = kvc_len(p.kv_len, it.b, p.kv_cap);
         int klo, khi, t0, t1;
-        kvc_block_key_range(p.causal, p.window, it.L, p.Sq, it.r0, min(it.r0 + it.nt * p.kv_sqb, p.Sq), klo, khi);
+        kvc_block_key_range(p.causal, p.window, it.L, it.sq, it.r0, min(it.r0 + it.nt * p.kv_sqb, it.sq), klo, khi);
         kvc_split_tiles((p.kv_cap + 127) >> 7, p.kv_nsplit, split, t0, t1);
         it.j_lo = max(klo >> 7, t0);
         it.n = khi > klo ? max(0, min((khi + 127) >> 7, t1) - it.j_lo) : 0;
@@ -301,6 +318,14 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     if constexpr (MASKED) { if (p.mtiles) return __ldg(p.mtiles + (size_t)im.lid * p.m_nkt + it); }
     return im.j_lo + it;
   };
+  if constexpr (KVC) {
+    if (p.kv_len && p.kv_slots) {
+      if (threadIdx.x == 0) *kv_owner = kvc_slot_owner(p.kv_cu_q, p.nbatch, p.kv_total, 2 * p.kv_sqb, (int)blockIdx.x % p.kv_slots);
+      __syncthreads();
+    }
+    // a query-item slot without rows: no TMA, no partial (the combine kernel never reads its slot)
+    if (p.kv_len && decode(blockIdx.x).nt == 0) return;
+  }
 
   if (threadIdx.x == 256) {
     for (int t = 0; t < 2; ++t) {
@@ -352,9 +377,11 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
         }
         if constexpr (KVC) {
           if (p.kv_len) {      // GQA-packed tile: box (64, kv_sqb, G) of the (D, Sq, G, Hkv, B) map lands as rows g * kv_sqb + s
+            // (packed Q: the (D, total_q, G, Hkv, 1) map from row q0; box rows past the sequence are dead rows)
             mbar_arrive_expect_tx(q_full(t2), p.kv_qbytes);
+            const int qrow = im.q0 + r0 + t2 * p.kv_sqb, qb = p.kv_cu_q ? 0 : b;
 #pragma unroll
-            for (int c = 0; c < C::kQChunks; ++c) tma_load_5d(sQ + t2 * QT + c * CHB, &p.tq, q_full(t2), c * 64, r0 + t2 * p.kv_sqb, 0, hk, b);
+            for (int c = 0; c < C::kQChunks; ++c) tma_load_5d(sQ + t2 * QT + c * CHB, &p.tq, q_full(t2), c * 64, qrow, 0, hk, qb);
             return;
           }
         }
@@ -565,10 +592,11 @@ __global__ void __launch_bounds__(kThreads, 1) fwd_tc_kernel(const __grid_consta
     bool kvc = false;
     if constexpr (KVC) kvc = p.kv_len != nullptr;
     if (kvc) {
-      // token s of query head g = row / kv_sqb; rows past G * kv_sqb (stale shared memory) and tokens past Sq (zero-filled) see no key
+      // token s of query head g = row / kv_sqb; rows past G * kv_sqb (stale shared memory) and tokens past the sequence's
+      // (zero-filled, or another sequence's) see no key
       const int s = r0 + t * p.kv_sqb + row % p.kv_sqb;
       clo = chi = 0;
-      if (row < p.kv_rows && s < p.Sq) kvc_row_key_range(p.causal, p.window, im.L, p.Sq, s, clo, chi);
+      if (row < p.kv_rows && s < im.sq) kvc_row_key_range(p.causal, p.window, im.L, im.sq, s, clo, chi);
     } else {
       row_key_range(p.causal, p.window, p.Sq, p.Skv, seg_q, seg_k, p.nseq, r, clo, chi);
     }
@@ -1390,7 +1418,7 @@ cudaError_t launch_fwd_tc_kernel(const FwdTcParams& prm_in, int D, int mode, cud
   prm.nbatch = B;
   ptx::watchdog_bind();
   const bool wide = mode == kFwdWideF16 || mode == kFwdWideBF16;
-  const long long items = prm.kv_len ? (long long)prm.kv_nqi * prm.kv_nsplit * prm.Hkv * B
+  const long long items = prm.kv_len ? (prm.kv_slots ? (long long)prm.kv_slots : (long long)prm.kv_nqi * B) * prm.kv_nsplit * prm.Hkv
                                      : (long long)((prm.Sq + 255) / 256) * prm.H * B * (wide ? 2 : 1);
   if (items <= 0 || items > 0x7fffffffLL) return cudaErrorInvalidValue;
   const dim3 grid((unsigned)items, 1, 1);        // one CTA per work item
@@ -1564,23 +1592,38 @@ struct KvcCombine {
   void* o;
   long long o_sb, o_sh, o_ss;
   int o_dtype;
-  float* lse;                // [B, H, Sq] or null
-  int H, Hkv, Sq, D, G, sqb, rows, nqi, nsplit;
+  float* lse;                // [B, H, Sq], or [H, total_q] with cu_q
+  const int* cu_q;           // KvCacheParams::cu_q
+  int H, Hkv, Sq, D, G, sqb, rows, nqi, nsplit, slots;
+  int nseq, nrows;           // sequences, and query rows per grid z (Sq, or total_q with cu_q)
 };
 
-// One warp per query row (b, h, s), grid (Sq / 8, H, B): merges the row's partials of every split (lse_merge_*), writes O in the output's type and
-// stride and L.  Splits without a visible key (L_k = -inf) are not read.  Lane i holds head dims [4i, 4i + 4).
+// One warp per query row t of sequence z (without cu_q) or of the packed rows (with cu_q, whose sequence a binary search finds),
+// grid (nrows / 8, H, B or 1): merges the row's partials of every split (lse_merge_*), writes O in the output's type and stride
+// and L.  Splits without a visible key (L_k = -inf) are not read; rows of no sequence are not written, and rows of a sequence
+// past Sq (max_seqlen_q) get O = +0, L = -inf.  Lane i holds head dims [4i, 4i + 4).
 __global__ void __launch_bounds__(256) kvcache_combine_kernel(const KvcCombine c) {
-  const int s = blockIdx.x * 8 + (threadIdx.x >> 5), h = blockIdx.y, b = blockIdx.z;
+  const int t = blockIdx.x * 8 + (threadIdx.x >> 5), h = blockIdx.y, z = blockIdx.z;
   const int lane = threadIdx.x & 31;
-  if (s >= c.Sq) return;
-  const long long rid = ((long long)b * c.H + h) * c.Sq + s;
+  if (t >= c.nrows) return;
+  int b = z, s = t;
+  if (c.cu_q) {
+    b = segment_of(c.cu_q, c.nseq, t);
+    const int q0 = seg_offset(c.cu_q, b, c.nrows);
+    if (t < q0 || t >= seg_offset(c.cu_q, b + 1, c.nrows)) return;
+    s = t - q0;
+  }
+  const long long rid = ((long long)z * c.H + h) * c.nrows + t;
   const int hk = h / c.G, chunk = s / c.sqb;
   const int r = (h % c.G) * c.sqb + s % c.sqb;
-  const long long item0 = ((long long)b * c.Hkv + hk) * c.nsplit * c.nqi + (chunk >> 1);     // split k: item0 + k * nqi
-  auto slot = [&](int k) { return ((item0 + (long long)k * c.nqi) * 2 + (chunk & 1)) * c.rows + r; };
+  // the items of this row's query item, split k at item0 + k * step (KvCachePlan: per-sequence or packed slots)
+  const long long item0 = c.slots ? (long long)hk * c.nsplit * c.slots + kvc_first_slot(c.cu_q, b, c.nrows, 2 * c.sqb) + (chunk >> 1)
+                                  : ((long long)b * c.Hkv + hk) * c.nsplit * c.nqi + (chunk >> 1);
+  const int step = c.slots ? c.slots : c.nqi;
+  auto slot = [&](int k) { return ((item0 + (long long)k * step) * 2 + (chunk & 1)) * c.rows + r; };
+  const int nk = s < c.Sq ? c.nsplit : 0;
   float m = -CUDART_INF_F;
-  for (int k = lane; k < c.nsplit; k += 32) m = fmaxf(m, __ldg(c.l_part + slot(k)));
+  for (int k = lane; k < nk; k += 32) m = fmaxf(m, __ldg(c.l_part + slot(k)));
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, o));
   float4 acc = make_float4(-0.f, -0.f, -0.f, -0.f);       // -0 + x == x for every x: one split passes through unchanged
@@ -1588,11 +1631,11 @@ __global__ void __launch_bounds__(256) kvcache_combine_kernel(const KvcCombine c
   const int c0 = lane * 4;
   if (m != -CUDART_INF_F) {
     float wsum = 0.f;
-    for (int k = lane; k < c.nsplit; k += 32) wsum += lse_merge_weight(__ldg(c.l_part + slot(k)), m);
+    for (int k = lane; k < nk; k += 32) wsum += lse_merge_weight(__ldg(c.l_part + slot(k)), m);
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) wsum += __shfl_xor_sync(0xffffffffu, wsum, o);
     L = lse_merge_total(m, wsum);
-    for (int k = 0; k < c.nsplit; ++k) {
+    for (int k = 0; k < nk; ++k) {
       const float lk = __ldg(c.l_part + slot(k));
       if (lk == -CUDART_INF_F || c0 >= c.D) continue;
       const float wk = lse_merge_weight(lk, m) / wsum;
@@ -1602,7 +1645,7 @@ __global__ void __launch_bounds__(256) kvcache_combine_kernel(const KvcCombine c
   }
   if (m == -CUDART_INF_F) acc = make_float4(0.f, 0.f, 0.f, 0.f);   // a row without keys: O = +0
   if (c0 < c.D) {
-    const long long off = (long long)b * c.o_sb + (long long)h * c.o_sh + (long long)s * c.o_ss + c0;
+    const long long off = (long long)z * c.o_sb + (long long)h * c.o_sh + (long long)t * c.o_ss + c0;
     auto put = [&](int i, float x) {
       if (c.o_dtype == kF32) reinterpret_cast<float*>(c.o)[off + i] = x;
       else reinterpret_cast<uint16_t*>(c.o)[off + i] = (uint16_t)((c.o_dtype == kBF16 ? pack_bf16(x, 0.f) : pack_f16(x, 0.f)) & 0xffffu);
@@ -1621,8 +1664,15 @@ KvCachePlan kvcache_plan(const KvCacheParams& p, int sm_count) {
   k.rows = k.G * k.sqb;
   const int chunks = (p.Sq + k.sqb - 1) / k.sqb;
   k.nqi = (chunks + 1) / 2;
+  // query-item slots per KV head and split: nqi per sequence, or with per-sequence token counts the packed slots when fewer
+  long long slots = (long long)p.B * k.nqi;
+  k.slots = 0;
+  if (p.cu_q) {
+    const long long packed = p.total_q / (2 * k.sqb) + p.B;
+    if (packed < slots) slots = k.slots = (int)packed;
+  }
   // split the keys when the items of the call leave SMs idle: about one wave of CTAs, each split at least two 128-key tiles
-  const long long base = (long long)p.B * p.Hkv * k.nqi;
+  const long long base = slots * p.Hkv;
   const int ntiles = (p.cap + 127) / 128;
   long long ns = base < sm_count ? sm_count / base : 1;
   ns = std::max(1LL, std::min(ns, (long long)ntiles / 2));
@@ -1649,7 +1699,8 @@ cudaError_t launch_fwd_kvcache(const KvCacheParams& p, const KvCachePlan& k, voi
     box = std::gcd(p.page_size, 128);
   }
   const TensorView ov = {o_part, 2LL * k.rows * p.D, (int64_t)k.rows * p.D, p.D, 1};
-  if (!tc::make_map_gqa(&prm.tq, p.q, p.in_dtype, p.B, p.Hkv, k.G, p.Sq, p.D, k.sqb) ||
+  const bool packed_q = p.cu_q != nullptr;      // Q as [1, H, total_q, D]
+  if (!tc::make_map_gqa(&prm.tq, p.q, p.in_dtype, packed_q ? 1 : p.B, p.Hkv, k.G, packed_q ? p.total_q : p.Sq, p.D, k.sqb) ||
       !make_map(&prm.tk, kv[0], p.in_dtype, kB, p.Hkv, kS, p.D, box) || !make_map(&prm.tv, kv[1], p.in_dtype, kB, p.Hkv, kS, p.D, box) ||
       !make_map(&prm.to, ov, kF32, (int)k.items, 2, k.rows, p.D, k.rows))
     return cudaErrorInvalidValue;
@@ -1665,6 +1716,7 @@ cudaError_t launch_fwd_kvcache(const KvCacheParams& p, const KvCachePlan& k, voi
   prm.kv_npb = paged ? p.cap / p.page_size : 0; prm.kv_box = box;
   prm.kv_g = k.G; prm.kv_sqb = k.sqb; prm.kv_rows = k.rows; prm.kv_nqi = k.nqi; prm.kv_nsplit = k.nsplit;
   prm.kv_qbytes = (Dk / 64) * 128 * k.rows;
+  prm.kv_cu_q = p.cu_q; prm.kv_total = p.total_q; prm.kv_slots = k.slots;
   const bool bf = p.in_dtype == kBF16;
   cudaError_t e = launch_fwd_tc_kernel(prm, Dk, bf ? kFwdBF16 : kFwdF16, st, p.B);
   if (e != cudaSuccess) return e;
@@ -1672,8 +1724,10 @@ cudaError_t launch_fwd_kvcache(const KvCacheParams& p, const KvCachePlan& k, voi
   c.o_part = o_part; c.l_part = l_part;
   c.o = const_cast<void*>(p.o.ptr); c.o_sb = p.o.sb; c.o_sh = p.o.sh; c.o_ss = p.o.ss; c.o_dtype = p.o_dtype;
   c.lse = p.lse;
+  c.cu_q = p.cu_q;
   c.H = p.H; c.Hkv = p.Hkv; c.Sq = p.Sq; c.D = p.D; c.G = k.G; c.sqb = k.sqb; c.rows = k.rows; c.nqi = k.nqi; c.nsplit = k.nsplit;
-  kvcache_combine_kernel<<<dim3((unsigned)((p.Sq + 7) / 8), (unsigned)p.H, (unsigned)p.B), 256, 0, st>>>(c);
+  c.slots = k.slots; c.nseq = p.B; c.nrows = packed_q ? p.total_q : p.Sq;
+  kvcache_combine_kernel<<<dim3((unsigned)((c.nrows + 7) / 8), (unsigned)p.H, packed_q ? 1u : (unsigned)p.B), 256, 0, st>>>(c);
   static const char* names[2][2][2] = {{{"fwd_tc_fp16_d64_kvcache", "fwd_tc_fp16_d64_kvcache_split"},
                                         {"fwd_tc_fp16_d128_kvcache", "fwd_tc_fp16_d128_kvcache_split"}},
                                        {{"fwd_tc_bf16_d64_kvcache", "fwd_tc_bf16_d64_kvcache_split"},

@@ -187,6 +187,28 @@ __host__ __device__ inline void kvc_block_key_range(int causal, int window, int 
   if (hi < lo) hi = lo;
 }
 
+// A per-sequence number of new tokens (cu_q: sequence b owns query rows [cu[b], cu[b+1]) of total_q, at most max_sq of them).
+// Offsets come from memory the host may not have checked: they are clamped to [0, total_q] (seg_offset), and sq_b to
+// [0, max_sq], so the rows of a segment past max_sq are rows that see no key.
+__host__ __device__ inline int kvc_seq_len(const int* cu, int b, int total, int max_sq) {
+  const int n = seg_offset(cu, b + 1, total) - seg_offset(cu, b, total);
+  return n < 0 ? 0 : n > max_sq ? max_sq : n;
+}
+
+// Packed item slots: with T query tokens per work item, sequence b's items start at slot cu[b] / T + b.  That is strictly
+// increasing in b and leaves each sequence at least ceil(sq_b / T) slots, total_q / T + num_seqs slots in all.
+__host__ __device__ inline int kvc_first_slot(const int* cu, int b, int total, int T) { return seg_offset(cu, b, total) / T + b; }
+
+// The sequence whose slots hold `slot` (binary search; 0 before the first).
+__host__ __device__ inline int kvc_slot_owner(const int* cu, int nseq, int total, int T, int slot) {
+  int lo = 0, hi = nseq - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (kvc_first_slot(cu, mid, total, T) <= slot) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
 // Key tiles [t0, t1) of split k when the ntiles 128-key tiles of the capacity are shared by nsplit splits.
 __host__ __device__ inline void kvc_split_tiles(int ntiles, int nsplit, int k, int& t0, int& t1) {
   const int per = (ntiles + nsplit - 1) / nsplit;
@@ -200,22 +222,27 @@ __host__ __device__ inline void kvc_split_tiles(int ntiles, int nsplit, int k, i
 __device__ __forceinline__ float lse_merge_weight(float lk, float m) { return lk == -__int_as_float(0x7f800000) ? 0.f : exp2f(lk - m); }
 __device__ __forceinline__ float lse_merge_total(float m, float wsum) { return m + log2f(wsum); }
 
-// Attention of Sq new tokens per sequence against that sequence's K/V cache (mfa_attention_forward_kvcache).
+// Attention of new tokens per sequence against that sequence's K/V cache (mfa_attention_forward_kvcache and, with cu_q,
+// mfa_attention_forward_kvcache_varlen).
 struct KvCacheParams {
-  TensorView q, o;           // [B, H, Sq, D] views (o in o_dtype)
+  TensorView q, o;           // [B, H, Sq, D] views (o in o_dtype); with cu_q [1, H, total_q, D]
   TensorView k, v;           // contiguous cache: [B, Hkv, cap, D] views; paged: base of the [num_pages, page_size, Hkv, D] pools
-  float* lse;                // [B, H, Sq] or null
+  float* lse;                // [B, H, Sq] or null; with cu_q [H, total_q]
   const int* seqlens;        // [B] device
   const int* block_table;    // [B, cap / page_size] device, or null (contiguous cache)
-  int B, H, Hkv, Sq, D, cap, page_size, num_pages;
+  const int* cu_q;           // [B + 1] device query offsets, or null: Sq new tokens per sequence
+  int B, H, Hkv, Sq, D, cap, page_size, num_pages;   // with cu_q, Sq is the largest number of new tokens (max_seqlen_q)
+  int total_q;               // query rows in all (B * Sq without cu_q)
   float scale;
   int causal, window, in_dtype, o_dtype;
 };
 // How a call is cut into work items: G query heads per KV head share a tile as rows g * sqb + s (rows = G * sqb live rows), a
-// work item holds two such tiles of consecutive tokens (nqi items per (b, KV head)), and the keys of the capacity are shared by
-// nsplit splits.  Chosen from the shape and the SM count only, never from the lengths.
+// work item holds two such tiles of consecutive tokens, and the keys of the capacity are shared by nsplit splits.  The items of
+// one KV head and split sit in query-item slots: nqi per sequence, or with cu_q whichever is fewer of that and the packed
+// slots (kvc_first_slot, slots != 0).  Chosen from the shape and the SM count only, never from the lengths.
 struct KvCachePlan {
   int G, sqb, rows, nqi, nsplit;
+  int slots;                 // packed slots, or 0: nqi slots per sequence
   long long items;
   size_t o_bytes, l_bytes;   // scratch: partial O (fp32 [items][2][rows][D]) and L ([items][2][rows])
 };

@@ -1266,26 +1266,32 @@ mfa_error_t mfa_attention_backward_varlen(
   return backward_core(C_(context), a);
 }
 
-mfa_error_t mfa_attention_forward_kvcache(
+// mfa_attention_forward_kvcache (cu_seqlens_q null: seq_len_q new tokens per sequence) and
+// mfa_attention_forward_kvcache_varlen (sequence b owns query rows [cu[b], cu[b+1]) of total_q, at most seq_len_q of them).
+static mfa_error_t kvcache_forward(
     mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
-    mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
-    uint32_t batch_size, uint32_t seq_len_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t batch_size, uint32_t seq_len_q, uint32_t total_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
     uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
     float softmax_scale, bool causal, int32_t window_size,
     mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream) {
-  if (!context || !q || !k_cache || !v_cache || !out || !cache_seqlens) return MFA_ERROR_INVALID_ARGS;
   const uint32_t B = batch_size, Sq = seq_len_q, H = num_heads, Hkv = num_kv_heads ? num_kv_heads : num_heads, D = head_dim;
   const uint32_t cap = cache_capacity;
+  const bool packed = cu_seqlens_q != nullptr;
   const int dt = header_precision_to_dtype(input_precision), odt = header_precision_to_dtype(output_precision);
   if ((dt != kBF16 && dt != kF16) || !valid_float_dtype(odt)) return MFA_ERROR_INVALID_ARGS;
   if (B == 0 || Sq == 0 || H == 0 || H % Hkv || H / Hkv > 128 || D < 8 || D > 128 || (D & 7) || cap == 0) return MFA_ERROR_INVALID_ARGS;
   if (B > 65535 || Sq > 0x7fffffffu || H > 65535 || cap > 0x7fffff80u || !(softmax_scale > 0.f)) return MFA_ERROR_INVALID_ARGS;
+  if (packed && (total_q == 0 || total_q > 0x7fffffffu || Sq > total_q)) return MFA_ERROR_INVALID_ARGS;
   const bool paged = page_size > 0;
   if (paged ? (!block_table || (page_size & 15) || cap % page_size || num_pages == 0 || num_pages > 0x7fffffffu) : block_table != nullptr)
     return MFA_ERROR_INVALID_ARGS;
   if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
   Buffer *bq = B_(q), *bk = B_(k_cache), *bv = B_(v_cache), *bo = B_(out), *bl = B_(lse), *bs = B_(cache_seqlens), *bt = B_(block_table);
-  if (!view_fits(bq, B, H, Sq, D, 2) || !view_fits(bo, B, H, Sq, D, dtype_bytes(odt))) return MFA_ERROR_INVALID_ARGS;
+  Buffer* bc = B_(cu_seqlens_q);
+  // Q / O / L: [B, H, Sq] rows, or the [1, H, total_q] packed rows
+  const uint32_t qB = packed ? 1 : B, qS = packed ? total_q : Sq;
+  if (!view_fits(bq, qB, H, qS, D, 2) || !view_fits(bo, qB, H, qS, D, dtype_bytes(odt))) return MFA_ERROR_INVALID_ARGS;
   if (paged) {
     const size_t pool = (size_t)num_pages * page_size * Hkv * D * 2;
     if (bk->ndim || bv->ndim || bk->bytes < pool || bv->bytes < pool) return MFA_ERROR_INVALID_ARGS;
@@ -1293,8 +1299,15 @@ mfa_error_t mfa_attention_forward_kvcache(
   } else if (!view_fits(bk, B, Hkv, cap, D, 2) || !view_fits(bv, B, Hkv, cap, D, 2)) {
     return MFA_ERROR_INVALID_ARGS;
   }
-  if (bs->ndim || bs->bytes < (size_t)B * 4 || (bl && bl->bytes < (size_t)B * H * Sq * 4)) return MFA_ERROR_INVALID_ARGS;
-  // lengths and page ids the host can read are checked here; device-resident ones are clamped by the kernel
+  if (bs->ndim || bs->bytes < (size_t)B * 4 || (bl && bl->bytes < (size_t)qB * H * qS * 4)) return MFA_ERROR_INVALID_ARGS;
+  if (packed && (bc->ndim || bc->bytes < ((size_t)B + 1) * 4)) return MFA_ERROR_INVALID_ARGS;
+  // offsets, lengths and page ids the host can read are checked here; device-resident ones are clamped by the kernels
+  if (packed && bc->host) {
+    const int32_t* cu = reinterpret_cast<const int32_t*>(bc->host);
+    if (cu[0] != 0 || cu[B] != (int64_t)total_q) return MFA_ERROR_INVALID_ARGS;
+    for (uint32_t b = 0; b < B; ++b)
+      if (cu[b + 1] < cu[b] || (int64_t)cu[b + 1] - cu[b] > (int64_t)Sq) return MFA_ERROR_INVALID_ARGS;
+  }
   if (bs->host) {
     const int32_t* len = reinterpret_cast<const int32_t*>(bs->host);
     for (uint32_t b = 0; b < B; ++b)
@@ -1306,26 +1319,29 @@ mfa_error_t mfa_attention_forward_kvcache(
       if (ids[i] < 0 || (uint32_t)ids[i] >= num_pages) return MFA_ERROR_INVALID_ARGS;
   }
   const bool async = stream != nullptr;
-  if (async && (bq->mirrored || bk->mirrored || bv->mirrored || bo->mirrored || (bl && bl->mirrored) || bs->mirrored || (bt && bt->mirrored)))
+  if (async && (bq->mirrored || bk->mirrored || bv->mirrored || bo->mirrored || (bl && bl->mirrored) || bs->mirrored || (bt && bt->mirrored) ||
+                (bc && bc->mirrored)))
     return MFA_ERROR_INVALID_ARGS;
 
   Context* ctx = C_(context);
   std::lock_guard<std::recursive_mutex> lock(ctx->mu);
   DeviceGuard dg(ctx->device);
   KvCacheParams p;
-  p.q = view_of(bq, H, Sq, D, false);
-  p.o = view_of(bo, H, Sq, D, false);
+  p.q = view_of(bq, H, qS, D, false);
+  p.o = view_of(bo, H, qS, D, false);
   p.k = view_of(bk, Hkv, cap, D, false);
   p.v = view_of(bv, Hkv, cap, D, false);
   p.lse = bl ? reinterpret_cast<float*>(bl->dev) : nullptr;
   p.seqlens = reinterpret_cast<const int*>(bs->dev);
   p.block_table = paged ? reinterpret_cast<const int*>(bt->dev) : nullptr;
+  p.cu_q = packed ? reinterpret_cast<const int*>(bc->dev) : nullptr;
   p.B = (int)B; p.H = (int)H; p.Hkv = (int)Hkv; p.Sq = (int)Sq; p.D = (int)D; p.cap = (int)cap;
   p.page_size = (int)page_size; p.num_pages = (int)num_pages;
+  p.total_q = packed ? (int)total_q : 0;
   p.scale = softmax_scale; p.causal = causal ? 1 : 0; p.window = window_size < 0 ? -1 : window_size;
   p.in_dtype = dt; p.o_dtype = odt;
   // TMA: 16-byte aligned bases and outer strides; out only needs unit stride along D (the combine kernel stores elements)
-  if (!tc::view_ok(p.q, H, B) || p.o.sd != 1 || (!paged && (!tc::view_ok(p.k, Hkv, B) || !tc::view_ok(p.v, Hkv, B))) ||
+  if (!tc::view_ok(p.q, H, qB) || p.o.sd != 1 || (!paged && (!tc::view_ok(p.k, Hkv, B) || !tc::view_ok(p.v, Hkv, B))) ||
       (paged && ((reinterpret_cast<uintptr_t>(bk->dev) | reinterpret_cast<uintptr_t>(bv->dev)) & 15)))
     return MFA_ERROR_INVALID_ARGS;
   static int sm_count[kMaxDevices] = {0};
@@ -1355,7 +1371,7 @@ mfa_error_t mfa_attention_forward_kvcache(
   Sync sync{ctx, st, async, {}};
   cudaError_t e;
   if ((e = sync.in(bq)) != cudaSuccess || (e = sync.in(bk)) != cudaSuccess || (e = sync.in(bv)) != cudaSuccess ||
-      (e = sync.in(bs)) != cudaSuccess || (e = sync.in(bt)) != cudaSuccess)
+      (e = sync.in(bs)) != cudaSuccess || (e = sync.in(bt)) != cudaSuccess || (e = sync.in(bc)) != cudaSuccess)
     return cuda_fail(e, "h2d");
   Timer tm(ctx, st, !async);
   e = launch_fwd_kvcache(p, plan, scratch, st);
@@ -1371,6 +1387,32 @@ mfa_error_t mfa_attention_forward_kvcache(
   if ((e = sync.finish()) != cudaSuccess) return cuda_fail(e, "kvcache forward sync");
   tm.read();
   return MFA_SUCCESS;
+}
+
+mfa_error_t mfa_attention_forward_kvcache(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t batch_size, uint32_t seq_len_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream) {
+  if (!context || !q || !k_cache || !v_cache || !out || !cache_seqlens) return MFA_ERROR_INVALID_ARGS;
+  return kvcache_forward(context, q, k_cache, v_cache, out, lse, nullptr, cache_seqlens, block_table, batch_size, seq_len_q, 0,
+                         num_heads, num_kv_heads, head_dim, cache_capacity, page_size, num_pages, softmax_scale, causal, window_size,
+                         input_precision, output_precision, stream);
+}
+
+mfa_error_t mfa_attention_forward_kvcache_varlen(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t k_cache, mfa_buffer_t v_cache, mfa_buffer_t out, mfa_buffer_t lse,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    uint32_t num_seqs, uint32_t total_q, uint32_t max_seqlen_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    float softmax_scale, bool causal, int32_t window_size,
+    mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream) {
+  if (!context || !q || !k_cache || !v_cache || !out || !cu_seqlens_q || !cache_seqlens) return MFA_ERROR_INVALID_ARGS;
+  return kvcache_forward(context, q, k_cache, v_cache, out, lse, cu_seqlens_q, cache_seqlens, block_table, num_seqs, max_seqlen_q,
+                         total_q, num_heads, num_kv_heads, head_dim, cache_capacity, page_size, num_pages, softmax_scale, causal,
+                         window_size, input_precision, output_precision, stream);
 }
 
 // ---- quantised forward family ---------------------------------------------------------------------

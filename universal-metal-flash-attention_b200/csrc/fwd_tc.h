@@ -59,7 +59,7 @@ struct FwdTcParams {
   const int* cu_k;
   int nseq;
   // decode over a K/V cache (common.h, kvc_*) when kv_len is set; read by the unmasked 16-bit instantiations only.  A work item is
-  // (query item, split, KV head, sequence); its tiles hold the G query heads of one KV head as rows g * kv_sqb + s (tq is the 5-D
+  // (query item, split, KV head, sequence), query items fastest; its tiles hold the G query heads of one KV head as rows g * kv_sqb + s (tq is the 5-D
   // (D, Sq, G, Hkv, B) map), and it leaves a normalised partial: O through `to` at (column, 0, tile, item) and L in
   // lse[(item * 2 + tile) * kv_rows + row].
   const int* kv_len;       // [B] valid keys per sequence
@@ -67,6 +67,11 @@ struct FwdTcParams {
   int kv_cap, kv_page, kv_npages, kv_npb, kv_box;   // capacity, page size, pages in the pool, pages per sequence, rows per K / V box
   int kv_g, kv_sqb, kv_rows, kv_nqi, kv_nsplit;     // see KvCachePlan
   int kv_qbytes;           // bytes TMA writes into one Q tile
+  // per-sequence new tokens: sequence b owns query rows [kv_cu_q[b], kv_cu_q[b+1]) of kv_total, at most Sq of them, and tq is
+  // the (D, kv_total, G, Hkv, 1) map.  Null: Sq rows per sequence.  kv_slots != 0: packed slots (common.h, kvc_first_slot);
+  // a work item is then (slot, split, KV head), slots fastest.
+  const int* kv_cu_q;
+  int kv_total, kv_slots;
 };
 
 bool fwd_tc_mask_ok(const AttnParams& p);

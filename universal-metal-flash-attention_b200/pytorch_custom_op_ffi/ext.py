@@ -386,6 +386,75 @@ def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block
     return (out, lse) if return_lse else out
 
 
+def metal_flash_attention_varlen_with_kvcache(q, k_cache, v_cache, cu_seqlens_q, cache_seqlens, max_seqlen_q, block_table=None,
+                                              is_causal=True, scale=None, window_size=None, return_lse=False):
+    """metal_flash_attention_with_kvcache with a per-sequence number of new tokens: one call for a continuous-batching step
+    that mixes decodes, speculative runs and prefill chunks.  q is [total_q, H, D]; sequence b owns query rows
+    cu_seqlens_q[b]:cu_seqlens_q[b+1] (int32 CUDA tensor of num_seqs + 1 offsets: 0, non-decreasing, ending at total_q), and
+    row s of it sits at position cache_seqlens[b] - sq_b + s (is_causal / window_size bottom-right aligned).  Caches,
+    block_table and cache_seqlens are those of metal_flash_attention_with_kvcache with batch = num_seqs.  max_seqlen_q is a Python
+    int bounding every segment: it sizes the work, so nothing is read back from the device.  Returns O [total_q, H, D] in q's
+    dtype (and L fp32 [H, total_q] in log2 units with return_lse).  Enqueued on torch's current stream with no copies of q or
+    the caches; it can be captured in a CUDA graph after one call of the shape outside the capture, and replays may carry new
+    cu_seqlens_q contents, cache lengths and cache contents.  Forward only."""
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (q, k_cache, v_cache)):
+        raise RuntimeError("metal_flash_attention_varlen_with_kvcache has no backward: call it under torch.no_grad() or on "
+                           "tensors that do not require grad")
+    if isinstance(max_seqlen_q, bool) or not isinstance(max_seqlen_q, int) or max_seqlen_q < 1:
+        raise RuntimeError("metal_flash_attention_varlen_with_kvcache: max_seqlen_q must be a Python int >= 1")
+    if not q.is_cuda or q.dim() != 3 or q.stride(-1) != 1:
+        raise RuntimeError("metal_flash_attention_varlen_with_kvcache: q must be a 3-D CUDA tensor [total_q, heads, head_dim] with "
+                           "unit stride along head_dim")
+    for t in (k_cache, v_cache):
+        if not t.is_cuda or t.dim() != 4 or t.stride(-1) != 1:
+            raise RuntimeError("metal_flash_attention_varlen_with_kvcache: k_cache, v_cache must be 4-D CUDA tensors with unit "
+                               "stride along head_dim")
+    if q.dtype not in (torch.float16, torch.bfloat16) or k_cache.dtype != q.dtype or v_cache.dtype != q.dtype:
+        raise RuntimeError("metal_flash_attention_varlen_with_kvcache: q, k_cache, v_cache must share float16 or bfloat16")
+    T, H, D = q.shape
+    if k_cache.shape != v_cache.shape or k_cache.size(3) != D or H % k_cache.size(2):
+        raise RuntimeError(f"metal_flash_attention_varlen_with_kvcache: shapes q={tuple(q.shape)} "
+                           f"k_cache={tuple(k_cache.shape)} v_cache={tuple(v_cache.shape)}")
+    Hkv = k_cache.size(2)
+    for name, t in (("cu_seqlens_q", cu_seqlens_q), ("cache_seqlens", cache_seqlens), ("block_table", block_table)):
+        if t is not None and (t.dtype != torch.int32 or t.device != q.device or not t.is_contiguous()):
+            raise RuntimeError(f"metal_flash_attention_varlen_with_kvcache: {name} must be a contiguous int32 tensor on q's device")
+    if cu_seqlens_q.dim() != 1 or cu_seqlens_q.numel() < 2:
+        raise RuntimeError("metal_flash_attention_varlen_with_kvcache: cu_seqlens_q must hold num_seqs + 1 >= 2 offsets")
+    B = cu_seqlens_q.numel() - 1
+    if cache_seqlens.shape != (B,):
+        raise RuntimeError(f"metal_flash_attention_varlen_with_kvcache: cache_seqlens must be [{B}], "
+                           f"got {tuple(cache_seqlens.shape)}")
+    if block_table is None:
+        if k_cache.size(0) != B:
+            raise RuntimeError(f"metal_flash_attention_varlen_with_kvcache: contiguous caches need batch {B}")
+        cap, page, npages = k_cache.size(1), 0, 0
+    else:
+        if block_table.dim() != 2 or block_table.size(0) != B:
+            raise RuntimeError("metal_flash_attention_varlen_with_kvcache: block_table must be [num_seqs, pages per sequence]")
+        if not (k_cache.is_contiguous() and v_cache.is_contiguous()):
+            raise RuntimeError("metal_flash_attention_varlen_with_kvcache: paged pools must be contiguous")
+        npages, page = k_cache.size(0), k_cache.size(1)
+        cap = block_table.size(1) * page
+    if scale is None or scale <= 0.0:
+        scale = 1.0 / math.sqrt(D)
+    out = torch.empty(q.shape, device=q.device, dtype=q.dtype)
+    lse = torch.empty((H, T), device=q.device, dtype=torch.float32) if return_lse else None
+    lib_ctx = _context(q.device)
+    stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(q.device).cuda_stream or 0), q)
+    with _Bound(lib_ctx) as bind:
+        paged = block_table is not None
+        rc = _lib.mfa_attention_forward_kvcache_varlen(
+            lib_ctx.handle, _thd_handle(bind, q), bind(k_cache) if paged else _bshd_handle(bind, k_cache),
+            bind(v_cache) if paged else _bshd_handle(bind, v_cache), _thd_handle(bind, out), bind(lse), bind(cu_seqlens_q),
+            bind(cache_seqlens), bind(block_table), B, T, max_seqlen_q, H, Hkv, D, cap, page, npages, float(scale),
+            bool(is_causal), -1 if window_size is None or window_size < 0 else int(window_size), _PREC[q.dtype], _PREC[q.dtype],
+            stream)
+    if rc != 0:
+        raise RuntimeError(f"Metal Flash Attention kvcache varlen forward failed with code {rc}: {_ffi._get_error_string(rc)}")
+    return (out, lse) if return_lse else out
+
+
 def _dense_mask_f32(mask, query, Skv):
     """The quantised entry points take NULL or a dense fp32 additive [B,H,Sq,Skv] mask (metal_sdpa_backend.cpp:3210-3231)."""
     if mask is None:

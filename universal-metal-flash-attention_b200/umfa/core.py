@@ -480,6 +480,69 @@ def flash_attention_kvcache(context: MFAContext, q, k_cache, v_cache, cache_seql
     return out, lse
 
 
+def _kvcache_varlen_dims(q, k_cache, v_cache, cu_seqlens_q, cache_seqlens, block_table, max_seqlen_q):
+    """(num_seqs, total_q, max_seqlen_q, H, Hkv, D, capacity, page_size, num_pages, cu_q, lens, table) of a K/V-cache call with
+    a per-sequence number of new tokens: q [total_q, H, D]; caches as in _kvcache_dims with batch = num_seqs."""
+    if not isinstance(q, np.ndarray) or q.ndim != 3:
+        raise ValueError("kvcache varlen q must be a 3-D numpy array [total_q, heads, head_dim]")
+    cu_q = np.ascontiguousarray(cu_seqlens_q, np.int32)
+    if cu_q.ndim != 1 or cu_q.size < 2:
+        raise ValueError("cu_seqlens_q must be a 1-D int32 array of num_seqs + 1 offsets")
+    T, H, D = q.shape
+    n = cu_q.size - 1
+    seg = np.diff(cu_q.astype(np.int64))
+    if cu_q[0] != 0 or cu_q[-1] != T or (seg < 0).any():
+        raise ValueError(f"cu_seqlens_q must start at 0, never decrease and end at total_q = {T}")
+    if max_seqlen_q is None:
+        max_seqlen_q = max(int(seg.max()), 1)
+    if seg.max() > max_seqlen_q:
+        raise ValueError(f"a segment of cu_seqlens_q is longer than max_seqlen_q = {max_seqlen_q}")
+    # the cache checks of the fixed-length call, with one (empty) query token per sequence standing in for q
+    _, _, _, Hkv, _, cap, page, npages, lens, table = _kvcache_dims(np.empty((n, 0, H, D), q.dtype), k_cache, v_cache,
+                                                                    cache_seqlens, block_table)
+    return n, T, int(max_seqlen_q), H, Hkv, D, cap, page, npages, cu_q, lens, table
+
+
+def flash_attention_kvcache_varlen(context: MFAContext, q, k_cache, v_cache, cu_seqlens_q, cache_seqlens, block_table=None, *,
+                                   max_seqlen_q: Optional[int] = None, causal: bool = True, window_size: Optional[int] = None,
+                                   softmax_scale: Optional[float] = None, input_precision: Precision = "bf16",
+                                   output_precision: Precision = "fp32"):
+    """K/V-cache attention with a per-sequence number of new tokens (mfa_attention_forward_kvcache_varlen): a continuous-batching
+    step that mixes decodes, speculative runs and prefill chunks in one call.  q is [total_q, H, D]; sequence b owns query rows
+    cu_seqlens_q[b]:cu_seqlens_q[b+1] (sq_b of them, possibly 0), and row s of it sits at position cache_seqlens[b] - sq_b + s
+    (causal / window_size bottom-right aligned).  Caches, block_table and cache_seqlens are those of flash_attention_kvcache with
+    batch = num_seqs.  max_seqlen_q (the longest segment) is computed from cu_seqlens_q when None.  Returns (O [total_q, H, D] in
+    output_precision, L fp32 [H, total_q] in log2 units); rows that see no key get O = 0, L = -inf."""
+    n, T, msq, H, Hkv, D, cap, page, npages, cu_q, lens, table = _kvcache_varlen_dims(
+        q, k_cache, v_cache, cu_seqlens_q, cache_seqlens, block_table, max_seqlen_q)
+    if softmax_scale is None:
+        softmax_scale = 1.0 / np.sqrt(D)
+    in_prec, out_prec = _parse_precision(input_precision), _parse_precision(output_precision)
+    for name, x in (("q", q), ("k_cache", k_cache), ("v_cache", v_cache)):
+        _check_input_dtype(x, in_prec, name)
+    out = np.zeros(q.shape, {MFA_PRECISION_FP32: np.float32, MFA_PRECISION_FP16: np.float16}.get(out_prec, np.uint16))
+    lse = np.zeros((H, T), np.float32)
+    bshd = lambda arr, S, Hn: MFABuffer(context, arr, shape=(n, Hn, S, D), strides=(S * Hn * D, D, Hn * D, 1))
+    bufs = [_varlen_operand(context, np.ascontiguousarray(q), H, T, D, "thd")]
+    if table is None:
+        bufs += [bshd(np.ascontiguousarray(k_cache), cap, Hkv), bshd(np.ascontiguousarray(v_cache), cap, Hkv)]
+    else:
+        bufs += [MFABuffer(context, np.ascontiguousarray(k_cache)), MFABuffer(context, np.ascontiguousarray(v_cache))]
+    bufs += [_varlen_operand(context, out, H, T, D, "thd"), MFABuffer(context, lse), MFABuffer(context, cu_q),
+             MFABuffer(context, lens)]
+    if table is not None:
+        bufs.append(MFABuffer(context, table))
+    h = [b.handle for b in bufs]
+    try:
+        _check_error(_lib.mfa_attention_forward_kvcache_varlen(
+            context.handle, *h[:7], h[7] if table is not None else None, n, T, msq, H, Hkv, D, cap, page, npages,
+            softmax_scale, causal, -1 if window_size is None else int(window_size), in_prec, out_prec, None))
+    finally:
+        for b in bufs:
+            b.close()
+    return out, lse
+
+
 def flash_attention_varlen_backward(context: MFAContext, d_out, q, k, v, out, lse, cu_seqlens_q, cu_seqlens_k, *,
                                     causal: bool = False, softmax_scale: Optional[float] = None,
                                     input_precision: Precision = "fp32", window_size: Optional[int] = None,
