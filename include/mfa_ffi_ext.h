@@ -157,8 +157,8 @@ mfa_error_t mfa_attention_forward_accumulate(
     uint32_t acc_row_offset, uint32_t acc_rows, void* stream);
 
 /* P V precision of the quantised tensor-core forward (int8 / int4 codes, head_dim 128): e4m3 P and V on the fp8 tensor pipe
- * (default: BASELINE.json config 3, "int8 Q K^T and fp8 P V") or bf16 P with V's codes widened exactly to bf16.  Process-wide;
- * MFA_TCQ_PV=bf16|fp8 in the environment sets the initial value.  MFA_PRECISION_FP8_E4M3 exists for this setter only. */
+ * (default: BASELINE.json config 3, "int8 Q K^T and fp8 P V") or bf16 P with V's codes widened exactly to bf16.  Process-wide.
+ * MFA_PRECISION_FP8_E4M3 exists for this setter only. */
 #define MFA_PRECISION_FP8_E4M3 5
 mfa_error_t mfa_set_quantized_pv_precision(mfa_context_t context, int32_t precision);   /* MFA_PRECISION_BF16 or MFA_PRECISION_FP8_E4M3 */
 int32_t mfa_get_quantized_pv_precision(mfa_context_t context);

@@ -33,7 +33,7 @@ def run(name, n):
     res[name] = {"ms": t * 1e3, "tflops": flops / t / 1e12, "kernel": ctx.last_kernel}
 run("fp32_tensor_core", steps)
 a = o.clone()
-os.environ["MFA_DISABLE_TC32"] = "1"
+os.environ["MFA_DISABLE_TC"] = "1"
 run("fp32_simt", 2)
 d = (a.double() - o.double()).abs().max().item() / o.double().abs().max().item()
 res["max_rel_diff_tc_vs_simt"] = d

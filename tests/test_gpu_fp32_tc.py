@@ -107,12 +107,12 @@ def test_fp32_tc_flux_length_two_heads(ctx):
     check(ctx, rand((1, 2, 4608, 128), 17), rand((1, 2, 4608, 128), 18), rand((1, 2, 4608, 128), 19))
 
 
-def test_fp32_tc_matches_exact_simt_path(ctx, monkeypatch):
+def test_fp32_tc_matches_simt_path_under_disable_tc(ctx, monkeypatch):
     import umfa
     q, k, v = rand((1, 2, 640, 128), 20), rand((1, 2, 640, 128), 21), rand((1, 2, 640, 128), 22)
     a = umfa.flash_attention_forward(ctx, q, k, v, input_precision="fp32", layout="bhsd", causal=True)
     assert ctx.last_kernel == "fwd_tc_fp32split_d128"
-    monkeypatch.setenv("MFA_DISABLE_TC32", "1")
+    monkeypatch.setenv("MFA_DISABLE_TC", "1")
     b = umfa.flash_attention_forward(ctx, q, k, v, input_precision="fp32", layout="bhsd", causal=True)
     assert ctx.last_kernel == "fwd_simt"
     assert rel_max(a, b) < TOL

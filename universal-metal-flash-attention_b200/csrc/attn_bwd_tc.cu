@@ -150,11 +150,7 @@ struct BCfg {
   static constexpr int kChunkBytes = 128 * 128;
   // ring depths: A = operand used last (Q / K), B = dO / V.  STAGED (external mask tiles in shared memory): the 32 KB mask tile
   // takes the place of the second B stage at D = 128 (dO_i / V_j have one reader group per step and a whole step to reload)
-#if defined(MFA_BWD_RA) && defined(MFA_BWD_RB)                  // ring-depth experiments (unmasked kernels, D = 128)
-  static constexpr int kRA = (!STAGED && D == 128) ? MFA_BWD_RA : 3, kRB = (STAGED && D == 128) ? 1 : (D == 128 ? MFA_BWD_RB : 2);
-#else
   static constexpr int kRA = 3, kRB = (STAGED && D == 128) ? 1 : 2;
-#endif
   static constexpr int kMaskBytes = STAGED ? 128 * 128 * 2 : 0;  // one 128 x 128 tile of 16-bit terms (bool bytes use half)
   static constexpr int kStatBytes = 2 * 2 * 128 * 4;             // [slot][L|D][128], own 2-deep ring
   static constexpr int kSmem = (2 + kRA + kRB) * kTile + kMaskBytes + kStatBytes + 256 + 512;   // D = 128: 232192 of 232448 B
@@ -927,14 +923,14 @@ cudaError_t launch_bwd(const BwdTcParams& prm, int B, bool want_dq, bool want_dk
 }  // namespace
 
 bool bwd_tc_eligible(const AttnParams& p) {
-  if (getenv("MFA_DISABLE_TC") || getenv("MFA_DISABLE_TC_BWD")) return false;
+  if (getenv("MFA_DISABLE_TC")) return false;
   if (p.in_dtype != kBF16 && p.in_dtype != kF16) return false;
   if (p.do_dtype != p.in_dtype) return false;
   // head dims 64 / 128 as they are; other multiples of 8 up to 128 on the next kernel width: TMA zero-fills the missing columns
   // of Q / K / V / dO and clips the gradient stores, so those need the TMA-store epilogues
   if (p.D < 8 || p.D > 128 || (p.D & 7)) return false;
-  if (p.D != 64 && p.D != 128 && (getenv("MFA_DISABLE_TMA_STORE") || getenv("MFA_DISABLE_TC_PADDED_D"))) return false;
-  if (p.mask_kind != kMaskNone && p.mask && (p.mask_sk != 1 || getenv("MFA_DISABLE_TC_MASK"))) return false;
+  if (p.D != 64 && p.D != 128 && getenv("MFA_DISABLE_TMA_STORE")) return false;
+  if (p.mask_kind != kMaskNone && p.mask && p.mask_sk != 1) return false;
   if (p.Sq <= 0 || p.Skv <= 0 || p.B <= 0 || p.H <= 0 || p.Hkv <= 0 || p.H % p.Hkv) return false;
   if (p.B > 65535 || p.H > 65535) return false;
   if (!tc::view_ok(p.q, p.H, p.B) || !tc::view_ok(p.k, p.Hkv, p.B) || !tc::view_ok(p.v, p.Hkv, p.B) ||

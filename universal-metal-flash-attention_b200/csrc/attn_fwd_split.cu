@@ -143,7 +143,7 @@ unsigned split_grid(unsigned long long n4) {
 
 // fp32 operands, head_dim 128, unit stride along D with 16-byte aligned rows; masks as for the 16-bit kernel
 bool fwd_split_eligible(const AttnParams& p) {
-  if (getenv("MFA_DISABLE_TC") || getenv("MFA_DISABLE_TC32")) return false;
+  if (getenv("MFA_DISABLE_TC")) return false;
   // head dims below 128 (multiples of 8) ride the same kernel: the (hi, lo) scratch tensors keep the true head dim, TMA zero-fills
   if (p.in_dtype != kF32 || p.D < 8 || p.D > 128 || (p.D & 7) || p.accumulate || !fwd_tc_mask_ok(p)) return false;
   if (!(p.scale > 0.f) || p.Sq <= 0 || p.Skv <= 0 || p.B <= 0 || p.H <= 0 || p.Hkv <= 0 || p.H % p.Hkv) return false;

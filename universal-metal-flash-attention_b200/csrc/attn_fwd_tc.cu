@@ -1443,9 +1443,7 @@ cudaError_t launch_fwd_tc_kernel(const FwdTcParams& prm_in, int D, int mode, cud
 
 // external masks the tensor-core forward reads itself: keys contiguous (the row of a tile is one 128-element run)
 bool fwd_tc_mask_ok(const AttnParams& p) {
-  if (p.mask_kind == kMaskNone || !p.mask) return true;
-  if (getenv("MFA_DISABLE_TC_MASK")) return false;
-  return p.mask_sk == 1;
+  return p.mask_kind == kMaskNone || !p.mask || p.mask_sk == 1;
 }
 
 void fwd_tc_set_mask(FwdTcParams& prm, const AttnParams& p) {
@@ -1533,9 +1531,7 @@ bool fwd_tc_eligible(const AttnParams& p) {
   // columns zero-filled by TMA on the way in (tensor extent < box extent) and left out on the way out (the TMA store clips
   // them, the direct stores stop at FwdTcParams::dv)
   if (p.D < 8 || p.D > 256 || (p.D & 7)) return false;
-  const bool native_d = p.D == 64 || p.D == 128 || p.D == 256;
   if (p.D > 128 && p.accumulate) return false;
-  if (!native_d && getenv("MFA_DISABLE_TC_PADDED_D")) return false;
   if (!fwd_tc_mask_ok(p)) return false;
   if (!(p.scale > 0.f) || p.Sq <= 0 || p.Skv <= 0 || p.B <= 0 || p.H <= 0 || p.Hkv <= 0 || p.H % p.Hkv) return false;
   if (p.B > 65535 || p.H > 65535) return false;

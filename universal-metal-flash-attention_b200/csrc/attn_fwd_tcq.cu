@@ -4,7 +4,7 @@
 //   P V in e4m3 (default; BASELINE.json config 3 "int8 Q K^T and fp8 P V"):
 //     P'    = 2^6 exp2(S c - m) -> e4m3 in TMEM,  O += P' V_e4m3      (kind::f8f6f4, 2x the bf16 MMA rate, half the V bytes);
 //             V_e4m3 = e4m3(code * vs[key block] / vh) with one scale vh per (b, head), applied to O in the epilogue
-//   P V in bf16 (mfa_set_quantized_pv_precision(ctx, MFA_PRECISION_BF16) / MFA_TCQ_PV=bf16):
+//   P V in bf16 (mfa_set_quantized_pv_precision(ctx, MFA_PRECISION_BF16)):
 //     P     = exp2(S c - m)  -> bf16 in TMEM,  O += (P * vs[key block]) V_codes      (kind::f16, V codes exact in bf16)
 // Replaces the reference's quantised forward (metal-flash-attention/Sources/FlashAttention/Attention/
 // QuantizedAttention.swift:71-91,358-463 -- attention on dequantised int8 operands with fp32 statistics) for symmetric
@@ -108,7 +108,7 @@ unsigned grid_for(uint64_t n, int threads) {
   return (unsigned)(g < cap ? (g ? g : 1) : cap);
 }
 
-int g_tcq_pv = -1;       // 0 = e4m3 P V (default), 1 = bf16 P V
+int g_tcq_pv = 0;        // 0 = e4m3 P V (default), 1 = bf16 P V
 
 bool scales_ok(const QuantView& q, bool need64) {
   if (q.zero_point != 0) return false;
@@ -133,17 +133,14 @@ cudaError_t launch_codes_to_bf16(const void* codes, int bits, void* dst, uint64_
 }  // namespace mfa
 
 namespace mfa {
-// P V precision of the quantised tensor-core forward: e4m3 (default) or bf16; MFA_TCQ_PV=bf16|fp8 sets the initial value
-int fwd_tcq_pv_mode() {
-  if (g_tcq_pv < 0) { const char* e = getenv("MFA_TCQ_PV"); g_tcq_pv = (e && (e[0] == 'b' || e[0] == 'B')) ? 1 : 0; }
-  return g_tcq_pv;
-}
+// P V precision of the quantised tensor-core forward: e4m3 (default) or bf16
+int fwd_tcq_pv_mode() { return g_tcq_pv; }
 void fwd_tcq_set_pv_mode(int bf16) { g_tcq_pv = bf16 ? 1 : 0; }
 
 // Eligibility of the int8 tensor-core forward: int8 or int4 codes, symmetric, head_dim 128, contiguous operands, per-tensor
 // scales or per-block scales with K / V blocks that are multiples of 64 tokens, no external mask.
 bool fwd_tcq_eligible(const AttnParams& p) {
-  if (getenv("MFA_DISABLE_TC") || getenv("MFA_DISABLE_TCQ")) return false;
+  if (getenv("MFA_DISABLE_TC")) return false;
   if (p.in_dtype != kI8 && p.in_dtype != kI4) return false;
   if (p.D != 128 || !fwd_tc_mask_ok(p)) return false;
   if (!(p.scale > 0.f) || p.Sq <= 0 || p.Skv <= 0 || p.B <= 0 || p.H <= 0 || p.Hkv <= 0 || p.H % p.Hkv) return false;

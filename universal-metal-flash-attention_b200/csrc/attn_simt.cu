@@ -479,16 +479,12 @@ cudaError_t launch_dterm(const AttnParams& p, cudaStream_t st) {
                    (p.D % 4) == 0 && !(reinterpret_cast<uintptr_t>(p.o.ptr) & 15) && !(reinterpret_cast<uintptr_t>(p.d_o.ptr) & 7) &&
                    !((p.o.ss | p.o.sh | p.o.sb) & 3) && !((p.d_o.ss | p.d_o.sh | p.d_o.sb) & 3);
   if (vec && (int64_t)p.B * p.H <= 65535) {
-    // rows per warp (8 warps per block): 4 by default -- FLUX shape, 85 MB in: 24.0 us with 1 row per warp, 20.0 with 2,
-    // 15.5 us = 5.5 TB/s = 0.84 of the measured copy rate with 4 (profiles/r02be_launches_dterm*.csv); MFA_DTERM_ROWS = 1 | 2 | 4 | 8
-    static int kr = 0;
-    if (!kr) { const char* e = getenv("MFA_DTERM_ROWS"); kr = e ? atoi(e) : 4; if (kr != 1 && kr != 2 && kr != 4 && kr != 8) kr = 4; }
-    const dim3 nb((unsigned)((p.Sq + 8 * kr - 1) / (8 * kr)), (unsigned)(p.B * p.H));
-    const bool bf = p.do_dtype == kBF16;
-    if (kr == 8) { if (bf) dterm_vec_kernel<true, 8><<<nb, 256, 0, st>>>(p); else dterm_vec_kernel<false, 8><<<nb, 256, 0, st>>>(p); }
-    else if (kr == 4) { if (bf) dterm_vec_kernel<true, 4><<<nb, 256, 0, st>>>(p); else dterm_vec_kernel<false, 4><<<nb, 256, 0, st>>>(p); }
-    else if (kr == 2) { if (bf) dterm_vec_kernel<true, 2><<<nb, 256, 0, st>>>(p); else dterm_vec_kernel<false, 2><<<nb, 256, 0, st>>>(p); }
-    else { if (bf) dterm_vec_kernel<true, 1><<<nb, 256, 0, st>>>(p); else dterm_vec_kernel<false, 1><<<nb, 256, 0, st>>>(p); }
+    // rows per warp (8 warps per block): 4 -- FLUX shape, 85 MB in: 24.0 us with 1 row per warp, 20.0 with 2,
+    // 15.5 us = 5.5 TB/s = 0.84 of the measured copy rate with 4 (profiles/r02be_launches_dterm*.csv)
+    constexpr int R = 4;
+    const dim3 nb((unsigned)((p.Sq + 8 * R - 1) / (8 * R)), (unsigned)(p.B * p.H));
+    if (p.do_dtype == kBF16) dterm_vec_kernel<true, R><<<nb, 256, 0, st>>>(p);
+    else dterm_vec_kernel<false, R><<<nb, 256, 0, st>>>(p);
   } else {
     dterm_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(p);
   }

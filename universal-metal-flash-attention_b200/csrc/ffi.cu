@@ -660,7 +660,7 @@ mfa_error_t backward_core(Context* ctx, const BwdArgs& a) {
   // Other head dims keep the exact SIMT route (dequantise on load).
   const char* tcq_name = nullptr;
   if ((p.in_dtype == kI8 || p.in_dtype == kI4) && a.D == 128 && !a.tq && !a.tk && !a.tv && !a.to &&
-      !getenv("MFA_DISABLE_TC") && !getenv("MFA_DISABLE_TCQ") && !getenv("MFA_DISABLE_TC_BWD")) {
+      !getenv("MFA_DISABLE_TC")) {
     auto packed_ok = [&](const TensorView& t, int64_t Hn, int64_t S) {
       return t.sd == 1 && t.ss == (int64_t)a.D && t.sh == S * (int64_t)a.D && t.sb == Hn * S * (int64_t)a.D;
     };

@@ -130,7 +130,7 @@ __global__ void __launch_bounds__(256) quant_span_kernel(const T* __restrict__ s
                                                          uint32_t block_rows, uint64_t group_rows, uint32_t nb_per_group,
                                                          uint64_t nblocks, float floor_v) {
   __shared__ float red[8];
-  const int nworker = WARP ? 32 : (int)blockDim.x;           // CTA variant: 256 or 128 threads (launcher)
+  const int nworker = WARP ? 32 : (int)blockDim.x;           // CTA variant: 256 threads (launcher)
   const int wid = WARP ? (threadIdx.x >> 5) : 0;
   const int lane = WARP ? (threadIdx.x & 31) : threadIdx.x;
   const uint64_t blk = WARP ? (uint64_t)blockIdx.x * 8 + wid : blockIdx.x;
@@ -185,77 +185,6 @@ __global__ void __launch_bounds__(256) quant_span_kernel(const T* __restrict__ s
 #pragma unroll
       for (int i = 0; i < 8; ++i) out |= (uint32_t)((q[i] + 8) & 0xF) << (4 * i);
       *reinterpret_cast<uint32_t*>(bcodes + (e >> 1)) = out;
-    }
-  }
-}
-
-// ---- single trip for 16-bit sources and blocks of up to 8192 elements (the 64-token x 128-dim blocks of the attention path): a CTA
-// per block, every thread ISSUES its (up to four) 16-byte loads before the first use and keeps the raw words in registers for the
-// apply step.  The two-trip kernel above walks its span in a loop whose abs-max consumes each load right away -- four serialised
-// memory latencies per thread in the first trip and four more L2 latencies in the second: 21.5 us per 28 MB FLUX tensor, 0.30 of
-// the copy rate, with only ~1.5 waves of CTAs (profiles/r02bg_helpers.csv).  Same code rule (quant_codes8): bit-exact.
-// MEASURED: no faster -- 21.8 us against 21.5 us (profiles/r02bh_helpers_single.csv / _two.csv), so the latencies were not the
-// limit; what is left is the ~16 instructions per element of convert / scale / round / tie check / pack (8 M warp instructions per
-// tensor).  Kept as an opt-in (MFA_QUANT_SINGLE_TRIP=1) with its parity tests; the two-trip kernel stays the default.
-template <typename T, int BITS>
-__global__ void __launch_bounds__(256) quant_span_reg_kernel(const T* __restrict__ src, uint8_t* __restrict__ codes,
-                                                             float* __restrict__ scales, uint64_t rows, uint64_t cols,
-                                                             uint32_t block_rows, uint64_t group_rows, uint32_t nb_per_group,
-                                                             float floor_v) {
-  static_assert(sizeof(T) == 2, "16-bit sources");
-  __shared__ float red[8];
-  const uint64_t blk = blockIdx.x;
-  const uint64_t g = blk / nb_per_group, lb = blk % nb_per_group;
-  const uint64_t r0 = g * group_rows + lb * block_rows;
-  uint64_t r1 = r0 + block_rows;
-  if (r1 > (g + 1) * group_rows) r1 = (g + 1) * group_rows;
-  if (r1 > rows) r1 = rows;
-  const uint64_t e0 = r0 * cols;
-  const uint32_t n = (uint32_t)((r1 - r0) * cols);              // <= 8192, a multiple of 8 (launcher)
-  const T* base = src + e0;
-  uint4 raw[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const uint32_t idx = (uint32_t)(k * 256 + threadIdx.x) * 8;
-    raw[k] = idx < n ? *reinterpret_cast<const uint4*>(base + idx) : make_uint4(0u, 0u, 0u, 0u);
-  }
-  float amax = 0.f;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const T* e = reinterpret_cast<const T*>(&raw[k]);
-#pragma unroll
-    for (int i = 0; i < 8; ++i) amax = fmaxf(amax, fabsf(to_f32<T>(e[i])));
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) amax = fmaxf(amax, __shfl_xor_sync(0xffffffffu, amax, o));
-  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = amax;
-  __syncthreads();
-  amax = red[0];
-#pragma unroll
-  for (int i = 1; i < 8; ++i) amax = fmaxf(amax, red[i]);
-  const float sc = make_scale(amax, BITS, floor_v);
-  const float inv = inv_scale(sc);
-  if (threadIdx.x == 0) scales[blk] = sc;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const uint32_t idx = (uint32_t)(k * 256 + threadIdx.x) * 8;
-    if (idx >= n) continue;
-    const T* e = reinterpret_cast<const T*>(&raw[k]);
-    int q[8];
-    float x[8];
-#pragma unroll
-    for (int i = 0; i < 8; ++i) x[i] = to_f32<T>(e[i]);
-    quant_codes8(x, sc, inv, BITS, q);
-    if (BITS == 8) {
-      uint2 out;
-      out.x = pack4_bytes(q[0], q[1], q[2], q[3]);
-      out.y = pack4_bytes(q[4], q[5], q[6], q[7]);
-      *reinterpret_cast<uint2*>(codes + e0 + idx) = out;
-    } else {
-      uint32_t out = 0;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) out |= (uint32_t)((q[i] + 8) & 0xF) << (4 * i);
-      *reinterpret_cast<uint32_t*>(codes + ((e0 + idx) >> 1)) = out;
     }
   }
 }
@@ -547,22 +476,13 @@ cudaError_t quantize_typed(const T* src, uint8_t* codes, float* scales, uint64_t
       unsigned grid = (unsigned)((nblocks + 7) / 8);
       if (bits == 8) quant_span_kernel<T, 8, true><<<grid, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
       else quant_span_kernel<T, 4, true><<<grid, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
-    } else if (sizeof(T) == 2 && span <= 8192 && nblocks <= 0x7fffffffull && getenv("MFA_QUANT_SINGLE_TRIP")) {
-      if constexpr (sizeof(T) == 2) {
-        if (bits == 8) quant_span_reg_kernel<T, 8><<<(unsigned)nblocks, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, floor_v);
-        else quant_span_reg_kernel<T, 4><<<(unsigned)nblocks, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, floor_v);
-      }
     } else {
       unsigned grid = (unsigned)nblocks;
       // CTA size: with 256 threads ~6 CTAs fit an SM (888 on the chip), so the 1728 blocks of a FLUX tensor run as two waves;
       // 128-thread CTAs (13 per SM) hold them all at once -- and measure SLOWER, 20.3 against 18.2 us under ncu
-      // (profiles/r02bo_helpers_{128,256}.csv): the wave count is not what bounds this pass either.  MFA_QUANT_SPAN_THREADS=128 keeps
-      // the experiment reachable.
-      static int forced = -1;
-      if (forced < 0) { const char* e = getenv("MFA_QUANT_SPAN_THREADS"); forced = e ? atoi(e) : 0; }
-      const unsigned threads = forced == 128 ? 128u : 256u;
-      if (bits == 8) quant_span_kernel<T, 8, false><<<grid, threads, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
-      else quant_span_kernel<T, 4, false><<<grid, threads, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
+      // (profiles/r02bo_helpers_{128,256}.csv): the wave count is not what bounds this pass either.
+      if (bits == 8) quant_span_kernel<T, 8, false><<<grid, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
+      else quant_span_kernel<T, 4, false><<<grid, 256, 0, st>>>(src, codes, scales, rows, cols, br, group_rows, nb_per_group, nblocks, floor_v);
     }
     ++g_launch_count;
     g_last_kernel = "quant_span";
@@ -733,7 +653,7 @@ void launch_hadamard_warp(float* data, uint32_t num_blocks, cudaStream_t st) {
 cudaError_t launch_hadamard(float* data, uint32_t block_size, uint32_t num_blocks, cudaStream_t st) {
   if (block_size == 0 || block_size > 1024 || (block_size & (block_size - 1))) return cudaErrorInvalidValue;
   if (num_blocks == 0) return cudaSuccess;
-  if (block_size >= 32 && (reinterpret_cast<uintptr_t>(data) & 15) == 0 && !getenv("MFA_HADAMARD_SMEM")) {
+  if (block_size >= 32 && (reinterpret_cast<uintptr_t>(data) & 15) == 0) {
     switch (block_size / 32) {
       case 1: launch_hadamard_warp<1>(data, num_blocks, st); break;
       case 2: launch_hadamard_warp<2>(data, num_blocks, st); break;
