@@ -299,6 +299,42 @@ mfa_error_t mfa_attention_forward_kvcache_varlen(
     float softmax_scale, bool causal, int32_t window_size,
     mfa_precision_t input_precision, mfa_precision_t output_precision, void* stream);
 
+/* Writes the K / V of new tokens into a K/V cache in one launch, ahead of mfa_attention_forward_kvcache{,_varlen}: K (and
+ * optionally Q) is rotated on the way (rotary embedding), V is copied unchanged.
+ * Layouts: with cu_seqlens_q NULL every sequence has max_seqlen_q new tokens, q / q_out are [num_seqs, num_heads, max_seqlen_q, D]
+ * views and k_new / v_new [num_seqs, num_kv_heads, max_seqlen_q, D] views (strided handles give BSHD); total_q is ignored.  With
+ * cu_seqlens_q (int32 [num_seqs + 1], as in mfa_attention_forward_kvcache_varlen) they are [1, heads, total_q, D] views (THD).
+ * Caches, block_table, cache_seqlens, page rules, dtypes (bf16 / fp16) and head_dim (a multiple of 8 up to 128) are those of
+ * mfa_attention_forward_kvcache; views need 16-byte aligned bases and outer strides.
+ * Positions follow the attention calls: sequence b has sq_b new tokens (max_seqlen_q, or cu[b+1] - cu[b]) and cache_seqlens[b] =
+ * L_b counts them.  Token s goes to cache row p = L_b - sq_b + s (contiguous: row p of sequence b; paged: row p % page_size of
+ * page block_table[b][p / page_size]) and is rotated with table row p.  Tokens with p < 0 (sq_b > L_b) write no K / V; their Q
+ * is rotated with table row 0.
+ * Rotary: rotary_cos / rotary_sin are fp32 [rotary_rows, rotary_dim / 2], one angle per pair (the table layout of flash-attn's
+ * flash_attn_with_kvcache); both NULL with rotary_dim 0 = no rotation.  rotary_dim is a multiple of 16, at most D; columns from
+ * rotary_dim to D are copied unrotated.  rotary_interleaved pairs (2i, 2i+1); otherwise pairs are (i, i + rotary_dim / 2) (the
+ * half-split "rotate_half" layout of Llama, Mistral, Qwen, NeoX).  A pair becomes (x0 c - x1 s, x0 s + x1 c), computed in fp32 and
+ * rounded once to the cache dtype, exactly as mfa_rope_rotate_encode_mtl rounds it.
+ * q and q_out are both NULL or both set (then the tables are required); q_out may be q itself.  The attention call then reads q_out.
+ * Host-readable cu_seqlens_q, cache_seqlens and block_table are checked as in the attention calls, and with tables also
+ * L_b <= rotary_rows; a failed check returns MFA_ERROR_INVALID_ARGS and nothing is written.  Device-resident arrays are not read by
+ * the host; the kernel clamps lengths to [0, cache_capacity], offsets to [0, total_q], sq_b to [0, max_seqlen_q], page ids to
+ * [0, num_pages) and table rows to [0, rotary_rows), so malformed arrays give wrong numbers but no access outside the buffers.
+ * Tokens outside every segment, or past max_seqlen_q in theirs, are not written at all (neither cache rows nor q_out).
+ * If two tokens of one call map to the same cache row (possible with pages shared between sequences, e.g. a common prefix), which
+ * value lands there is unspecified.
+ * stream != NULL only enqueues work (all buffers device-resident) and uses no scratch, so the call can be captured in a CUDA graph
+ * with no earlier call, and replayed with new contents of every input, lengths and offsets included.  stream NULL blocks on the
+ * context stream; host-mirrored caches and q_out are copied back like any other output. */
+mfa_error_t mfa_kvcache_append(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t q_out, mfa_buffer_t k_new, mfa_buffer_t v_new,
+    mfa_buffer_t k_cache, mfa_buffer_t v_cache,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    mfa_buffer_t rotary_cos, mfa_buffer_t rotary_sin, uint32_t rotary_rows, uint16_t rotary_dim, bool rotary_interleaved,
+    uint32_t num_seqs, uint32_t total_q, uint32_t max_seqlen_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    mfa_precision_t input_precision, void* stream);
+
 /* Device quantiser (GEMMQuantization.swift:305-623 / GEMMRuntimeQuantization.swift:80-181 contract):
  * src is a row-major [rows, cols] matrix of src_precision; scale[b] = absmax(block b) / 127 (int8) or / 7
  * (int4), floored at scale_floor when scale_floor > 0 (the reference GPU path uses 1e-8); codes =

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "lib")
 LIB = os.path.join(OUT_DIR, "libMFAFFI.so")
-SOURCES = ["ffi.cu", "attn_simt.cu", "attn_fwd_tc.cu", "attn_bwd_tc.cu", "attn_fwd_tcq.cu", "attn_fwd_split.cu", "quant.cu", "ring.cu"]
+SOURCES = ["ffi.cu", "attn_simt.cu", "attn_fwd_tc.cu", "attn_bwd_tc.cu", "attn_fwd_tcq.cu", "attn_fwd_split.cu", "quant.cu", "ring.cu", "kvcache_append.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "--cudart", "static",
          "-Xcompiler", "-fPIC,-O3", "--expt-relaxed-constexpr", "-ccbin", "/usr/bin/g++"]

@@ -222,6 +222,31 @@ __host__ __device__ inline void kvc_split_tiles(int ntiles, int nsplit, int k, i
 __device__ __forceinline__ float lse_merge_weight(float lk, float m) { return lk == -__int_as_float(0x7f800000) ? 0.f : exp2f(lk - m); }
 __device__ __forceinline__ float lse_merge_total(float m, float wsum) { return m + log2f(wsum); }
 
+// Rotary embedding of one pair: (x0, x1) -> (x0 c - x1 s, x0 s + x1 c) in fp32, each product pair fused the same way in every
+// kernel that rotates (rope_kernel, kvcache_append_kernel), so their outputs agree bit for bit.
+__device__ __forceinline__ void rope_pair(float x0, float x1, float c, float s, float& y0, float& y1) {
+  y0 = __fmaf_rn(x0, c, -__fmul_rn(x1, s));
+  y1 = __fmaf_rn(x0, s, __fmul_rn(x1, c));
+}
+
+// Writing new tokens' K / V into a K/V cache (mfa_kvcache_append), K and optionally Q rotated on the way.  Token s of sequence b
+// goes to cache row p = L_b - sq_b + s (the decode rule above) and reads rotary table row p.
+struct KvAppendParams {
+  TensorView q, q_out;       // [B, H, Sq, D] views (with cu_q [1, H, total_q, D]); q.ptr == null: Q is not rotated
+  TensorView k_new, v_new;   // [B, Hkv, Sq, D] views (with cu_q [1, Hkv, total_q, D])
+  TensorView k, v;           // caches as in KvCacheParams
+  const int* seqlens;        // [B] device
+  const int* block_table;    // [B, cap / page_size] device, or null (contiguous cache)
+  const int* cu_q;           // [B + 1] device query offsets, or null: Sq new tokens per sequence
+  const float* cos_t;        // fp32 [rotary_rows, rotary_dim / 2] (one angle per pair), or null: no rotation
+  const float* sin_t;
+  int rotary_rows, rotary_dim, interleaved;   // interleaved: pairs (2i, 2i+1); else half-split pairs (i, i + rotary_dim / 2)
+  int B, H, Hkv, Sq, D, cap, page_size, num_pages;   // with cu_q, Sq is max_seqlen_q
+  int total_q;               // token rows in all (B * Sq without cu_q)
+  int dtype;                 // kBF16 or kF16
+};
+cudaError_t launch_kvcache_append(const KvAppendParams& p, cudaStream_t st);
+
 // Attention of new tokens per sequence against that sequence's K/V cache (mfa_attention_forward_kvcache and, with cu_q,
 // mfa_attention_forward_kvcache_varlen).
 struct KvCacheParams {

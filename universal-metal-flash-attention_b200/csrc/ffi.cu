@@ -1266,6 +1266,59 @@ mfa_error_t mfa_attention_backward_varlen(
   return backward_core(C_(context), a);
 }
 
+// The cache geometry shared by the K/V-cache attention calls and mfa_kvcache_append.  Sq is seq_len_q, or with packed
+// (cu_seqlens_q) rows the largest number of new tokens of a sequence, total_q the number of packed rows.
+struct KvCacheShape {
+  uint32_t B, Sq, total_q, H, Hkv, D, cap, page_size, num_pages;
+  int dtype;
+  bool packed, paged;
+};
+
+// Scalar arguments, checked before anything is known about the device.
+static bool kvcache_shape_ok(const KvCacheShape& s, mfa_buffer_t block_table) {
+  if (s.dtype != kBF16 && s.dtype != kF16) return false;
+  if (s.B == 0 || s.Sq == 0 || s.H == 0 || s.H % s.Hkv || s.H / s.Hkv > 128 || s.D < 8 || s.D > 128 || (s.D & 7) || s.cap == 0) return false;
+  if (s.B > 65535 || s.Sq > 0x7fffffffu || s.H > 65535 || s.cap > 0x7fffff80u) return false;
+  if (s.packed && (s.total_q == 0 || s.total_q > 0x7fffffffu || s.Sq > s.total_q)) return false;
+  if (s.paged ? (!block_table || (s.page_size & 15) || s.cap % s.page_size || s.num_pages == 0 || s.num_pages > 0x7fffffffu)
+              : block_table != nullptr)
+    return false;
+  return true;
+}
+
+// The caches, cache_seqlens, block_table and cu_seqlens_q handles cover their shapes; offsets, lengths (at most max_len) and page
+// ids the host can read are checked here.  Device-resident ones are left to the kernels, which clamp them.
+static mfa_error_t check_kvcache_arrays(const KvCacheShape& s, const Buffer* bk, const Buffer* bv, const Buffer* bs, const Buffer* bt,
+                                        const Buffer* bc, uint32_t max_len) {
+  const uint32_t B = s.B, cap = s.cap;
+  if (s.paged) {
+    const size_t pool = (size_t)s.num_pages * s.page_size * s.Hkv * s.D * 2;
+    if (bk->ndim || bv->ndim || bk->bytes < pool || bv->bytes < pool) return MFA_ERROR_INVALID_ARGS;
+    if (bt->ndim || bt->bytes < (size_t)B * (cap / s.page_size) * 4) return MFA_ERROR_INVALID_ARGS;
+  } else if (!view_fits(bk, B, s.Hkv, cap, s.D, 2) || !view_fits(bv, B, s.Hkv, cap, s.D, 2)) {
+    return MFA_ERROR_INVALID_ARGS;
+  }
+  if (bs->ndim || bs->bytes < (size_t)B * 4) return MFA_ERROR_INVALID_ARGS;
+  if (s.packed && (bc->ndim || bc->bytes < ((size_t)B + 1) * 4)) return MFA_ERROR_INVALID_ARGS;
+  if (s.packed && bc->host) {
+    const int32_t* cu = reinterpret_cast<const int32_t*>(bc->host);
+    if (cu[0] != 0 || cu[B] != (int64_t)s.total_q) return MFA_ERROR_INVALID_ARGS;
+    for (uint32_t b = 0; b < B; ++b)
+      if (cu[b + 1] < cu[b] || (int64_t)cu[b + 1] - cu[b] > (int64_t)s.Sq) return MFA_ERROR_INVALID_ARGS;
+  }
+  if (bs->host) {
+    const int32_t* len = reinterpret_cast<const int32_t*>(bs->host);
+    for (uint32_t b = 0; b < B; ++b)
+      if (len[b] < 0 || (uint32_t)len[b] > max_len) return MFA_ERROR_INVALID_ARGS;
+  }
+  if (s.paged && bt->host) {
+    const int32_t* ids = reinterpret_cast<const int32_t*>(bt->host);
+    for (size_t i = 0, n = (size_t)B * (cap / s.page_size); i < n; ++i)
+      if (ids[i] < 0 || (uint32_t)ids[i] >= s.num_pages) return MFA_ERROR_INVALID_ARGS;
+  }
+  return MFA_SUCCESS;
+}
+
 // mfa_attention_forward_kvcache (cu_seqlens_q null: seq_len_q new tokens per sequence) and
 // mfa_attention_forward_kvcache_varlen (sequence b owns query rows [cu[b], cu[b+1]) of total_q, at most seq_len_q of them).
 static mfa_error_t kvcache_forward(
@@ -1279,45 +1332,18 @@ static mfa_error_t kvcache_forward(
   const uint32_t cap = cache_capacity;
   const bool packed = cu_seqlens_q != nullptr;
   const int dt = header_precision_to_dtype(input_precision), odt = header_precision_to_dtype(output_precision);
-  if ((dt != kBF16 && dt != kF16) || !valid_float_dtype(odt)) return MFA_ERROR_INVALID_ARGS;
-  if (B == 0 || Sq == 0 || H == 0 || H % Hkv || H / Hkv > 128 || D < 8 || D > 128 || (D & 7) || cap == 0) return MFA_ERROR_INVALID_ARGS;
-  if (B > 65535 || Sq > 0x7fffffffu || H > 65535 || cap > 0x7fffff80u || !(softmax_scale > 0.f)) return MFA_ERROR_INVALID_ARGS;
-  if (packed && (total_q == 0 || total_q > 0x7fffffffu || Sq > total_q)) return MFA_ERROR_INVALID_ARGS;
-  const bool paged = page_size > 0;
-  if (paged ? (!block_table || (page_size & 15) || cap % page_size || num_pages == 0 || num_pages > 0x7fffffffu) : block_table != nullptr)
-    return MFA_ERROR_INVALID_ARGS;
+  if (!valid_float_dtype(odt) || !(softmax_scale > 0.f)) return MFA_ERROR_INVALID_ARGS;
+  const KvCacheShape shape{B, Sq, total_q, H, Hkv, D, cap, page_size, num_pages, dt, packed, page_size > 0};
+  if (!kvcache_shape_ok(shape, block_table)) return MFA_ERROR_INVALID_ARGS;
+  const bool paged = shape.paged;
   if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
   Buffer *bq = B_(q), *bk = B_(k_cache), *bv = B_(v_cache), *bo = B_(out), *bl = B_(lse), *bs = B_(cache_seqlens), *bt = B_(block_table);
   Buffer* bc = B_(cu_seqlens_q);
   // Q / O / L: [B, H, Sq] rows, or the [1, H, total_q] packed rows
   const uint32_t qB = packed ? 1 : B, qS = packed ? total_q : Sq;
   if (!view_fits(bq, qB, H, qS, D, 2) || !view_fits(bo, qB, H, qS, D, dtype_bytes(odt))) return MFA_ERROR_INVALID_ARGS;
-  if (paged) {
-    const size_t pool = (size_t)num_pages * page_size * Hkv * D * 2;
-    if (bk->ndim || bv->ndim || bk->bytes < pool || bv->bytes < pool) return MFA_ERROR_INVALID_ARGS;
-    if (bt->ndim || bt->bytes < (size_t)B * (cap / page_size) * 4) return MFA_ERROR_INVALID_ARGS;
-  } else if (!view_fits(bk, B, Hkv, cap, D, 2) || !view_fits(bv, B, Hkv, cap, D, 2)) {
-    return MFA_ERROR_INVALID_ARGS;
-  }
-  if (bs->ndim || bs->bytes < (size_t)B * 4 || (bl && bl->bytes < (size_t)qB * H * qS * 4)) return MFA_ERROR_INVALID_ARGS;
-  if (packed && (bc->ndim || bc->bytes < ((size_t)B + 1) * 4)) return MFA_ERROR_INVALID_ARGS;
-  // offsets, lengths and page ids the host can read are checked here; device-resident ones are clamped by the kernels
-  if (packed && bc->host) {
-    const int32_t* cu = reinterpret_cast<const int32_t*>(bc->host);
-    if (cu[0] != 0 || cu[B] != (int64_t)total_q) return MFA_ERROR_INVALID_ARGS;
-    for (uint32_t b = 0; b < B; ++b)
-      if (cu[b + 1] < cu[b] || (int64_t)cu[b + 1] - cu[b] > (int64_t)Sq) return MFA_ERROR_INVALID_ARGS;
-  }
-  if (bs->host) {
-    const int32_t* len = reinterpret_cast<const int32_t*>(bs->host);
-    for (uint32_t b = 0; b < B; ++b)
-      if (len[b] < 0 || (uint32_t)len[b] > cap) return MFA_ERROR_INVALID_ARGS;
-  }
-  if (paged && bt->host) {
-    const int32_t* ids = reinterpret_cast<const int32_t*>(bt->host);
-    for (size_t i = 0, n = (size_t)B * (cap / page_size); i < n; ++i)
-      if (ids[i] < 0 || (uint32_t)ids[i] >= num_pages) return MFA_ERROR_INVALID_ARGS;
-  }
+  if (bl && bl->bytes < (size_t)qB * H * qS * 4) return MFA_ERROR_INVALID_ARGS;
+  if (mfa_error_t e = check_kvcache_arrays(shape, bk, bv, bs, bt, bc, cap)) return e;
   const bool async = stream != nullptr;
   if (async && (bq->mirrored || bk->mirrored || bv->mirrored || bo->mirrored || (bl && bl->mirrored) || bs->mirrored || (bt && bt->mirrored) ||
                 (bc && bc->mirrored)))
@@ -1413,6 +1439,89 @@ mfa_error_t mfa_attention_forward_kvcache_varlen(
   return kvcache_forward(context, q, k_cache, v_cache, out, lse, cu_seqlens_q, cache_seqlens, block_table, num_seqs, max_seqlen_q,
                          total_q, num_heads, num_kv_heads, head_dim, cache_capacity, page_size, num_pages, softmax_scale, causal,
                          window_size, input_precision, output_precision, stream);
+}
+
+mfa_error_t mfa_kvcache_append(
+    mfa_context_t context, mfa_buffer_t q, mfa_buffer_t q_out, mfa_buffer_t k_new, mfa_buffer_t v_new,
+    mfa_buffer_t k_cache, mfa_buffer_t v_cache,
+    mfa_buffer_t cu_seqlens_q, mfa_buffer_t cache_seqlens, mfa_buffer_t block_table,
+    mfa_buffer_t rotary_cos, mfa_buffer_t rotary_sin, uint32_t rotary_rows, uint16_t rotary_dim, bool rotary_interleaved,
+    uint32_t num_seqs, uint32_t total_q, uint32_t max_seqlen_q, uint32_t num_heads, uint32_t num_kv_heads, uint16_t head_dim,
+    uint32_t cache_capacity, uint32_t page_size, uint32_t num_pages,
+    mfa_precision_t input_precision, void* stream) {
+  if (!context || !k_new || !v_new || !k_cache || !v_cache || !cache_seqlens) return MFA_ERROR_INVALID_ARGS;
+  const bool packed = cu_seqlens_q != nullptr, rotary = rotary_cos != nullptr;
+  const uint32_t B = num_seqs, Sq = max_seqlen_q, H = num_heads, Hkv = num_kv_heads ? num_kv_heads : num_heads, D = head_dim;
+  if ((q == nullptr) != (q_out == nullptr) || (q && !rotary) || (rotary_sin != nullptr) != rotary) return MFA_ERROR_INVALID_ARGS;
+  if (rotary ? (rotary_dim == 0 || (rotary_dim & 15) || rotary_dim > D || rotary_rows == 0 || rotary_rows > 0x7fffffffu)
+             : rotary_dim != 0)
+    return MFA_ERROR_INVALID_ARGS;
+  const KvCacheShape shape{B, Sq, total_q, H, Hkv, D, cache_capacity, page_size, num_pages,
+                           header_precision_to_dtype(input_precision), packed, page_size > 0};
+  if (!kvcache_shape_ok(shape, block_table)) return MFA_ERROR_INVALID_ARGS;
+  const uint64_t tokens = packed ? total_q : (uint64_t)B * Sq;        // one CTA per token
+  if (tokens > 0x7fffffffu) return MFA_ERROR_INVALID_ARGS;
+  if (!device_ok()) return MFA_ERROR_DEVICE_NOT_SUPPORTED;
+  Buffer *bq = B_(q), *bqo = B_(q_out), *bkn = B_(k_new), *bvn = B_(v_new), *bk = B_(k_cache), *bv = B_(v_cache);
+  Buffer *bc = B_(cu_seqlens_q), *bs = B_(cache_seqlens), *bt = B_(block_table), *bcos = B_(rotary_cos), *bsin = B_(rotary_sin);
+  const uint32_t qB = packed ? 1 : B, qS = packed ? total_q : Sq;
+  if (q && (!view_fits(bq, qB, H, qS, D, 2) || !view_fits(bqo, qB, H, qS, D, 2))) return MFA_ERROR_INVALID_ARGS;
+  if (!view_fits(bkn, qB, Hkv, qS, D, 2) || !view_fits(bvn, qB, Hkv, qS, D, 2)) return MFA_ERROR_INVALID_ARGS;
+  const size_t table_bytes = (size_t)rotary_rows * (rotary_dim / 2) * 4;
+  if (rotary && (bcos->ndim || bsin->ndim || bcos->bytes < table_bytes || bsin->bytes < table_bytes)) return MFA_ERROR_INVALID_ARGS;
+  if (mfa_error_t e = check_kvcache_arrays(shape, bk, bv, bs, bt, bc, rotary ? std::min(cache_capacity, rotary_rows) : cache_capacity))
+    return e;
+  const bool async = stream != nullptr;
+  const Buffer* all[] = {bq, bqo, bkn, bvn, bk, bv, bc, bs, bt, bcos, bsin};
+  if (async)
+    for (const Buffer* b : all)
+      if (b && b->mirrored) return MFA_ERROR_INVALID_ARGS;
+
+  Context* ctx = C_(context);
+  std::lock_guard<std::recursive_mutex> lock(ctx->mu);
+  DeviceGuard dg(ctx->device);
+  KvAppendParams p;
+  memset(&p, 0, sizeof(p));
+  if (q) {
+    p.q = view_of(bq, H, qS, D, false);
+    p.q_out = view_of(bqo, H, qS, D, false);
+  }
+  p.k_new = view_of(bkn, Hkv, qS, D, false);
+  p.v_new = view_of(bvn, Hkv, qS, D, false);
+  p.k = view_of(bk, Hkv, cache_capacity, D, false);
+  p.v = view_of(bv, Hkv, cache_capacity, D, false);
+  p.seqlens = reinterpret_cast<const int*>(bs->dev);
+  p.block_table = shape.paged ? reinterpret_cast<const int*>(bt->dev) : nullptr;
+  p.cu_q = packed ? reinterpret_cast<const int*>(bc->dev) : nullptr;
+  p.cos_t = rotary ? reinterpret_cast<const float*>(bcos->dev) : nullptr;
+  p.sin_t = rotary ? reinterpret_cast<const float*>(bsin->dev) : nullptr;
+  p.rotary_rows = (int)rotary_rows; p.rotary_dim = rotary_dim; p.interleaved = rotary_interleaved ? 1 : 0;
+  p.B = (int)B; p.H = (int)H; p.Hkv = (int)Hkv; p.Sq = (int)Sq; p.D = (int)D; p.cap = (int)cache_capacity;
+  p.page_size = (int)page_size; p.num_pages = (int)num_pages;
+  p.total_q = (int)tokens; p.dtype = shape.dtype;
+  // 16-byte vector accesses: aligned bases and outer strides, unit stride along D
+  if ((q && (!tc::view_ok(p.q, H, qB) || !tc::view_ok(p.q_out, H, qB))) || !tc::view_ok(p.k_new, Hkv, qB) ||
+      !tc::view_ok(p.v_new, Hkv, qB) || (!shape.paged && (!tc::view_ok(p.k, Hkv, B) || !tc::view_ok(p.v, Hkv, B))) ||
+      ((reinterpret_cast<uintptr_t>(bk->dev) | reinterpret_cast<uintptr_t>(bv->dev)) & 15) ||
+      (rotary && ((reinterpret_cast<uintptr_t>(bcos->dev) | reinterpret_cast<uintptr_t>(bsin->dev)) & 15)))
+    return MFA_ERROR_INVALID_ARGS;
+
+  cudaStream_t st = async ? reinterpret_cast<cudaStream_t>(stream) : ctx->stream;
+  Sync sync{ctx, st, async, {}};
+  cudaError_t e = cudaSuccess;
+  // the caches and q_out are copied in too: rows the kernel does not write must come back unchanged
+  for (const Buffer* b : all)
+    if (e == cudaSuccess) e = sync.in(const_cast<Buffer*>(b));
+  if (e != cudaSuccess) return cuda_fail(e, "h2d");
+  Timer tm(ctx, st, !async);
+  e = launch_kvcache_append(p, st);
+  tm.stop();
+  ctx->last_kernel = g_last_kernel;
+  if (e != cudaSuccess) return cuda_fail(e, "kvcache append launch");
+  sync.out(bk); sync.out(bv); sync.out(bqo);
+  if ((e = sync.finish()) != cudaSuccess) return cuda_fail(e, "kvcache append sync");
+  tm.read();
+  return MFA_SUCCESS;
 }
 
 // ---- quantised forward family ---------------------------------------------------------------------

@@ -418,7 +418,7 @@ __global__ void hadamard_kernel(float* __restrict__ data, uint32_t n, uint32_t n
   }
 }
 
-// ---- interleaved-pair RoPE (Sources/MFABridge/MFABridge.swift:269-319): (x0, x1) -> (x0 c - x1 s, x0 s + x1 c).
+// ---- interleaved-pair RoPE (Sources/MFABridge/MFABridge.swift:269-319): (x0, x1) -> (x0 c - x1 s, x0 s + x1 c) (rope_pair).
 // Tables follow the reference contract exactly: pair-duplicated fp32 [S, D] (only the even entry of a pair is read),
 // element t = b * table_batch_stride + s * D + 2 * pair, table_batch_stride = 0 (shared) or S * D ([B, S, D]).
 template <typename T> __device__ __forceinline__ T from_f32(float x);
@@ -443,9 +443,10 @@ __global__ void rope_kernel(const T* __restrict__ src, T* __restrict__ dst, cons
     const int64_t ti = b * table_batch_stride + (int64_t)s * D + 2 * j;
     float c = cos_t[ti], sn = sin_t[ti];
     if (negate_sin) sn = -sn;
-    float x0 = to_f32<T>(src[in]), x1 = to_f32<T>(src[in + 1]);
-    dst[out] = from_f32<T>(x0 * c - x1 * sn);
-    dst[out + 1] = from_f32<T>(x0 * sn + x1 * c);
+    float y0, y1;
+    rope_pair(to_f32<T>(src[in]), to_f32<T>(src[in + 1]), c, sn, y0, y1);
+    dst[out] = from_f32<T>(y0);
+    dst[out + 1] = from_f32<T>(y1);
   }
 }
 

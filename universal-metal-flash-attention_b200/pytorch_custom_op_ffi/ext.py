@@ -325,8 +325,57 @@ def _bshd_handle(bind, t):
     return h
 
 
+def _check_append_args(fn, q, k_cache, k, v, rotary_cos, rotary_sin):
+    """Arguments of the cache append of the K/V-cache calls: k / v shaped like q with the caches' KV heads, fp32 rotary tables
+    [rotary_rows, rotary_dim / 2] with rotary_dim a multiple of 16 up to D, and no tables without k / v."""
+    if (k is None) != (v is None):
+        raise RuntimeError(f"{fn}: k and v go together")
+    if (rotary_cos is None) != (rotary_sin is None):
+        raise RuntimeError(f"{fn}: rotary_cos and rotary_sin go together")
+    if k is None:
+        if rotary_cos is not None:
+            raise RuntimeError(f"{fn}: rotary_cos / rotary_sin need k and v: the new tokens' keys are rotated on their way into "
+                               "the cache, and q with them")
+        return
+    if torch.is_grad_enabled() and (k.requires_grad or v.requires_grad):
+        raise RuntimeError(f"{fn} has no backward: call it under torch.no_grad() or on tensors that do not require grad")
+    want = (*q.shape[:-2], k_cache.size(2) if k_cache.dim() == 4 else -1, q.size(-1))
+    for name, t in (("k", k), ("v", v)):
+        if tuple(t.shape) != want or t.dtype != q.dtype or t.device != q.device or t.stride(-1) != 1:
+            raise RuntimeError(f"{fn}: {name} must be {want} in q's dtype on q's device with unit stride along head_dim, got "
+                               f"{tuple(t.shape)} {t.dtype} on {t.device}")
+    if rotary_cos is None:
+        return
+    if rotary_cos.dtype != torch.float32 or rotary_sin.dtype != torch.float32:
+        raise RuntimeError(f"{fn}: rotary_cos / rotary_sin must be float32")
+    if rotary_cos.dim() != 2 or rotary_cos.shape != rotary_sin.shape or rotary_cos.size(0) == 0:
+        raise RuntimeError(f"{fn}: rotary_cos / rotary_sin must be [rotary_rows, rotary_dim / 2], got "
+                           f"{tuple(rotary_cos.shape)} and {tuple(rotary_sin.shape)}")
+    rd = 2 * rotary_cos.size(1)
+    if rd == 0 or rd % 16 or rd > q.size(-1):
+        raise RuntimeError(f"{fn}: rotary_dim = {rd} must be a multiple of 16 and at most head_dim = {q.size(-1)}")
+    for t in (rotary_cos, rotary_sin):
+        if t.device != q.device or not t.is_contiguous():
+            raise RuntimeError(f"{fn}: rotary_cos / rotary_sin must be contiguous tensors on q's device")
+
+
+def _append(bind, handle, stream, q, k, v, kch, vch, cu_seqlens_q, cache_seqlens, block_table, rotary_cos, rotary_sin,
+            interleaved, B, T, max_sq, H, Hkv, D, cap, page, npages):
+    """Enqueues mfa_kvcache_append; returns the Q the attention reads (rotated into a new tensor when there are tables)."""
+    q_out = None if rotary_cos is None else torch.empty(q.shape, device=q.device, dtype=q.dtype)
+    rows, rd = (0, 0) if rotary_cos is None else (rotary_cos.size(0), 2 * rotary_cos.size(1))
+    rc = _lib.mfa_kvcache_append(
+        bind.ctx.handle, None if q_out is None else handle(bind, q), None if q_out is None else handle(bind, q_out),
+        handle(bind, k), handle(bind, v), kch, vch, bind(cu_seqlens_q), bind(cache_seqlens), bind(block_table), bind(rotary_cos),
+        bind(rotary_sin), rows, rd, bool(interleaved), B, T, max_sq, H, Hkv, D, cap, page, npages, _PREC[q.dtype], stream)
+    if rc != 0:
+        raise RuntimeError(f"Metal Flash Attention kvcache append failed with code {rc}: {_ffi._get_error_string(rc)}")
+    return q if q_out is None else q_out
+
+
 def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block_table=None, is_causal=True, scale=None,
-                                       window=-1, return_lse=False):
+                                       window=-1, return_lse=False, *, k=None, v=None, rotary_cos=None, rotary_sin=None,
+                                       rotary_interleaved=False):
     """Attention of the Sq new tokens of each sequence against that sequence's K/V cache (inference decode, speculative
     decode, chunked prefill).  q is [B, Sq, H, D] (bf16 / fp16, D a multiple of 8 up to 128); k_cache / v_cache are
     [B, capacity, Hkv, D], or with block_table (int32 [B, capacity / page_size] page ids) paged pools
@@ -337,7 +386,16 @@ def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block
     the last 128-key tile (in a paged cache: rows of the pages that block_table points to there) are read and enter P V with
     weight 0, so they must hold finite values: allocate pools with torch.zeros, not torch.empty.  Enqueued on torch's current
     stream with no copies of q or the caches, so it can be captured in a CUDA graph after one call of the shape outside the
-    capture; the graph stays valid when later calls of other shapes run.  Forward only."""
+    capture; the graph stays valid when later calls of other shapes run.  Forward only.
+
+    With k / v ([B, Sq, Hkv, D], the new tokens' keys and values) the call first writes them into the caches, in place, at rows
+    cache_seqlens[b] - Sq + s, then runs the attention; both are enqueued on the current stream.  Unlike flash-attn's
+    flash_attn_with_kvcache, cache_seqlens keeps its meaning here: the lengths after the append, the new tokens included.  With
+    rotary_cos / rotary_sin (fp32 [rotary_rows, rotary_dim / 2], one angle per pair, rotary_dim a multiple of 16 up to D) K is
+    rotated on its way into the cache and Q with it, both at their cache positions (table row = cache row): rotary_interleaved
+    pairs (2i, 2i+1), otherwise the half-split pairs (i, i + rotary_dim / 2) of Llama / NeoX.  The rotated Q goes to a new tensor;
+    q itself is not modified.  Rotary tables without k / v raise, as in flash-attn."""
+    _check_append_args("metal_flash_attention_with_kvcache", q, k_cache, k, v, rotary_cos, rotary_sin)
     if torch.is_grad_enabled() and any(t.requires_grad for t in (q, k_cache, v_cache)):
         raise RuntimeError("metal_flash_attention_with_kvcache has no backward: call it under torch.no_grad() or on "
                            "tensors that do not require grad")
@@ -376,9 +434,13 @@ def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block
     stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(q.device).cuda_stream or 0), q)
     with _Bound(lib_ctx) as bind:
         paged = block_table is not None
+        kch = bind(k_cache) if paged else _bshd_handle(bind, k_cache)
+        vch = bind(v_cache) if paged else _bshd_handle(bind, v_cache)
+        if k is not None:
+            q = _append(bind, _bshd_handle, stream, q, k, v, kch, vch, None, cache_seqlens, block_table, rotary_cos, rotary_sin,
+                        rotary_interleaved, B, 0, Sq, H, Hkv, D, cap, page, npages)
         rc = _lib.mfa_attention_forward_kvcache(
-            lib_ctx.handle, _bshd_handle(bind, q), bind(k_cache) if paged else _bshd_handle(bind, k_cache),
-            bind(v_cache) if paged else _bshd_handle(bind, v_cache), _bshd_handle(bind, out), bind(lse), bind(cache_seqlens),
+            lib_ctx.handle, _bshd_handle(bind, q), kch, vch, _bshd_handle(bind, out), bind(lse), bind(cache_seqlens),
             bind(block_table), B, Sq, H, Hkv, D, cap, page, npages, float(scale), bool(is_causal),
             -1 if window is None or window < 0 else int(window), _PREC[q.dtype], _PREC[q.dtype], stream)
     if rc != 0:
@@ -387,7 +449,8 @@ def metal_flash_attention_with_kvcache(q, k_cache, v_cache, cache_seqlens, block
 
 
 def metal_flash_attention_varlen_with_kvcache(q, k_cache, v_cache, cu_seqlens_q, cache_seqlens, max_seqlen_q, block_table=None,
-                                              is_causal=True, scale=None, window_size=None, return_lse=False):
+                                              is_causal=True, scale=None, window_size=None, return_lse=False, *, k=None, v=None,
+                                              rotary_cos=None, rotary_sin=None, rotary_interleaved=False):
     """metal_flash_attention_with_kvcache with a per-sequence number of new tokens: one call for a continuous-batching step
     that mixes decodes, speculative runs and prefill chunks.  q is [total_q, H, D]; sequence b owns query rows
     cu_seqlens_q[b]:cu_seqlens_q[b+1] (int32 CUDA tensor of num_seqs + 1 offsets: 0, non-decreasing, ending at total_q), and
@@ -396,7 +459,12 @@ def metal_flash_attention_varlen_with_kvcache(q, k_cache, v_cache, cu_seqlens_q,
     int bounding every segment: it sizes the work, so nothing is read back from the device.  Returns O [total_q, H, D] in q's
     dtype (and L fp32 [H, total_q] in log2 units with return_lse).  Enqueued on torch's current stream with no copies of q or
     the caches; it can be captured in a CUDA graph after one call of the shape outside the capture, and replays may carry new
-    cu_seqlens_q contents, cache lengths and cache contents.  Forward only."""
+    cu_seqlens_q contents, cache lengths and cache contents.  Forward only.
+
+    k / v ([total_q, Hkv, D]), rotary_cos / rotary_sin and rotary_interleaved append the new tokens' K / V (rotated) to the caches
+    first, as in metal_flash_attention_with_kvcache: token s of sequence b goes to cache row and table row
+    cache_seqlens[b] - sq_b + s, and cache_seqlens counts the new tokens (unlike flash-attn)."""
+    _check_append_args("metal_flash_attention_varlen_with_kvcache", q, k_cache, k, v, rotary_cos, rotary_sin)
     if torch.is_grad_enabled() and any(t.requires_grad for t in (q, k_cache, v_cache)):
         raise RuntimeError("metal_flash_attention_varlen_with_kvcache has no backward: call it under torch.no_grad() or on "
                            "tensors that do not require grad")
@@ -444,9 +512,13 @@ def metal_flash_attention_varlen_with_kvcache(q, k_cache, v_cache, cu_seqlens_q,
     stream = _stream_arg(ctypes.c_void_p(torch.cuda.current_stream(q.device).cuda_stream or 0), q)
     with _Bound(lib_ctx) as bind:
         paged = block_table is not None
+        kch = bind(k_cache) if paged else _bshd_handle(bind, k_cache)
+        vch = bind(v_cache) if paged else _bshd_handle(bind, v_cache)
+        if k is not None:
+            q = _append(bind, _thd_handle, stream, q, k, v, kch, vch, cu_seqlens_q, cache_seqlens, block_table, rotary_cos,
+                        rotary_sin, rotary_interleaved, B, T, max_seqlen_q, H, Hkv, D, cap, page, npages)
         rc = _lib.mfa_attention_forward_kvcache_varlen(
-            lib_ctx.handle, _thd_handle(bind, q), bind(k_cache) if paged else _bshd_handle(bind, k_cache),
-            bind(v_cache) if paged else _bshd_handle(bind, v_cache), _thd_handle(bind, out), bind(lse), bind(cu_seqlens_q),
+            lib_ctx.handle, _thd_handle(bind, q), kch, vch, _thd_handle(bind, out), bind(lse), bind(cu_seqlens_q),
             bind(cache_seqlens), bind(block_table), B, T, max_seqlen_q, H, Hkv, D, cap, page, npages, float(scale),
             bool(is_causal), -1 if window_size is None or window_size < 0 else int(window_size), _PREC[q.dtype], _PREC[q.dtype],
             stream)

@@ -135,6 +135,8 @@ SIGNATURES = {
                                       [_f32, _b, _i32, _i32, _i32, _vp]),
     "mfa_attention_forward_kvcache_varlen": (_i32, [_ctx] + [_buf] * 8 + [_u32, _u32, _u32, _u32, _u32, _u16, _u32, _u32, _u32] +
                                              [_f32, _b, _i32, _i32, _i32, _vp]),
+    "mfa_kvcache_append": (_i32, [_ctx] + [_buf] * 11 + [_u32, _u16, _b, _u32, _u32, _u32, _u32, _u32, _u16, _u32, _u32, _u32,
+                                                        _i32, _vp]),
     "mfa_quantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _i32, _f32, _vp]),
     "mfa_dequantize": (_i32, [_ctx, _buf, _buf, _buf, _u64, _u64, _u32, _u32, _i32, _vp]),
     "mfa_merge_partials": (_i32, [_ctx, _buf, _buf, _buf, _buf, _u64, _u32, _vp]),

@@ -543,6 +543,82 @@ def flash_attention_kvcache_varlen(context: MFAContext, q, k_cache, v_cache, cu_
     return out, lse
 
 
+def _rotary_tables(rotary_cos, rotary_sin, D):
+    """(cos, sin, rotary_rows, rotary_dim) of fp32 [rotary_rows, rotary_dim / 2] tables, or (None, None, 0, 0)."""
+    if rotary_cos is None and rotary_sin is None:
+        return None, None, 0, 0
+    if rotary_cos is None or rotary_sin is None:
+        raise ValueError("rotary_cos and rotary_sin go together")
+    cos, sin = (np.ascontiguousarray(t) for t in (rotary_cos, rotary_sin))
+    if cos.dtype != np.float32 or sin.dtype != np.float32:
+        raise ValueError("rotary_cos / rotary_sin must be float32")
+    if cos.ndim != 2 or cos.shape != sin.shape or cos.shape[0] == 0:
+        raise ValueError(f"rotary_cos / rotary_sin must be [rotary_rows, rotary_dim / 2], got {cos.shape} and {sin.shape}")
+    rd = 2 * cos.shape[1]
+    if rd == 0 or rd % 16 or rd > D:
+        raise ValueError(f"rotary_dim = {rd} must be a multiple of 16 and at most head_dim = {D}")
+    return cos, sin, cos.shape[0], rd
+
+
+def kvcache_append(context: MFAContext, k_new, v_new, k_cache, v_cache, cache_seqlens, block_table=None, *, q=None,
+                   cu_seqlens_q=None, max_seqlen_q: Optional[int] = None, rotary_cos=None, rotary_sin=None,
+                   rotary_interleaved: bool = False, input_precision: Precision = "bf16"):
+    """Writes the new tokens' K / V into a K/V cache (mfa_kvcache_append), rotating K (and q, when given) with the rotary tables.
+    k_new / v_new are [B, Sq, Hkv, D] (q [B, Sq, H, D]), or with cu_seqlens_q [total_q, Hkv, D] (q [total_q, H, D]).  Caches,
+    block_table and cache_seqlens are those of flash_attention_kvcache: cache_seqlens[b] counts the new tokens, and token s of
+    sequence b goes to cache row (and table row) cache_seqlens[b] - sq_b + s.  rotary_cos / rotary_sin are fp32
+    [rotary_rows, rotary_dim / 2]; rotary_interleaved pairs (2i, 2i+1), otherwise (i, i + rotary_dim / 2).  k_cache / v_cache must
+    be C-contiguous arrays and are updated in place.  Returns the rotated q (a new array) or None."""
+    cos, sin, rows, rd = _rotary_tables(rotary_cos, rotary_sin, np.shape(k_new)[-1])
+    if q is not None and cos is None:
+        raise ValueError("rotating q needs rotary_cos / rotary_sin")
+    for name, x in (("k_cache", k_cache), ("v_cache", v_cache)):
+        if not isinstance(x, np.ndarray) or not x.flags.c_contiguous:
+            raise ValueError(f"{name} must be a C-contiguous numpy array (it is updated in place)")
+    in_prec = _parse_precision(input_precision)
+    packed = cu_seqlens_q is not None
+    if packed:
+        if not isinstance(k_new, np.ndarray) or k_new.ndim != 3:
+            raise ValueError("with cu_seqlens_q, k_new / v_new must be [total_q, kv_heads, head_dim]")
+        qs = q if q is not None else np.empty(k_new.shape, k_new.dtype)
+        n, T, msq, H, Hkv, D, cap, page, npages, cu_q, lens, table = _kvcache_varlen_dims(
+            qs, k_cache, v_cache, cu_seqlens_q, cache_seqlens, block_table, max_seqlen_q)
+        kv_shape = (T, Hkv, D)
+        op = lambda arr, Hn: _varlen_operand(context, arr, Hn, T, D, "thd")                            # noqa: E731
+    else:
+        if not isinstance(k_new, np.ndarray) or k_new.ndim != 4:
+            raise ValueError("k_new / v_new must be [batch, new tokens, kv_heads, head_dim]")
+        qs = q if q is not None else np.empty(k_new.shape, k_new.dtype)
+        n, msq, H, Hkv, D, cap, page, npages, lens, table = _kvcache_dims(qs, k_cache, v_cache, cache_seqlens, block_table)
+        T, cu_q, kv_shape = 0, None, (n, msq, Hkv, D)
+        op = lambda arr, Hn: MFABuffer(context, arr, shape=(n, Hn, msq, D), strides=(msq * Hn * D, D, Hn * D, 1))   # noqa: E731
+    if np.shape(k_new) != kv_shape or np.shape(v_new) != kv_shape:
+        raise ValueError(f"k_new / v_new must be {kv_shape}, got {np.shape(k_new)} and {np.shape(v_new)}")
+    for name, x in (("q", q), ("k_new", k_new), ("v_new", v_new), ("k_cache", k_cache), ("v_cache", v_cache)):
+        if x is not None:
+            _check_input_dtype(x, in_prec, name)
+    q_out = None if q is None else np.zeros(q.shape, q.dtype)
+    bufs = [None if q is None else op(np.ascontiguousarray(q), H), None if q is None else op(q_out, H),
+            op(np.ascontiguousarray(k_new), Hkv), op(np.ascontiguousarray(v_new), Hkv)]
+    if table is None:
+        bshd = lambda arr: MFABuffer(context, arr, shape=(n, Hkv, cap, D), strides=(cap * Hkv * D, D, Hkv * D, 1))   # noqa: E731
+        bufs += [bshd(k_cache), bshd(v_cache)]
+    else:
+        bufs += [MFABuffer(context, k_cache), MFABuffer(context, v_cache)]
+    bufs += [None if cu_q is None else MFABuffer(context, cu_q), MFABuffer(context, lens),
+             None if table is None else MFABuffer(context, table),
+             None if cos is None else MFABuffer(context, cos), None if sin is None else MFABuffer(context, sin)]
+    try:
+        _check_error(_lib.mfa_kvcache_append(
+            context.handle, *[None if b is None else b.handle for b in bufs], rows, rd, bool(rotary_interleaved), n, T, msq,
+            H, Hkv, D, cap, page, npages, in_prec, None))
+    finally:
+        for b in bufs:
+            if b is not None:
+                b.close()
+    return q_out
+
+
 def flash_attention_varlen_backward(context: MFAContext, d_out, q, k, v, out, lse, cu_seqlens_q, cu_seqlens_k, *,
                                     causal: bool = False, softmax_scale: Optional[float] = None,
                                     input_precision: Precision = "fp32", window_size: Optional[int] = None,
